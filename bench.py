@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the soundgen source-filter synthesis path on B200.
 
-  python bench.py --gpus N --steps K --warmup W [--config 3] [--batch B]
+  python bench.py --gpus N --steps K --warmup W [--config 3] [--batch B] [--dump-outputs DIR]
   python bench.py --impl reference ...      (the reference algorithm on the host cores)
 
 A "step" is one pass of the whole hot path (control stage, amplitude matrices, additive
@@ -10,6 +10,10 @@ synthetic soundgen() calls of the chosen BASELINE.json config.  `value` is audio
 synthesised per second with inputs resident in HBM; `e2e` includes the H2D copy of the
 step's inputs from pinned host memory and the D2H read of every waveform.
 One JSON line is printed by rank 0.
+
+The inputs are seeded: the same arguments give the same calls on every run, and
+`--dump-outputs DIR` writes what the last timed step returned (see `dump_outputs`), so two
+builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -26,6 +30,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # a benchmark run leaves the tree as it found it: no __pycache__ beside the sources
 
 T_START = time.perf_counter()
 METRIC = 'audio_seconds_synthesised_per_second'
@@ -194,6 +199,33 @@ def parity_sample(calls, outs, idx):
             'dense_over_reference_partials': (pdense / pref) if pref else None}
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, out, lens, status):
+    """Writes what the timed path returned in its last step as .npy files under `path`:
+      lengths.npy           float64, the waveform length of every call of the batch
+      status.npy            float64, the status code of every call (0 = ok)
+      sample_calls.npy      float64, indices of the sampled calls, ascending
+      sample_waveforms.npy  float32, the waveforms of those calls, concatenated in that order
+    Every call is sampled when the files fit in DUMP_BYTES.  Otherwise the calls are visited in an order
+    drawn with a fixed seed from the batch size alone, and each one is kept while its waveform still fits."""
+    os.makedirs(path, exist_ok=True)
+    offs = np.concatenate(([0], np.cumsum(lens)))
+    budget = DUMP_BYTES - 24 * lens.size - 4 * 128     # the three float64 arrays and the four .npy headers
+    pick, used = [], 0
+    for i in np.random.default_rng(2026).permutation(lens.size):
+        if used + 4 * int(lens[i]) <= budget:
+            pick.append(int(i))
+            used += 4 * int(lens[i])
+    pick.sort()
+    np.save(os.path.join(path, 'lengths.npy'), lens.astype(np.float64))
+    np.save(os.path.join(path, 'status.npy'), status.astype(np.float64))
+    np.save(os.path.join(path, 'sample_calls.npy'), np.array(pick, dtype=np.float64))
+    np.save(os.path.join(path, 'sample_waveforms.npy'),
+            np.concatenate([out[offs[i]:offs[i + 1]] for i in pick] + [np.zeros(0, np.float32)]).astype(np.float32))
+
+
 def oracle_one(kw):
     """One soundgen() call through the CPU oracle; returns (seconds of audio, samples)."""
     from oracle import soundgen_oracle as so
@@ -281,7 +313,13 @@ def main():
                     help='host threads that run kernels in the end-to-end pipeline (plus one uploader, one fetcher); '
                          '0 = 4 when the rank has at least 8 host cores to itself, else 3')
     ap.add_argument('--watchdog', type=int, default=1500, help='seconds after which a stuck run dumps its stacks and exits')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step (rank 0) as DIR/<name>.npy, see dump_outputs()')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the GPU path; --impl reference has none')
     faulthandler.dump_traceback_later(args.watchdog, exit=True)   # a stuck run reports where, instead of hanging the box
     rank, world, local = env_int('RANK', 0), env_int('WORLD_SIZE', 1), env_int('LOCAL_RANK', 0)
     if args.impl == 'reference':
@@ -419,11 +457,15 @@ def main():
     d2h_bytes = d2h_f32
     clocks = sampler.stop()
     stage_ms /= args.steps
+    # ---- the waveforms of the last timed step (bt ran nothing since) ----
+    if (not args.no_parity or args.dump_outputs) and rank == 0:
+        bt.fetch(np.float32, out=out)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, bt.lengths(), bt.status())
     # ---- parity of the timed batch itself: a random sample of its calls against the CPU oracle ----
     parity = None
     if not args.no_parity and rank == 0:
         offs = np.concatenate(([0], np.cumsum(lens)))
-        bt.fetch(np.float32, out=out)
         pick = np.random.default_rng(7).choice(len(calls), size=min(args.parity_calls, len(calls)), replace=False)
         outs_pick = {int(i): out[offs[i]:offs[i + 1]] for i in pick}
         parity = parity_sample(calls, outs_pick, [int(i) for i in pick])

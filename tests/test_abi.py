@@ -4,7 +4,6 @@ import ctypes as C
 import os
 import re
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -42,17 +41,29 @@ def test_sass_has_tma_and_no_library_fft():
     assert 'cufft' not in ldd and 'torch' not in ldd
 
 
+NO_DEVICE_CHECK = '''
+import numpy as np
+import pytest
+import soundgen_beta_b200 as sg
+assert sg._abi.load().sgb_device_count() == 0
+with pytest.raises(sg.SoundgenError) as ei:
+    sg.soundgen(sylLen=300, pitchAnchors=[100, 150], temperature=0)
+assert ei.value.code == -2
+with pytest.raises(sg.SoundgenError):
+    sg.getRolloff([150.0])
+with pytest.raises(sg.SoundgenError):
+    sg.filter_sound(np.zeros(4000), np.ones(400), 800)
+'''
+
+
 def test_no_cpu_fallback(built_lib):
-    import soundgen_beta_b200 as sg
-    if built_lib.sgb_device_count() > 0:
-        pytest.skip('a GPU is present')
-    with pytest.raises(sg.SoundgenError) as ei:
-        sg.soundgen(sylLen=300, pitchAnchors=[100, 150], temperature=0)
-    assert ei.value.code == -2
-    with pytest.raises(sg.SoundgenError):
-        sg.getRolloff([150.0])
-    with pytest.raises(sg.SoundgenError):
-        sg.filter_sound(np.zeros(4000), np.ones(400), 800)
+    # a fresh process with every device hidden, so the no-device path runs on GPU machines too
+    import subprocess
+    import sys
+    code = 'import sys; sys.path.insert(0, %r)\n' % ROOT + NO_DEVICE_CHECK
+    r = subprocess.run([sys.executable, '-c', code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=''),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_product_never_imports_oracle():
