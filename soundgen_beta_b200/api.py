@@ -422,10 +422,8 @@ class BatchBuilder:
                 self.n_formants += f.shape[0]
         ma = host.as_anchors(mouthAnchors)
         if ma is not None and not np.any(np.isnan(ma[1])):
-            if 3 <= ma[0].size <= 10 and contour_method != 'spline':
-                raise NotImplementedError('mouthAnchors with 3-10 anchors use loess in the reference '
-                                          "(pass contour_method='spline')")
             e.mouth_off, e.mouth_n = self._add_anchors(ma)
+            e.mouth_method = _METHODS[contour_method]
         else:
             e.mouth_n = 0
         e.nc_fixed = int(nc_fixed)
@@ -460,10 +458,8 @@ class BatchBuilder:
         s.z_off, s.z_cap = self._add_z(z)
         an = host.as_anchors(amplAnchors)
         if an is not None:
-            if 3 <= an[0].size <= 10 and contour_method != 'spline':
-                raise NotImplementedError('amplAnchors with 3-10 anchors use loess in the reference '
-                                          "(pass contour_method='spline')")
             s.ampl_off, s.ampl_n = self._add_anchors(an)
+            s.ampl_method = _METHODS[contour_method]
         d = dict(attackLen=50, nonlinBalance=0, jitterDep=0, jitterLen=1, vibratoFreq=100, vibratoDep=0,
                  shimmerDep=0, rolloff=-18, rolloffOct=-2, rolloffKHz=-6, rolloffParab=0,
                  rolloffParabHarm=3, rolloff_perAmpl=12, temperature=0, pitchDriftDep=.5,
@@ -501,10 +497,8 @@ class BatchBuilder:
             n.strength_pre_off = self._add_pre(strength)
             n.anchor_n = 0
         else:
-            if 3 <= an[0].size <= 10 and contour_method != 'spline':
-                raise NotImplementedError('noiseAnchors with 3-10 anchors use loess in the reference: pass a '
-                                          "pre-evaluated `strength` contour or contour_method='spline'")
             n.anchor_off, n.anchor_n = self._add_anchors(an)
+            n.anchor_method = _METHODS[contour_method]
         n.env_id = int(env_id)
         n.rolloffNoise, n.attackLen = float(rolloffNoise), float(attackLen)
         n.samplingRate, n.overlap = float(samplingRate), float(overlap)
@@ -513,13 +507,14 @@ class BatchBuilder:
 
     def add_bout(self, syl_begin, syl_end, noise_begin, noise_end, env_id, moving, wl, overlap=75,
                  lead_silence=0, tail_silence=0, amplAnchorsGlobal=None, amDep=0, amFreq=30, amShape=0,
-                 samplingRate=16000, throwaway=-120):
+                 samplingRate=16000, throwaway=-120, contour_method='loess'):
         b = Bout()
         b.syl_begin, b.syl_end, b.noise_begin, b.noise_end = syl_begin, syl_end, noise_begin, noise_end
         b.env_id, b.moving, b.wl = int(env_id), int(bool(moving)), int(wl)
         b.lead_silence, b.tail_silence = int(lead_silence), int(tail_silence)
         if amplAnchorsGlobal is not None:
             b.aglobal_off, b.aglobal_n = self._add_anchors(amplAnchorsGlobal)
+            b.aglobal_method = _METHODS[contour_method]
         b.overlap, b.amDep, b.amFreq, b.amShape = float(overlap), float(amDep), float(amFreq), float(amShape)
         b.samplingRate, b.throwaway = float(samplingRate), float(throwaway)
         self.bouts.append(b)
@@ -969,9 +964,9 @@ def generateHarmonics(pitch, attackLen=50, nonlinBalance=0, nonlinDep=0, jitterD
 
 def generateNoise(len, noiseAnchors=((0, 300), (-120, -120)), rolloffNoise=-6, attackLen=10,
                   windowLength_points=1024, samplingRate=16000, overlap=75, throwaway=-120, filterNoise=None,
-                  u=None, strength=None):
+                  u=None, strength=None, contour_method='loess'):
     """generateNoise() (R/source.R:57-68).  `u`: the runif(nr * nc) draws; filterNoise:
-    None or an (nr x k) matrix (as returned by getSpectralEnvelope)."""
+    None or an (nr x k) matrix (as returned by getSpectralEnvelope).  `contour_method` smooths noiseAnchors."""
     bb = BatchBuilder()
     bb.add_silent_syllable(8)
     env = bb.add_envelope(None, samplingRate=samplingRate)
@@ -983,7 +978,7 @@ def generateNoise(len, noiseAnchors=((0, 300), (-120, -120)), rolloffNoise=-6, a
         env_n = bb.add_envelope_matrix(fm, samplingRate=samplingRate)
     bb.add_noise(len, noiseAnchors, u, rolloffNoise=rolloffNoise, attackLen=attackLen,
                  windowLength_points=windowLength_points, samplingRate=samplingRate, overlap=overlap,
-                 insertion=1, mix=0, strength=strength, env_id=env_n)
+                 insertion=1, mix=0, strength=strength, env_id=env_n, contour_method=contour_method)
     bb.add_bout(0, 1, 0, 1, env, False, max(4, int(windowLength_points)), samplingRate=samplingRate,
                 throwaway=throwaway)
     bb.add_call(0, 1)
@@ -1016,9 +1011,9 @@ def getRolloff(pitch_per_gc=(440,), nHarmonics=100, rolloff=-12, rolloffOct=-2, 
 def getSpectralEnvelope(nr, nc, formants=None, formantDep=1, rolloffLip=6, mouthAnchors=None,
                         mouthOpenThres=0, openMouthBoost=0, vocalTract=None, temperature=0, formDrift=.3,
                         formDisp=.2, formantDepStoch=30, smoothLinearFactor=1, samplingRate=16000,
-                        speedSound=35400, plot=False, formants_upsampled=None):
+                        speedSound=35400, plot=False, formants_upsampled=None, contour_method='loess'):
     """getSpectralEnvelope() (R/sourceSpectrum.R:261-283), deterministic part; with
-    temperature > 0 pass the host-drawn tracks as `formants_upsampled`."""
+    temperature > 0 pass the host-drawn tracks as `formants_upsampled`.  `contour_method` smooths mouthAnchors."""
     if temperature > 0 and formants_upsampled is None:
         raise NotImplementedError('stochastic formants are drawn on the host from R\'s RNG')
     L = _abi.load()
@@ -1026,7 +1021,8 @@ def getSpectralEnvelope(nr, nc, formants=None, formantDep=1, rolloffLip=6, mouth
     eid = bb.add_envelope(formants, formantDep=formantDep, rolloffLip=rolloffLip, mouthAnchors=mouthAnchors,
                           mouthOpenThres=mouthOpenThres, openMouthBoost=openMouthBoost, vocalTract=vocalTract,
                           samplingRate=samplingRate, speedSound=speedSound,
-                          smoothLinearFactor=smoothLinearFactor, tracks=formants_upsampled)
+                          smoothLinearFactor=smoothLinearFactor, tracks=formants_upsampled,
+                          contour_method=contour_method)
     e = bb.envs[eid]
     fm = np.ascontiguousarray(np.concatenate(bb.formants)) if bb.formants else np.zeros(4)
     fn = np.array([r.n for r in bb.frefs], dtype=np.int32) if bb.frefs else np.zeros(1, dtype=np.int32)

@@ -19,7 +19,6 @@
 #include "../../include/soundgen_b200.h"
 
 #define SGB_MAX_EPOCHS 128     // sub-harmonic epochs per syllable
-#define SGB_MAX_RW_KNOTS 64    // knots of a smoothed random walk (2^(1/rw_smoothing))
 
 // Per-syllable results of the control-rate stage (K0), device resident.
 struct SylCtrl {

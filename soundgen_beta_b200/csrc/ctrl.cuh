@@ -4,6 +4,9 @@
 // and the per-glottal-cycle arrays the sample-rate kernels consume.
 #pragma once
 #include "contour.cuh"
+#if !defined(__CUDACC__)
+#include <vector>
+#endif
 
 // ---------------------------------------------------------------- helpers ---
 // noiseThresholdsDict (data-raw/noiseThresholdsDict.R:4-18); a fractional
@@ -154,9 +157,10 @@ SGB_HD double ctrl_vibrato(const sgb_syllable &sp, int i, double p) {
 // Everything of generateHarmonics between the vibrato and the harmonic loop that is
 // inherently sequential per syllable.  A.pitch must already hold the vibrato'd
 // pitch contour.  ampl_contour: getSmoothContour(amplAnchors, len = nGC) is
-// evaluated by the caller-supplied anchors (1, 2 anchors or spline).
-SGB_HD void ctrl_sequential(const sgb_syllable &sp, const double *anchors, const double *zpool,
-                            SylArrays &A, SylCtrl &C) {
+// evaluated from atab / aknots, prepared with contour_prepare(len = 0, valueFloor = 0,
+// valueCeiling = -throwaway); a loess fit is done here for len = nGC.
+SGB_HD void ctrl_sequential(const sgb_syllable &sp, const double *anchors, const ContourTab *atab,
+                            const double *aknots, const double *zpool, SylArrays &A, SylCtrl &C) {
   const int P = sp.pitch_len;
   const double psr = sp.pitchSamplingRate, sr = sp.samplingRate;
   const double *z = zpool + sp.z_off;
@@ -193,12 +197,11 @@ SGB_HD void ctrl_sequential(const sgb_syllable &sp, const double *anchors, const
   double *rolloffAmpl = A.t4;
   if (C.use_ampl) {
     // getSmoothContour(len = nGC, valueFloor = 0, valueCeiling = -throwaway, samplingRate)
-    ContourTab T;
-    contour_prepare(&T, anchors + 2 * sp.ampl_off, sp.ampl_n, G, sp.samplingRate, true, 0.0, true,
-                    -sp.throwaway, false, sp.ampl_method);
+    ContourTab T = *atab;
+    contour_fit_len(&T, aknots, G, sp.samplingRate);
     if (T.status != SGB_OK) { C.status = T.status; return; }
     for (int g = 0; g < G; g++) {
-      double v = contour_eval(&T, G, g);
+      double v = contour_eval(&T, aknots, G, g);
       rolloffAmpl[g] = (v / fabs(sp.throwaway) - 1.0) * sp.rolloff_perAmpl;
     }
   } else {
@@ -424,6 +427,20 @@ SGB_HD void ctrl_sequential(const sgb_syllable &sp, const double *anchors, const
     }
   }
 }
+
+#if !defined(__CUDACC__)
+// Host builds of the scalar code: the same stage with the amplitude contour prepared here from the anchors,
+// as k_syl_contours prepares it for K0 (no length: a loess fit is done above for len = nGC).
+SGB_HD void ctrl_sequential(const sgb_syllable &sp, const double *anchors, const double *zpool, SylArrays &A,
+                            SylCtrl &C) {
+  ContourTab T{};
+  std::vector<double> K((size_t)contour_knot_doubles(sp.ampl_n > 0 ? sp.ampl_n : 1));
+  if (sp.ampl_n > 0)
+    contour_prepare(&T, K.data(), anchors + 2 * sp.ampl_off, sp.ampl_n, 0, sp.samplingRate, true, 0.0, true,
+                    -sp.throwaway, false, sp.ampl_method);
+  ctrl_sequential(sp, anchors, &T, K.data(), zpool, A, C);
+}
+#endif
 
 // column maximum of r[, g] (R/sourceSpectrum.R:146): one glottal cycle.
 SGB_HD double ctrl_colmax(const sgb_syllable &sp, const SylArrays &A, const SylCtrl &C, int g) {

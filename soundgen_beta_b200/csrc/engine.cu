@@ -25,7 +25,6 @@ void launch_tiles_amp(const sgb_syllable *, int, const SylCtrl *, const SylLayou
 void launch_rolloff_api(const double *, int, int, const double *, int, const double *, int, const double *, int,
                         double, double, double, double, double, double, double *, int *, double *, int *);
 void launch_fp32_peak(float2 *, int, int, int);
-#define ENV_MAXK_HOST 64
 void launch_synth(const SynthTile *, int, const sgb_syllable *, const SylCtrl *, const SylLayout *, const Pools &,
                   const float4 *, float *, int *, cudaStream_t);
 void launch_build_tiles_tc(const sgb_syllable *, const SylCtrl *, int, const SylLayout *, const Pools &, TcUnit *, cudaStream_t);
@@ -37,7 +36,7 @@ void launch_compose(const sgb_syllable *, int, SylCtrl *, const SylLayout *, con
 void launch_place_voiced(const sgb_syllable *, int, const SylCtrl *, const SylLayout *, const SylPlace *,
                          const Pools &, const float *, float *, int, cudaStream_t);
 void launch_env_tracks(const EnvInst *, int, const sgb_envelope *, const sgb_formant_ref *, const double *,
-                       const double *, double *, double *, void *, cudaStream_t);
+                       const double *, double *, double *, void *, double *, cudaStream_t);
 void launch_envelope_f32(const EnvInst *, int, int, const sgb_envelope *, const sgb_formant_ref *, const double *,
                          const double *, const double *, const double *, const double *, float *, cudaStream_t);
 void launch_envelope_f64(const EnvInst *, int, int, const sgb_envelope *, const sgb_formant_ref *, const double *,
@@ -49,10 +48,10 @@ cudaError_t launch_stft(int mode, int u_is_float, int spec, const FftSeg *, int,
                         size_t, cudaStream_t);
 int stft_spec_of(int n, const int *radix, int npass);
 void launch_noise_final(const sgb_noise *, int, const NoiseLayout *, const double *, const double *, const int *, int,
-                        const float *, float *, void *, int, cudaStream_t);
+                        const float *, float *, void *, double *, const int64_t *, int, cudaStream_t);
 size_t contour_tab_bytes();
 void launch_sound_mix(const sgb_bout *, int, const BoutLayout *, const sgb_noise *, const NoiseLayout *,
-                      const double *, const float *, float *, int, cudaStream_t);
+                      const double *, const float *, float *, void *, double *, const int64_t *, bool, int, cudaStream_t);
 void launch_finalize(int, const sgb_bout *, int, const BoutLayout *, const sgb_noise *, const NoiseLayout *,
                      const float *, const float *, const float *, const int *, void *, int, cudaStream_t);
 
@@ -190,6 +189,9 @@ struct sgb_batch {
   DBuf d_pcm, d_calltab;
   DBuf d_amp, d_amp32, d_wave, d_raw, d_sound, d_voiced, d_filt, d_noise_raw, d_noise_fin, d_env, d_out, d_out64;
   DBuf d_trk, d_mouth, d_formants_late, d_tiles_tc, d_ntabs, d_order, d_mtabs;
+  DBuf d_knots, d_koff, d_ctab, d_btabs, d_envk;   // contour knot pool, per-contour offsets, headers (contour.cuh)
+  int64_t knot_total = 0;
+  bool any_aglobal = false;
   struct RunState *rs = nullptr;     // state carried from run_begin to run_finish
   std::vector<double> late_rows;     // host-drawn formant tracks set between begin and finish
   std::vector<int32_t> h_order;
@@ -381,7 +383,8 @@ void sgb_batch_destroy(sgb_batch *b) {
                  &b->d_totals, &b->d_summary, &b->d_tiles, &b->d_epmax, &b->p_pitch_w, &b->d_amp, &b->d_amp32, &b->d_wave, &b->d_raw,
                  &b->d_sound, &b->d_voiced, &b->d_filt, &b->d_noise_raw, &b->d_noise_fin, &b->d_env, &b->d_out,
                  &b->d_out64, &b->d_bl, &b->d_place, &b->d_nl, &b->d_envinst, &b->d_plans, &b->d_tw, &b->d_win,
-                 &b->d_fjobs, &b->d_njobs, &b->d_fsegs, &b->d_nsegs, &b->d_max, &b->d_trk, &b->d_mouth, &b->d_formants_late, &b->d_tiles_tc, &b->d_ntabs, &b->d_order, &b->d_mtabs};
+                 &b->d_fjobs, &b->d_njobs, &b->d_fsegs, &b->d_nsegs, &b->d_max, &b->d_trk, &b->d_mouth, &b->d_formants_late, &b->d_tiles_tc, &b->d_ntabs, &b->d_order, &b->d_mtabs,
+                 &b->d_knots, &b->d_koff, &b->d_ctab, &b->d_btabs, &b->d_envk};
   for (auto d : all) d->release();
   for (auto &d : b->p_i32) d.release();
   for (auto &d : b->p_f64) d.release();
@@ -422,7 +425,6 @@ int sgb_batch_upload(sgb_batch *b, const sgb_batch_desc *D) {
     if (B.wl < 4) return fail(SGB_ERR_INVALID, "bout %d: windowLength_points %d < 4", i, B.wl);
     if (!(B.overlap >= 0.0 && B.overlap < 100.0)) return fail(SGB_ERR_INVALID, "bout %d: overlap out of range", i);
     if (!(B.samplingRate > 0)) return fail(SGB_ERR_INVALID, "bout %d: samplingRate", i);
-    if (B.aglobal_n > ENV_MAXK_HOST) return fail(SGB_ERR_UNSUPPORTED, "bout %d: more than %d amplAnchorsGlobal", i, ENV_MAXK_HOST);
     if (B.aglobal_n < 0 || (B.aglobal_n > 0 && (B.aglobal_off < 0 || B.aglobal_off + B.aglobal_n > D->n_anchors)))
       return fail(SGB_ERR_INVALID, "bout %d: amplAnchorsGlobal range outside the anchor pool", i);
     if (!(B.throwaway < 0)) return fail(SGB_ERR_INVALID, "bout %d: throwaway must be negative", i);
@@ -435,9 +437,7 @@ int sgb_batch_upload(sgb_batch *b, const sgb_batch_desc *D) {
     if (Y.pitch_len < 1 || Y.pitch_off < 0 || (!dev_pitch && Y.pitch_off + Y.pitch_len > D->n_pitch))
       return fail(SGB_ERR_INVALID, "syllable %d: pitch range outside the pool", s);
     if (Y.kind == 1 && Y.pitch_anchor_n != 0) {
-      if (Y.pitch_anchor_n < 0 || Y.pitch_anchor_n > ENV_MAXK_HOST)
-        return fail(SGB_ERR_UNSUPPORTED, "syllable %d: more than %d pitchAnchors", s, ENV_MAXK_HOST);
-      if (Y.pitch_anchor_off < 0 || Y.pitch_anchor_off + Y.pitch_anchor_n > D->n_anchors)
+      if (Y.pitch_anchor_n < 0 || Y.pitch_anchor_off < 0 || Y.pitch_anchor_off + Y.pitch_anchor_n > D->n_anchors)
         return fail(SGB_ERR_INVALID, "syllable %d: pitchAnchors range outside the anchor pool", s);
     }
     if (Y.kind == 2) continue;
@@ -445,7 +445,7 @@ int sgb_batch_upload(sgb_batch *b, const sgb_batch_desc *D) {
     if (!(Y.samplingRate > 0) || !(Y.pitchSamplingRate > 0) || !(Y.pitchFloor > 0) || !(Y.pitchCeiling >= Y.pitchFloor))
       return fail(SGB_ERR_INVALID, "syllable %d: sampling rates / pitch bounds", s);
     if (Y.z_cap < 0 || Y.z_off < 0 || Y.z_off + Y.z_cap > D->n_z) return fail(SGB_ERR_INVALID, "syllable %d: z range", s);
-    if (Y.ampl_n < 0 || Y.ampl_n > SGB_MAX_RW_KNOTS || (Y.ampl_n > 0 && (Y.ampl_off < 0 || Y.ampl_off + Y.ampl_n > D->n_anchors)))
+    if (Y.ampl_n < 0 || (Y.ampl_n > 0 && (Y.ampl_off < 0 || Y.ampl_off + Y.ampl_n > D->n_anchors)))
       return fail(SGB_ERR_INVALID, "syllable %d: amplAnchors range", s);
     if (!(Y.throwaway < 0)) return fail(SGB_ERR_INVALID, "syllable %d: throwaway must be negative", s);
   }
@@ -454,7 +454,7 @@ int sgb_batch_upload(sgb_batch *b, const sgb_batch_desc *D) {
     if (N.len < 1) return fail(SGB_ERR_INVALID, "noise %d: len < 1", n);
     if (N.wl < 4 || (N.wl & 1)) return fail(SGB_ERR_UNSUPPORTED, "noise %d: odd or tiny window", n);
     if (N.env_id >= D->n_envelopes) return fail(SGB_ERR_INVALID, "noise %d: env_id", n);
-    if (N.strength_pre_off < 0 && (N.anchor_n < 1 || N.anchor_n > ENV_MAXK_HOST || N.anchor_off < 0 || N.anchor_off + N.anchor_n > D->n_anchors))
+    if (N.strength_pre_off < 0 && (N.anchor_n < 1 || N.anchor_off < 0 || N.anchor_off + N.anchor_n > D->n_anchors))
       return fail(SGB_ERR_INVALID, "noise %d: anchors", n);
     if (N.strength_pre_off >= 0 && N.strength_pre_off + N.len > D->n_pre) return fail(SGB_ERR_INVALID, "noise %d: pre-evaluated contour range", n);
     double h = N.wl - (N.overlap * N.wl / 100.0);
@@ -468,8 +468,7 @@ int sgb_batch_upload(sgb_batch *b, const sgb_batch_desc *D) {
     if (E.n_formants < 0 || E.n_formants > 62) return fail(SGB_ERR_UNSUPPORTED, "envelope %d: more than 62 formants", e);
     if (E.n_formants > 0 && (E.formant_off < 0 || E.formant_off + E.n_formants > D->n_formant_refs))
       return fail(SGB_ERR_INVALID, "envelope %d: formant refs", e);
-    if (E.mouth_n < 0 || E.mouth_n > ENV_MAXK_HOST) return fail(SGB_ERR_UNSUPPORTED, "envelope %d: more than %d mouth anchors", e, ENV_MAXK_HOST);
-    if (E.mouth_n > 0 && (E.mouth_off < 0 || E.mouth_off + E.mouth_n > D->n_anchors))
+    if (E.mouth_n < 0 || (E.mouth_n > 0 && (E.mouth_off < 0 || E.mouth_off + E.mouth_n > D->n_anchors)))
       return fail(SGB_ERR_INVALID, "envelope %d: mouthAnchors range outside the anchor pool", e);
     if (E.tracks_given < 0 || E.tracks_given > 3) return fail(SGB_ERR_INVALID, "envelope %d: tracks_given", e);
     if (E.tracks_given == 2) {
@@ -482,8 +481,8 @@ int sgb_batch_upload(sgb_batch *b, const sgb_batch_desc *D) {
         if (E.tracks_given == 1 && E.nc_fixed > 0 && R.n < E.nc_fixed)
           return fail(SGB_ERR_INVALID, "envelope %d: formant %d has %d track rows for %d columns", e, f, R.n, E.nc_fixed);
       }
-      if (E.tracks_given == 0 && np > 1 && (double)np + std::exp2(E.smoothLinearFactor) > (double)ENV_MAXK_HOST)
-        return fail(SGB_ERR_UNSUPPORTED, "envelope %d: %d formant time points (+ 2^smoothLinearFactor) exceed the %d knots supported", e, np, ENV_MAXK_HOST);
+      if (E.tracks_given == 0 && np > 1 && !(E.smoothLinearFactor <= 20.0))    // 2^20 knots per track
+        return fail(SGB_ERR_UNSUPPORTED, "envelope %d: smoothLinearFactor above 20", e);
     }
   }
   for (int f = 0; f < D->n_formant_refs; f++) {
@@ -550,9 +549,31 @@ int sgb_batch_upload(sgb_batch *b, const sgb_batch_desc *D) {
   b->gc_total = g; b->h_total = h;
   if ((rc = upload_array(b, b->d_gc_off, gc_off.data(), 8 * (size_t)(S + 1)))) return rc;
   if ((rc = upload_array(b, b->d_h_off, h_off.data(), 8 * (size_t)(S + 1)))) return rc;
+  // the contour knot pool (contour.cuh): per syllable its pitch and two amplitude contours, then per noise its
+  // strength contour, then per bout amplAnchorsGlobal; each contour of n anchors owns 5 n doubles
+  const int NN = D->n_noises, NB = D->n_bouts;
+  std::vector<int64_t> koff((size_t)3 * S + NN + NB);
+  int64_t kt = 0;
+  b->any_aglobal = false;
+  for (int s = 0; s < S; s++) {
+    const sgb_syllable &Y = b->syls[s];
+    const int na[3] = {Y.kind == 1 ? Y.pitch_anchor_n : 0, Y.kind == 1 ? Y.ampl_n : 0, Y.kind == 1 ? Y.ampl_n : 0};
+    for (int r = 0; r < 3; r++) { koff[3 * (size_t)s + r] = kt; kt += contour_knot_doubles(na[r]); }
+  }
+  for (int n = 0; n < NN; n++) {
+    koff[3 * (size_t)S + n] = kt;
+    if (D->noises[n].strength_pre_off < 0) kt += contour_knot_doubles(D->noises[n].anchor_n);
+  }
+  for (int i = 0; i < NB; i++) {
+    koff[3 * (size_t)S + NN + i] = kt;
+    kt += contour_knot_doubles(D->bouts[i].aglobal_n);
+    if (D->bouts[i].aglobal_n > 0) b->any_aglobal = true;
+  }
+  b->knot_total = kt;
+  if ((rc = upload_array(b, b->d_koff, koff.data(), 8 * koff.size()))) return rc;
   CK(cudaEventRecord(b->ev[SGB_T_COUNT + 1], b->st));
   b->where = 10;
-  CK(wait_stream(b));   // gc_off / h_off are stack vectors
+  CK(wait_stream(b));   // gc_off / h_off / koff are stack vectors
   b->where = 0;
   CK(cudaEventElapsedTime(&b->info.ms[SGB_T_H2D], b->ev[SGB_T_COUNT], b->ev[SGB_T_COUNT + 1]));
 
@@ -574,6 +595,12 @@ int sgb_batch_upload(sgb_batch *b, const sgb_batch_desc *D) {
   P.pc = b->p_pc.as<double>();
   P.gc_off = b->d_gc_off.as<int64_t>();
   P.h_off = b->d_h_off.as<int64_t>();
+  CK(b->d_knots.ensure(8 * (size_t)std::max<int64_t>(b->knot_total, 1)));
+  CK(b->d_ctab.ensure(contour_tab_bytes() * 3 * (size_t)S));
+  CK(b->d_btabs.ensure(contour_tab_bytes() * (size_t)D->n_bouts));
+  P.ctab = b->d_ctab.as<ContourTab>();
+  P.knots = b->d_knots.as<double>();
+  P.koff = b->d_koff.as<int64_t>();
   CK(b->d_ctrl.ensure(sizeof(SylCtrl) * (size_t)S));
   CK(b->d_lay.ensure(sizeof(SylLayout) * (size_t)S));
   CK(b->d_totals.ensure(64));
@@ -624,8 +651,25 @@ static bool contour_fits(int na, int method, int len, double samplingRate, bool 
                          double hi, const double *an) {
   if (na < 3 || na > 10 || method != SGB_CONTOUR_LOESS || len < 1) return true;
   ContourTab T;
-  contour_prepare(&T, an, na, len, samplingRate, has_lo, lo, has_hi, hi, false, method);
+  double K[5 * 10];
+  contour_prepare(&T, K, an, na, len, samplingRate, has_lo, lo, has_hi, hi, false, method);
   return T.status == SGB_OK;
+}
+
+// Places an envelope instance's contour knots in the envelope knot pool from doubles `at` on: the mouth-opening
+// contour's knots, then per moving formant track (3 per formant) the scratch of k_env_tracks: the nPoints time
+// points and values and the 5 arrays of the na = nPoints + 2^smoothLinearFactor knots of approx().  Returns the end.
+static int64_t env_knot_layout(EnvInst &I, const sgb_envelope &E, const sgb_formant_ref *refs, int64_t at) {
+  I.mouth_koff = -1; I.fit_off = -1;
+  if (E.mouth_n > 0) { I.mouth_koff = at; at += contour_knot_doubles(E.mouth_n); }
+  if (I.trk_off >= 0 && E.tracks_given == 0) {
+    int np = 0;
+    for (int f = 0; f < E.n_formants; f++) np = std::max(np, (int)refs[E.formant_off + f].n);
+    const int64_t na = (int64_t)std::ceil((double)np + std::exp2(E.smoothLinearFactor)) + 1;  // + 1: exp2 on the device
+    I.fit_off = at;
+    at += 3 * (int64_t)E.n_formants * (2 * (int64_t)np + 5 * na);
+  }
+  return at;
 }
 
 // FFT plans + twiddle / window tables (seewave hamming.w / hanning.w, seewave.r:7431-7450)
@@ -763,7 +807,7 @@ int sgb_batch_run_begin(sgb_batch *b) {
   launch_control(d_syl, S, b->ctrl_dense, b->d_order.as<int32_t>(), b->d_pitch.as<double>(), b->d_anchors.as<double>(), b->d_z.as<double>(), P, d_ctrl, d_lay,
                  d_tot, st);
   CKL("launch_control");
-  launches += 2;
+  launches += 3;
   CK(b->h_tot.ensure(64));
   CK(b->h_summary.ensure(sizeof(SylSummary) * (size_t)S));
   CK(b->h_lay.ensure(sizeof(SylLayout) * (size_t)S));
@@ -1076,7 +1120,7 @@ int sgb_batch_run_finish(sgb_batch *b, sgb_run_info *info_out) {
   const int64_t tw_total = (int64_t)tw_host.size(), win_total = (int64_t)win_host.size();
   // ---- upload layout ----
   int max_nc = 0;   // total (instance, column) work items of K4: the kernel runs one CTA per item
-  int64_t trk_total = 0;
+  int64_t trk_total = 0, envk_total = 0;
   for (auto &I : envinst) {
     I.col0 = max_nc; max_nc += I.nc;
     const sgb_envelope &E = b->envs[I.env_id];
@@ -1084,8 +1128,10 @@ int sgb_batch_run_finish(sgb_batch *b, sgb_run_info *info_out) {
     if (E.tracks_given == 0)
       for (int f = 0; f < E.n_formants; f++) if (b->frefs[E.formant_off + f].n > 1) moving = true;
     if (moving) { I.trk_off = trk_total; trk_total += (int64_t)I.nc * E.n_formants * 3; }
+    envk_total = env_knot_layout(I, E, b->frefs.data(), envk_total);
   }
   CK(b->d_trk.ensure(8 * (size_t)std::max<int64_t>(trk_total, 1)));
+  CK(b->d_envk.ensure(8 * (size_t)std::max<int64_t>(envk_total, 1)));
   CK(b->d_mouth.ensure(8 * (size_t)std::max(max_nc, 1)));
   CK(b->d_bl.ensure(sizeof(BoutLayout) * (size_t)NB));
   CK(b->d_place.ensure(sizeof(SylPlace) * (size_t)S));
@@ -1142,7 +1188,7 @@ int sgb_batch_run_finish(sgb_batch *b, sgb_run_info *info_out) {
   CK(b->d_mtabs.ensure(contour_tab_bytes() * std::max<size_t>(envinst.size(), 1)));
   launch_env_tracks(b->d_envinst.as<EnvInst>(), (int)envinst.size(), b->d_envs.as<sgb_envelope>(),
                     b->d_frefs.as<sgb_formant_ref>(), b->d_formants.as<double>(), b->d_anchors.as<double>(),
-                    b->d_trk.as<double>(), b->d_mouth.as<double>(), b->d_mtabs.p, st);
+                    b->d_trk.as<double>(), b->d_mouth.as<double>(), b->d_mtabs.p, b->d_envk.as<double>(), st);
   CKL("launch_env_tracks");
   launch_envelope_f32(b->d_envinst.as<EnvInst>(), (int)envinst.size(), max_nc, b->d_envs.as<sgb_envelope>(),
                       b->d_frefs.as<sgb_formant_ref>(), b->d_formants.as<double>(), b->d_formants_late.as<double>(), b->d_trk.as<double>(),
@@ -1166,7 +1212,8 @@ int sgb_batch_run_finish(sgb_batch *b, sgb_run_info *info_out) {
     CK(b->d_ntabs.ensure(contour_tab_bytes() * (size_t)NN));
     launch_noise_final(b->d_noises.as<sgb_noise>(), NN, b->d_nl.as<NoiseLayout>(), b->d_anchors.as<double>(),
                        b->d_pre.as<double>(), b->d_max.as<int>(), NB, b->d_noise_raw.as<float>(),
-                       b->d_noise_fin.as<float>(), b->d_ntabs.p, 16, st);
+                       b->d_noise_fin.as<float>(), b->d_ntabs.p, b->d_knots.as<double>(),
+                       b->d_koff.as<int64_t>() + 3 * (size_t)S, 16, st);
     CKL("launch_noise_final");
     launches += 1;
   }
@@ -1174,9 +1221,10 @@ int sgb_batch_run_finish(sgb_batch *b, sgb_run_info *info_out) {
   // ---- sound = voiced + breathing, global envelope ----
   launch_sound_mix(b->d_bouts.as<sgb_bout>(), NB, b->d_bl.as<BoutLayout>(), b->d_noises.as<sgb_noise>(),
                    b->d_nl.as<NoiseLayout>(), b->d_anchors.as<double>(), b->d_noise_fin.as<float>(),
-                   b->d_sound.as<float>(), chunks, st);
+                   b->d_sound.as<float>(), b->d_btabs.p, b->d_knots.as<double>(), b->d_koff.as<int64_t>() + 3 * (size_t)S + NN,
+                   b->any_aglobal, chunks, st);
   CKL("launch_sound_mix");
-  launches++;
+  launches += b->any_aglobal ? 2 : 1;
   CK(cudaEventRecord(ev[8], st)); trace_mark(b, 8);
   // ---- K2 filter ----
   for (auto &gr : fgroups) {
@@ -1538,14 +1586,13 @@ int sgb_get_spectral_envelope(int32_t nr, int32_t nc, const sgb_envelope *env, c
   int np = 0;
   if (!E.tracks_given) for (int f = 0; f < E.n_formants; f++) np = std::max(np, (int)refs[f].n);
   if (np > 1) {
-    if ((double)np + std::exp2(E.smoothLinearFactor) > (double)ENV_MAXK_HOST)
-      return fail(SGB_ERR_UNSUPPORTED, "%d formant time points (+ 2^smoothLinearFactor) exceed the %d knots supported", np, ENV_MAXK_HOST);
+    if (!(E.smoothLinearFactor <= 20.0)) return fail(SGB_ERR_UNSUPPORTED, "smoothLinearFactor above 20");
     I.trk_off = 0;
   }
-  if (E.mouth_n > ENV_MAXK_HOST) return fail(SGB_ERR_UNSUPPORTED, "more than %d mouth anchors", ENV_MAXK_HOST);
+  const int64_t env_knots = env_knot_layout(I, E, refs.data(), 0);
   if (E.mouth_n > 0 && !contour_fits(E.mouth_n, E.mouth_method, nc, 16000.0, true, 0.0, true, 1.0, mouth_anchors))
     return fail(SGB_ERR_SYNTH, "loess: span is too small (mouthAnchors)");
-  DBuf dE, dR, dF, dA, dI, dO, dT, dM;
+  DBuf dE, dR, dF, dA, dI, dO, dT, dM, dTab, dK;
   auto run = [&]() -> int {
     CK(dE.ensure(sizeof E)); CK(dR.ensure(sizeof(sgb_formant_ref) * refs.size())); CK(dF.ensure(32 * (size_t)std::max<int64_t>(rows, 1)));
     CK(dA.ensure(16 * (size_t)std::max(1, E.mouth_n))); CK(dI.ensure(sizeof I)); CK(dO.ensure(8 * (size_t)nr * nc));
@@ -1555,10 +1602,9 @@ int sgb_get_spectral_envelope(int32_t nr, int32_t nc, const sgb_envelope *env, c
     if (E.mouth_n) CK(cudaMemcpy(dA.p, mouth_anchors, 16 * (size_t)E.mouth_n, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(dI.p, &I, sizeof I, cudaMemcpyHostToDevice));
     CK(dT.ensure(8 * (size_t)std::max(1, nc * E.n_formants * 3))); CK(dM.ensure(8 * (size_t)nc));
-    DBuf dTab;
-    CK(dTab.ensure(contour_tab_bytes()));
+    CK(dTab.ensure(contour_tab_bytes())); CK(dK.ensure(8 * (size_t)std::max<int64_t>(env_knots, 1)));
     launch_env_tracks(dI.as<EnvInst>(), 1, dE.as<sgb_envelope>(), dR.as<sgb_formant_ref>(), dF.as<double>(),
-                      dA.as<double>(), dT.as<double>(), dM.as<double>(), dTab.p, 0);
+                      dA.as<double>(), dT.as<double>(), dM.as<double>(), dTab.p, dK.as<double>(), 0);
     CKL("launch_env_tracks");
     launch_envelope_f64(dI.as<EnvInst>(), 1, nc, dE.as<sgb_envelope>(), dR.as<sgb_formant_ref>(), dF.as<double>(),
                         nullptr, dT.as<double>(), dM.as<double>(), nullptr, dO.as<double>(), 0);
@@ -1568,6 +1614,7 @@ int sgb_get_spectral_envelope(int32_t nr, int32_t nc, const sgb_envelope *env, c
   };
   int rc = run();
   dE.release(); dR.release(); dF.release(); dA.release(); dI.release(); dO.release(); dT.release(); dM.release();
+  dTab.release(); dK.release();
   return rc;
 }
 

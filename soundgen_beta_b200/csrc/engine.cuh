@@ -19,6 +19,11 @@ struct Pools {
   double *pc;              // [6 * cap] per spline piece: knot, quartic phase polynomial (K1)
   const int64_t *gc_off;   // [S+1] prefix of (cap+1)
   const int64_t *h_off;    // [S+1] prefix of hcap
+  // per syllable three contours, index 3 s + role: 0 the pitch, 1 the amplitude envelope over the glottal cycles
+  // (K0), 2 the amplitude envelope over the composed syllable (K6); they differ in their ceiling
+  ContourTab *ctab;        // [3 S] headers (k_syl_contours)
+  double *knots;           // the batch's knot pool (contour.cuh)
+  const int64_t *koff;     // [3 S + noises + bouts] first knot of each contour in the pool
 };
 
 __device__ inline SylArrays make_arrays(const Pools &P, const sgb_syllable &sp, int s) {
@@ -104,6 +109,8 @@ struct EnvInst {
   int32_t nc;
   int32_t col0;         // first column of this instance in the flat (instance, column) work list
   int64_t trk_off;      // doubles into the formant-track scratch (nc x F x 3), -1: formants do not move
+  int64_t mouth_koff;   // doubles into the envelope knot pool: the mouth-opening contour's knots, -1 none
+  int64_t fit_off;      // doubles into the envelope knot pool: per moving track 2 nPoints + 5 na (k_env_tracks)
 };
 
 

@@ -535,9 +535,11 @@ static int build_call(const sgb_frontend *fe, const sgb_soundgen_args *args, Cal
       std::vector<double> an;
       for (int i = 0; i < C.pitchAnchorsGlobal.n(); i++) { an.push_back(C.pitchAnchorsGlobal.t[i]); an.push_back(C.pitchAnchorsGlobal.v[i]); }
       ContourTab T;
-      contour_prepare(&T, an.data(), C.pitchAnchorsGlobal.n(), C.nSyl, 16000.0, false, 0, false, 0, false, SGB_CONTOUR_SPLINE);
-      if (T.status != SGB_OK) { return ffail(T.status, "pitchAnchorsGlobal: too many anchors"); }
-      for (int s = 0; s < C.nSyl; s++) C.pitchDeltas[s] = std::pow(2.0, contour_eval(&T, C.nSyl, s) / 12);
+      std::vector<double> K((size_t)contour_knot_doubles(C.pitchAnchorsGlobal.n()));
+      contour_prepare(&T, K.data(), an.data(), C.pitchAnchorsGlobal.n(), C.nSyl, 16000.0, false, 0, false, 0, false,
+                      SGB_CONTOUR_SPLINE);
+      if (T.status != SGB_OK) { return ffail(T.status, "pitchAnchorsGlobal: no anchors"); }
+      for (int s = 0; s < C.nSyl; s++) C.pitchDeltas[s] = std::pow(2.0, contour_eval(&T, K.data(), C.nSyl, s) / 12);
     }
   }
   // ---- pitchAnchors$time to 0..1 (:465-472) ----
@@ -776,12 +778,13 @@ bool emit_bout(sgb_frontend *fe, int ci, int b) {
         std::vector<double> an;
         for (int i = 0; i < pitchA.n(); i++) { an.push_back(pitchA.t[i]); an.push_back(pitchA.v[i]); }
         ContourTab Tb;
-        contour_prepare(&Tb, an.data(), pitchA.n(), y.pitch_len, a.pitchSamplingRate, true, a.pitchFloor, true,
+        std::vector<double> Kb((size_t)contour_knot_doubles(pitchA.n()));
+        contour_prepare(&Tb, Kb.data(), an.data(), pitchA.n(), y.pitch_len, a.pitchSamplingRate, true, a.pitchFloor, true,
                         a.pitchCeiling, true, a.contour_method);
         if (Tb.status != SGB_OK) { C.status = Tb.status; y.kind = 0; y.silent_len = 0; R.syls.push_back(y); R.syl_z_drawn.push_back(0); R.syl_call.push_back(ci); continue; }
         R.pitch.resize(R.pitch.size() + y.pitch_len);
         double *pc = R.pitch.data() + y.pitch_off;
-        for (int i = 0; i < y.pitch_len; i++) pc[i] = contour_eval(&Tb, y.pitch_len, i) * C.pitchDeltas[s];
+        for (int i = 0; i < y.pitch_len; i++) pc[i] = contour_eval(&Tb, Kb.data(), y.pitch_len, i) * C.pitchDeltas[s];
         y.pitch_anchor_n = 0;             // the device reads the contour the host evaluated
         if (C.use_rng && draws) {
           int nGC = 0;
@@ -1167,14 +1170,14 @@ int sgb_smooth_contour(const double *time, const double *value, int32_t n, int32
                        int32_t has_floor, double valueFloor, int32_t has_ceiling, double valueCeiling,
                        int32_t thisIsPitch, int32_t method, double *out) {
   if (!value || !out || n < 1 || len < 1) return ffail(SGB_ERR_INVALID, "bad argument");
-  if (n > ENV_MAXK) return ffail(SGB_ERR_UNSUPPORTED, "more than %d anchors", ENV_MAXK);
   std::vector<double> an(2 * (size_t)n);
   for (int i = 0; i < n; i++) { an[2 * i] = time ? time[i] : r_seq_at(0.0, 1.0, n, i); an[2 * i + 1] = value[i]; }
   ContourTab T;
-  contour_prepare(&T, an.data(), n, len, samplingRate, has_floor != 0, valueFloor, has_ceiling != 0, valueCeiling,
+  std::vector<double> K((size_t)contour_knot_doubles(n));
+  contour_prepare(&T, K.data(), an.data(), n, len, samplingRate, has_floor != 0, valueFloor, has_ceiling != 0, valueCeiling,
                   thisIsPitch != 0, method);
   if (T.status != SGB_OK) return ffail(T.status, "getSmoothContour: loess() stops (span is too small)");
-  for (int k = 0; k < len; k++) out[k] = contour_eval(&T, len, k);
+  for (int k = 0; k < len; k++) out[k] = contour_eval(&T, K.data(), len, k);
   return SGB_OK;
 }
 

@@ -104,6 +104,12 @@ __device__ __forceinline__ int sign3(float v, float tol) {
   return (fabsf(v) >= tol) ? (v > 0.0f ? 1 : -1) : 0;
 }
 
+// the loess fit of the amplitude envelope (3-10 anchors) for the composed length, kept out of line: one thread runs
+// it, and inlined it would take registers from the cross-fade loops
+__device__ __noinline__ void compose_ampl_fit(ContourTab *T, const double *K, int len, double samplingRate) {
+  contour_fit_len(T, K, len, samplingRate);
+}
+
 #ifndef COMPOSE_MIN_CTAS
 #define COMPOSE_MIN_CTAS 4     // one CTA per syllable, bound by memory latency: four resident CTAs (64 registers, some spills) beat two (cfg3: 2.9 -> 2.0 ms)
 #endif
@@ -273,19 +279,21 @@ k_compose(const sgb_syllable *__restrict__ syl, int S, SylCtrl *__restrict__ ctr
   // ---- amplitude envelope (source.R:436-448) ----
   if (C.use_ampl) {
     // getSmoothContour(amplAnchors, len = length(waveform), valueFloor = 0, samplingRate): no ceiling
+    // (prepared by k_syl_contours; a loess fit depends on the length and is done here)
     __shared__ ContourTab T;
-    if (threadIdx.x == 0)
-      contour_prepare(&T, anchors + 2 * sp.ampl_off, sp.ampl_n, Lc, sp.samplingRate, true, 0.0, false, 0.0, false,
-                      sp.ampl_method);
+    __shared__ double win[5 * CONTOUR_WIN];
+    __shared__ int wi[3];
+    const double *K = P.knots + P.koff[3 * s + 2];
+    contour_tab_load(&T, P.ctab + 3 * s + 2);
+    __syncthreads();
+    if (threadIdx.x == 0) compose_ampl_fit(&T, K, Lc, sp.samplingRate);
     __syncthreads();
     if (T.status != SGB_OK) {
       if (threadIdx.x == 0) { C.status = T.status; C.out_len = 0; C.raw_max = 1.0; }
       return;
     }
-    for (int k = threadIdx.x; k < Lc; k += blockDim.x) {
-      double v = contour_eval(&T, Lc, k);
-      comp[k] = (float)((double)comp[k] * exp2(v / 10.0));
-    }
+    contour_eval_run(T, K, win, wi, Lc, 0, Lc,
+                     [&](int k, double v) { comp[k] = (float)((double)comp[k] * exp2(v / 10.0)); });
     __syncthreads();
   }
 

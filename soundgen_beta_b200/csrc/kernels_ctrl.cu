@@ -1,6 +1,28 @@
 // K0 (control-rate prologue), size scan, K1 work list, K3 (amplitude matrices).
 #include "engine.cuh"
 
+// The syllables' contours, one thread each (index 3 s + role, see Pools): the sequential FMM solve (or the sort and
+// loess fit) once per contour, ahead of K0.  The amplitude envelopes' lengths (glottal cycles, composed samples) are
+// only known later: their loess fits (3-10 anchors) are done where they are used, for the length of the use.
+__global__ void k_syl_contours(const sgb_syllable *__restrict__ syl, int S, const double *__restrict__ anchors, Pools P) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= 3 * S) return;
+  const int s = t / 3, role = t - 3 * s;
+  const sgb_syllable &sp = syl[s];
+  if (sp.kind != 1) return;
+  double *K = P.knots + P.koff[t];
+  if (role == 0) {
+    if (sp.pitch_anchor_n > 0)
+      contour_prepare(P.ctab + t, K, anchors + 2 * sp.pitch_anchor_off, sp.pitch_anchor_n, sp.pitch_len,
+                      sp.pitchSamplingRate, true, sp.pitchFloor, true, sp.pitchCeiling, true, sp.pitch_method);
+  } else if (sp.ampl_n > 0) {
+    // getSmoothContour(amplAnchors, valueFloor = 0, samplingRate): K0 adds valueCeiling = -throwaway (source.R:221-235),
+    // K6 passes no ceiling (source.R:436-448)
+    contour_prepare(P.ctab + t, K, anchors + 2 * sp.ampl_off, sp.ampl_n, 0, sp.samplingRate, true, 0.0, role == 1,
+                    -sp.throwaway, false, sp.ampl_method);
+  }
+}
+
 // One CTA per syllable.  Parallel: vibrato, column maxima, row pruning.
 // Sequential (thread 0): glottal cycles, random walks, jitter, drift, epochs,
 // upsampling knots -- R/source.R:206-385.
@@ -30,11 +52,12 @@ k_control(const sgb_syllable *syl, int S, const int32_t *__restrict__ order, con
   SylArrays A = make_arrays(P, sp, s);
   if (sp.pitch_anchor_n > 0) {
     // pitchContour_syl = getSmoothContour(pitchAnchors, len, samplingRate = pitchSamplingRate, pitchFloor,
-    //                                     pitchCeiling, thisIsPitch = TRUE) * pitchDeltas[s]  (soundgen.R:596-603)
+    //                                     pitchCeiling, thisIsPitch = TRUE) * pitchDeltas[s]  (soundgen.R:596-603),
+    // prepared by k_syl_contours
     __shared__ ContourTab T;
-    if (threadIdx.x == 0)
-      contour_prepare(&T, anchors + 2 * sp.pitch_anchor_off, sp.pitch_anchor_n, sp.pitch_len, sp.pitchSamplingRate,
-                      true, sp.pitchFloor, true, sp.pitchCeiling, true, sp.pitch_method);
+    __shared__ double win[5 * CONTOUR_WIN];
+    __shared__ int wi[3];
+    contour_tab_load(&T, P.ctab + 3 * s);
     __syncthreads();
     if (T.status != SGB_OK) {
       if (threadIdx.x == 0) {
@@ -43,15 +66,15 @@ k_control(const sgb_syllable *syl, int S, const int32_t *__restrict__ order, con
       }
       return;
     }
-    for (int i = threadIdx.x; i < sp.pitch_len; i += blockDim.x)
-      A.pitch[i] = ctrl_vibrato(sp, i + 1, contour_eval(&T, sp.pitch_len, i) * sp.pitch_scale);
+    contour_eval_run(T, P.knots + P.koff[3 * s], win, wi, sp.pitch_len, 0, sp.pitch_len,
+                     [&](int i, double v) { A.pitch[i] = ctrl_vibrato(sp, i + 1, v * sp.pitch_scale); });
   } else {
     const double *pin = pitch + sp.pitch_off;
     for (int i = threadIdx.x; i < sp.pitch_len; i += blockDim.x) A.pitch[i] = ctrl_vibrato(sp, i + 1, pin[i]);
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    ctrl_sequential(sp, anchors, z, A, C);
+    ctrl_sequential(sp, anchors, P.ctab + 3 * s + 1, P.knots + P.koff[3 * s + 1], z, A, C);
     sh_status = C.status;
   }
   __syncthreads();
@@ -439,6 +462,7 @@ void synth_min_rows_set(int v) { g_tc_min_rows = v; }
 int synth_min_rows() { return g_tc_min_rows; }
 void launch_control(const sgb_syllable *syl, int S, bool dense, const int32_t *order, const double *pitch, const double *anchors, const double *z,
                     const Pools &P, SylCtrl *ctrl, SylLayout *lay, int64_t *totals, cudaStream_t st) {
+  k_syl_contours<<<(3 * S + 127) / 128, 128, 0, st>>>(syl, S, anchors, P);
   if (dense) k_control<32><<<S, CTRL_THREADS, 0, st>>>(syl, S, order, pitch, anchors, z, P, ctrl, g_tc_min_rows);
   else k_control<16><<<S, CTRL_THREADS, 0, st>>>(syl, S, order, pitch, anchors, z, P, ctrl, g_tc_min_rows);
   k_scan_sizes<<<1, 1024, 0, st>>>(ctrl, S, lay, totals);

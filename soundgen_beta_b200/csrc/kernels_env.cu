@@ -8,7 +8,6 @@
 #define ENV_THREADS 128
 #define ENV_WARPS (ENV_THREADS / 32)
 #define ENV_MAXF 64        // formants per filter (incl. stochastic extras and the nasal pole / zero)
-#define ENV_MAXK 64        // knots after the approx() pre-smoothing
 
 template <typename OutT>
 __global__ void __launch_bounds__(ENV_THREADS, 6)
@@ -161,7 +160,8 @@ k_envelope(const EnvInst *__restrict__ inst, const sgb_envelope *__restrict__ en
 // The mouth-opening contour's fit (a loess fit is a millisecond of FP64 on one thread): one thread per instance
 // here, instead of thread 0 of every 128-thread CTA of k_env_tracks while the other 127 wait.
 __global__ void k_mouth_tabs(const EnvInst *__restrict__ inst, int n_inst, const sgb_envelope *__restrict__ envs,
-                             const double *__restrict__ anchors, ContourTab *__restrict__ tabs) {
+                             const double *__restrict__ anchors, ContourTab *__restrict__ tabs,
+                             double *__restrict__ knots) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_inst) return;
   const EnvInst I = inst[i];
@@ -169,57 +169,67 @@ __global__ void k_mouth_tabs(const EnvInst *__restrict__ inst, int n_inst, const
   if (E.mouth_n > 0 && E.n_formants > 0 && E.tracks_given != 2) {
     // getSmoothContour(len = nc, mouthAnchors, valueFloor = 0, valueCeiling = 1): samplingRate is
     // not passed, so the span heuristic sees getSmoothContour's own default of 16000
-    contour_prepare(&tabs[i], anchors + 2 * E.mouth_off, E.mouth_n, I.nc, 16000.0, true, 0.0, true, 1.0, false,
-                    E.mouth_method);       // a failing fit is reported by the host (contour_fits)
+    contour_prepare(&tabs[i], knots + I.mouth_koff, anchors + 2 * E.mouth_off, E.mouth_n, I.nc, 16000.0, true, 0.0,
+                    true, 1.0, false, E.mouth_method);       // a failing fit is reported by the host (contour_fits)
   }
 }
 
+// knots: the envelope knot pool, written here (the mouth knots by k_mouth_tabs, the tracks' scratch below): plain
+// loads, not the read-only path
 __global__ void __launch_bounds__(ENV_THREADS)
 k_env_tracks(const EnvInst *__restrict__ inst, const sgb_envelope *__restrict__ envs,
              const sgb_formant_ref *__restrict__ fidx, const double *__restrict__ formants,
-             const ContourTab *__restrict__ tabs, double *__restrict__ trk, double *__restrict__ mouth) {
+             const ContourTab *__restrict__ tabs, double *knots, double *__restrict__ trk, double *__restrict__ mouth) {
   const EnvInst I = inst[blockIdx.x];
   const sgb_envelope E = envs[I.env_id];
   const int nc = I.nc, F = E.n_formants;
   __shared__ ContourTab T;
   if (E.mouth_n > 0 && F > 0 && E.tracks_given != 2) {
-    {
-      static_assert(sizeof(ContourTab) % 8 == 0, "ContourTab is copied as doubles");
-      const double *g = reinterpret_cast<const double *>(&tabs[blockIdx.x]);
-      double *d = reinterpret_cast<double *>(&T);
-      for (int i = threadIdx.x; i < (int)(sizeof(ContourTab) / 8); i += blockDim.x) d[i] = g[i];
-    }
+    contour_tab_load(&T, &tabs[blockIdx.x]);
     __syncthreads();
-    for (int c = threadIdx.x; c < nc; c += blockDim.x) mouth[I.col0 + c] = (T.status == SGB_OK) ? contour_eval(&T, nc, c) : 0.5;
+    const double *K = knots + I.mouth_koff;
+    for (int c = threadIdx.x; c < nc; c += blockDim.x) mouth[I.col0 + c] = (T.status == SGB_OK) ? contour_eval(&T, K, nc, c) : 0.5;
   }
   if (I.trk_off < 0 || E.tracks_given) return;
   int nPoints = 0;
   for (int f = 0; f < F; f++) nPoints = max(nPoints, fidx[E.formant_off + f].n);
   const int na = (int)ceil((double)nPoints + exp2(E.smoothLinearFactor));
+  const int64_t per = 2 * (int64_t)nPoints + 5 * (int64_t)na;     // scratch doubles per track
+  // the coefficients: one thread per moving track, sequential FMM solve (tx, ty: the time points; ax, ay: approx())
   for (int t = threadIdx.x; t < 3 * F; t += blockDim.x) {
     const int f = t / 3, j = t % 3;
     const sgb_formant_ref R = fidx[E.formant_off + f];
+    if (R.n <= 1) continue;
     const double *rows = formants + 4 * R.off;
-    double *dst = trk + I.trk_off + (int64_t)f * 3 + j;
-    if (R.n <= 1) {
-      for (int c = 0; c < nc; c++) dst[(int64_t)c * F * 3] = rows[1 + j];
-      continue;
-    }
-    double tx[ENV_MAXK], ty[ENV_MAXK], ax[ENV_MAXK], ay[ENV_MAXK], b[ENV_MAXK], cc[ENV_MAXK], d[ENV_MAXK];
-    const int n = R.n;                                   // n, na <= ENV_MAXK, checked at upload
+    double *tx = knots + I.fit_off + t * per, *ty = tx + nPoints, *ax = ty + nPoints, *ay = ax + na;
+    const int n = R.n;
     for (int i = 0; i < n; i++) { tx[i] = rows[4 * i]; ty[i] = rows[4 * i + 1 + j]; }
     for (int i = 0; i < na; i++) { ax[i] = (double)(i + 1); ay[i] = r_approx_at(n, tx, ty, na, i); }
-    fmm_coef(na, ax, ay, b, cc, d);
-    for (int c = 0; c < nc; c++) dst[(int64_t)c * F * 3] = r_spline_at(na, ax, ay, b, cc, d, nc, c);
+    fmm_coef(na, ax, ay, ay + na, ay + 2 * na, ay + 3 * na);
+  }
+  __syncthreads();
+  // the values: (column, track) pairs across the CTA, in the order of trk
+  for (int64_t q = threadIdx.x; q < (int64_t)nc * 3 * F; q += blockDim.x) {
+    const int c = (int)(q / (3 * F)), t = (int)(q - (int64_t)c * 3 * F);
+    const int f = t / 3, j = t % 3;
+    const sgb_formant_ref R = fidx[E.formant_off + f];
+    double v;
+    if (R.n <= 1) {
+      v = formants[4 * R.off + 1 + j];
+    } else {
+      const double *ax = knots + I.fit_off + t * per + 2 * nPoints, *ay = ax + na;
+      v = r_spline_at(na, ax, ay, ay + na, ay + 2 * na, ay + 3 * na, nc, c);
+    }
+    trk[I.trk_off + q] = v;
   }
 }
 
 void launch_env_tracks(const EnvInst *inst, int n_inst, const sgb_envelope *envs, const sgb_formant_ref *fidx,
                        const double *formants, const double *anchors, double *trk, double *mouth, void *tabs,
-                       cudaStream_t st) {
+                       double *knots, cudaStream_t st) {
   if (n_inst <= 0) return;
-  k_mouth_tabs<<<(n_inst + 31) / 32, 32, 0, st>>>(inst, n_inst, envs, anchors, (ContourTab *)tabs);
-  k_env_tracks<<<n_inst, ENV_THREADS, 0, st>>>(inst, envs, fidx, formants, (const ContourTab *)tabs, trk, mouth);
+  k_mouth_tabs<<<(n_inst + 31) / 32, 32, 0, st>>>(inst, n_inst, envs, anchors, (ContourTab *)tabs, knots);
+  k_env_tracks<<<n_inst, ENV_THREADS, 0, st>>>(inst, envs, fidx, formants, (const ContourTab *)tabs, knots, trk, mouth);
 }
 
 void launch_envelope_f32(const EnvInst *inst, int n_inst, int max_nc, const sgb_envelope *envs,

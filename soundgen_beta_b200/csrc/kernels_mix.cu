@@ -6,24 +6,31 @@
 
 // breathingStrength = getSmoothContour(len, noiseAnchors, floor -120, ceiling 40, samplingRate): the fit (FMM
 // spline or loess: a millisecond of FP64 on one thread) once per noise, one thread each, instead of once per CTA of
-// k_noise_final with 255 threads waiting
+// k_noise_final with 255 threads waiting.  The knots go to the noise's slice of the batch's knot pool.
 __global__ void k_noise_tabs(const sgb_noise *__restrict__ noises, int n_noise, const double *__restrict__ anchors,
-                             ContourTab *__restrict__ tabs) {
+                             ContourTab *__restrict__ tabs, double *__restrict__ knots, const int64_t *__restrict__ koff) {
   const int n = blockIdx.x * blockDim.x + threadIdx.x;
   if (n >= n_noise) return;
   const sgb_noise N = noises[n];
   if (N.strength_pre_off < 0)
-    contour_prepare(&tabs[n], anchors + 2 * N.anchor_off, N.anchor_n, N.len, N.samplingRate, true, -120.0, true, 40.0,
-                    false, N.anchor_method);
+    contour_prepare(&tabs[n], knots + koff[n], anchors + 2 * N.anchor_off, N.anchor_n, N.len, N.samplingRate, true,
+                    -120.0, true, 40.0, false, N.anchor_method);
+}
+
+// [k0, k1): the contiguous share of chunk `part` of `parts` in L points
+__device__ __forceinline__ void chunk_range(int L, int part, int parts, int *k0, int *k1) {
+  const int per = (L + parts - 1) / parts;
+  *k0 = min(L, part * per);
+  *k1 = min(L, *k0 + per);
 }
 
 // generateNoise tail (R/source.R:70-81,125-131):
-// breathing / max(breathing) * 2^(contour/10), then fadeInOut.  grid (noises, chunks).
+// breathing / max(breathing) * 2^(contour/10), then fadeInOut.  grid (noises, chunks): each CTA a contiguous run.
 __global__ void __launch_bounds__(256)
 k_noise_final(const sgb_noise *__restrict__ noises, const NoiseLayout *__restrict__ nl,
-              const ContourTab *__restrict__ tabs, const double *__restrict__ pre,
-              const int *__restrict__ maxpool, int max_base, const float *__restrict__ raw,
-              float *__restrict__ fin) {
+              const ContourTab *__restrict__ tabs, const double *__restrict__ knots, const int64_t *__restrict__ koff,
+              const double *__restrict__ pre, const int *__restrict__ maxpool, int max_base,
+              const float *__restrict__ raw, float *__restrict__ fin) {
   const int n = blockIdx.x;
   const sgb_noise N = noises[n];
   const int L = N.len;
@@ -34,34 +41,50 @@ k_noise_final(const sgb_noise *__restrict__ noises, const NoiseLayout *__restric
   int lf = (int)floor(N.attackLen * N.samplingRate / 1000.0);
   if (lf < 2) lf = 0;
   if (lf > L) lf = L;
-  __shared__ ContourTab T;
-  if (N.strength_pre_off < 0) {
-    static_assert(sizeof(ContourTab) % 8 == 0, "ContourTab is copied as doubles");
-    const double *g = reinterpret_cast<const double *>(&tabs[n]);
-    double *d = reinterpret_cast<double *>(&T);
-    for (int i = threadIdx.x; i < (int)(sizeof(ContourTab) / 8); i += blockDim.x) d[i] = g[i];
-    __syncthreads();
-  }
-  for (int k = blockIdx.y * blockDim.x + threadIdx.x; k < L; k += gridDim.y * blockDim.x) {
-    double c = (N.strength_pre_off >= 0) ? pre[N.strength_pre_off + k] : contour_eval(&T, L, k);
+  auto emit = [&](int k, double c) {
     double v = (double)src[k] * rcp_mx * exp2(c / 10.0);
     if (lf > 0) {
       if (k < lf) v = v * r_seq_at(0.0, 1.0, lf, k);
       if (k >= L - lf) v = v * r_seq_at(0.0, 1.0, lf, (L - 1) - k);
     }
     dst[k] = (float)v;
+  };
+  int k0, k1;
+  chunk_range(L, blockIdx.y, gridDim.y, &k0, &k1);
+  if (N.strength_pre_off >= 0) {
+    for (int k = k0 + threadIdx.x; k < k1; k += blockDim.x) emit(k, pre[N.strength_pre_off + k]);
+    return;
   }
+  __shared__ ContourTab T;
+  __shared__ double win[5 * CONTOUR_WIN];
+  __shared__ int wi[3];
+  contour_tab_load(&T, &tabs[n]);
+  __syncthreads();
+  contour_eval_run(T, knots + koff[n], win, wi, L, k0, k1, emit);
+}
+
+// amplEnvelope = getSmoothContour(amplAnchorsGlobal, len = length(sound), 0, -throwaway, samplingRate), once per
+// bout (one thread each) now that length(sound) is known
+__global__ void k_aglobal_tabs(const sgb_bout *__restrict__ bouts, int n_bouts, const BoutLayout *__restrict__ bl,
+                               const double *__restrict__ anchors, ContourTab *__restrict__ tabs,
+                               double *__restrict__ knots, const int64_t *__restrict__ koff) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= n_bouts) return;
+  const sgb_bout &B = bouts[b];
+  if (B.aglobal_n > 0)
+    contour_prepare(&tabs[b], knots + koff[b], anchors + 2 * B.aglobal_off, B.aglobal_n, bl[b].sound_len,
+                    B.samplingRate, true, 0.0, true, -B.throwaway, false, B.aglobal_method);
 }
 
 // sound = voiced (+ breathing noise added BEFORE filtering, soundgen.R:708-714), then the
 // global amplitude envelope (soundgen.R:721-733).  The voiced syllables are already in
 // place; this pass adds the noises in call order and applies the envelope.
-// grid (chunks, bouts).
+// grid (bouts, chunks): each CTA a contiguous run.
 __global__ void __launch_bounds__(256)
 k_sound_mix(const sgb_bout *__restrict__ bouts, const BoutLayout *__restrict__ bl,
             const sgb_noise *__restrict__ noises, const NoiseLayout *__restrict__ nl,
-            const double *__restrict__ anchors, const float *__restrict__ noise_fin,
-            float *__restrict__ sound) {
+            const ContourTab *__restrict__ tabs, const double *__restrict__ knots, const int64_t *__restrict__ koff,
+            const float *__restrict__ noise_fin, float *__restrict__ sound) {
   const int b = blockIdx.x;
   const sgb_bout B = bouts[b];
   const BoutLayout L = bl[b];
@@ -70,27 +93,28 @@ k_sound_mix(const sgb_bout *__restrict__ bouts, const BoutLayout *__restrict__ b
   bool any_noise = false;
   for (int n = B.noise_begin; n < B.noise_end; n++) if (noises[n].mix == 0) any_noise = true;
   if (!any_noise && !has_env) return;
-  // amplEnvelope = getSmoothContour(amplAnchorsGlobal, len = length(sound), 0, -throwaway, samplingRate)
-  __shared__ ContourTab T;
-  if (has_env) {
-    if (threadIdx.x == 0)
-      contour_prepare(&T, anchors + 2 * B.aglobal_off, B.aglobal_n, L.sound_len, B.samplingRate, true, 0.0, true,
-                      -B.throwaway, false, B.aglobal_method);
-    __syncthreads();
-  }
-  for (int k = blockIdx.y * blockDim.x + threadIdx.x; k < L.sound_len; k += gridDim.y * blockDim.x) {
+  auto mix = [&](int k) {
     float v = snd[k];
     for (int n = B.noise_begin; n < B.noise_end; n++) {
       if (noises[n].mix != 0) continue;
       int64_t rel = (L.sound_off + k) - nl[n].dst_off;
       if (rel >= 0 && rel < noises[n].len) v = v + noise_fin[nl[n].raw_off + rel];
     }
-    if (has_env) {
-      double e = contour_eval(&T, L.sound_len, k);
-      v = (float)((double)v * e);
-    }
-    snd[k] = v;
+    return v;
+  };
+  int k0, k1;
+  chunk_range(L.sound_len, blockIdx.y, gridDim.y, &k0, &k1);
+  if (!has_env) {
+    for (int k = k0 + threadIdx.x; k < k1; k += blockDim.x) snd[k] = mix(k);
+    return;
   }
+  __shared__ ContourTab T;
+  __shared__ double win[5 * CONTOUR_WIN];
+  __shared__ int wi[3];
+  contour_tab_load(&T, &tabs[b]);
+  __syncthreads();
+  contour_eval_run(T, knots + koff[b], win, wi, L.sound_len, k0, k1,
+                   [&](int k, double e) { snd[k] = (float)((double)mix(k) * e); });
 }
 
 // soundFiltered / max, + separately filtered noise (soundgen.R:807-818), AM trill
@@ -147,20 +171,22 @@ k_finalize(const sgb_bout *__restrict__ bouts, const BoutLayout *__restrict__ bl
 
 void launch_noise_final(const sgb_noise *noises, int n_noise, const NoiseLayout *nl, const double *anchors,
                         const double *pre, const int *maxpool, int max_base, const float *raw, float *fin,
-                        void *tabs, int chunks, cudaStream_t st) {
+                        void *tabs, double *knots, const int64_t *koff, int chunks, cudaStream_t st) {
   if (n_noise <= 0) return;
-  k_noise_tabs<<<(n_noise + 31) / 32, 32, 0, st>>>(noises, n_noise, anchors, (ContourTab *)tabs);
+  k_noise_tabs<<<(n_noise + 31) / 32, 32, 0, st>>>(noises, n_noise, anchors, (ContourTab *)tabs, knots, koff);
   dim3 g(n_noise, chunks);
-  k_noise_final<<<g, 256, 0, st>>>(noises, nl, (const ContourTab *)tabs, pre, maxpool, max_base, raw, fin);
+  k_noise_final<<<g, 256, 0, st>>>(noises, nl, (const ContourTab *)tabs, knots, koff, pre, maxpool, max_base, raw, fin);
 }
 size_t contour_tab_bytes() { return sizeof(ContourTab); }
 
 void launch_sound_mix(const sgb_bout *bouts, int n_bouts, const BoutLayout *bl, const sgb_noise *noises,
                       const NoiseLayout *nl, const double *anchors, const float *noise_fin, float *sound,
-                      int chunks, cudaStream_t st) {
+                      void *tabs, double *knots, const int64_t *koff, bool any_env, int chunks, cudaStream_t st) {
   if (n_bouts <= 0) return;
+  if (any_env)
+    k_aglobal_tabs<<<(n_bouts + 31) / 32, 32, 0, st>>>(bouts, n_bouts, bl, anchors, (ContourTab *)tabs, knots, koff);
   dim3 g(n_bouts, chunks);
-  k_sound_mix<<<g, 256, 0, st>>>(bouts, bl, noises, nl, anchors, noise_fin, sound);
+  k_sound_mix<<<g, 256, 0, st>>>(bouts, bl, noises, nl, (const ContourTab *)tabs, knots, koff, noise_fin, sound);
 }
 
 void launch_finalize(int f64, const sgb_bout *bouts, int n_bouts, const BoutLayout *bl,

@@ -113,6 +113,68 @@ def config4(n=65536, seed=0):
     return out
 
 
+def _smooth(r, n, lo, hi, log=False):
+    """n points of a slow random walk (a measured track, say) rescaled into a random sub-range of [lo, hi],
+    log-uniformly when `log`"""
+    w = np.cumsum(r.standard_normal(n))
+    w = np.convolve(np.pad(w, 4, mode='edge'), np.ones(9) / 9, mode='valid')
+    w = (w - w.min()) / max(float(np.ptp(w)), 1e-9)
+    a, b = np.sort(r.uniform(0, 1, 2))
+    f = a + (b - a) * w
+    if log:
+        return np.exp(np.log(lo) + (np.log(hi) - np.log(lo)) * f)
+    return lo + (hi - lo) * f
+
+
+def resynthesis(n=4096, seed=20260005, points=101):
+    """resynthesis from measured tracks: n x 2 s at 22.05 kHz, temperature 0, one anchor per 20 ms (`points`)
+    for pitchAnchors (80-600 Hz), amplAnchors, noiseAnchors, mouthAnchors and amplAnchorsGlobal, and 4 formants
+    that move through `points` time points."""
+    r = np.random.default_rng(seed)
+    sr, wl, dur = 22050, 1102, 2000
+    t01 = host.seq_len(0, 1, points)
+    out = []
+    for i in range(n):
+        tms = t01 * dur
+        ulen = int(np.rint((tms[-1] - tms[0]) * sr / 1000))
+        fm = []
+        for f0 in np.sort(r.uniform(400, 4500, 4)):
+            fm.append(np.column_stack([t01, _smooth(r, points, 0.8 * f0, 1.25 * f0), _smooth(r, points, 20, 50),
+                                       _smooth(r, points, 80, 300)]))
+        out.append(dict(
+            sylLen=dur, samplingRate=sr, temperature=0, nonlinBalance=0, contour_method='spline',
+            pitchAnchors=(t01, _smooth(r, points, 80, 600, log=True)),
+            amplAnchors=(t01, _smooth(r, points, 40, 120)),
+            noiseAnchors=(tms, _smooth(r, points, -60, 10)),
+            mouthAnchors=(t01, _smooth(r, points, 0, 1)),
+            amplAnchorsGlobal=(t01, _smooth(r, points, 60, 120)),
+            formants=fm, rolloffNoise=-8,
+            u=[r.random(noise_uniform_count(ulen, wl))]))
+    return out
+
+
+def thinned(calls, points=60):
+    """the same calls with every contour and formant track resampled (linearly) to `points` points"""
+    def rs(t, v):
+        t = np.asarray(t, dtype=np.float64)
+        tn = host.seq_len(float(t[0]), float(t[-1]), points)
+        return tn, np.interp(tn, t, np.asarray(v, dtype=np.float64))
+    out = []
+    for kw in calls:
+        kw = dict(kw)
+        for k in ('pitchAnchors', 'amplAnchors', 'noiseAnchors', 'mouthAnchors', 'amplAnchorsGlobal'):
+            if k in kw:
+                kw[k] = rs(*kw[k])
+        if 'formants' in kw:
+            fm = []
+            for f in kw['formants']:
+                tn = rs(f[:, 0], f[:, 1])[0]
+                fm.append(np.column_stack([tn] + [rs(f[:, 0], f[:, j])[1] for j in (1, 2, 3)]))
+            kw['formants'] = fm
+        out.append(kw)
+    return out
+
+
 CONFIGS = {0: config0, 1: config1, 2: config2, 3: config3, 4: config4}
 NAMES = {0: 'cfg0 soundgen() defaults, 1 x 1000 ms @ 16 kHz',
          1: 'cfg1 voiced batch, 1024 x 500 ms @ 44.1 kHz',
