@@ -215,6 +215,45 @@ int sgb_batch_fetch_pcm16(sgb_batch *b, int16_t *out, int64_t n);
 /* Per-call failure flags (0 = ok, else an SGB_ERR_* code). */
 int sgb_batch_status(sgb_batch *b, int32_t *out_status /* n_calls */);
 
+/* Device output: results written straight into caller-owned device memory (for a consumer on the same GPU,
+ * e.g. a model trained with PyTorch), with no trip through host memory.
+ *
+ * Row c is written from element dst_off[c] on: exactly cap[c] elements, the first min(len_c, cap_c) samples of the
+ * row and then zeros (a padded [rows, T] tensor needs no separate clearing pass).  SGB_OUT_F32 copies the samples
+ * bit for bit as sgb_batch_fetch_f32 returns them; SGB_OUT_PCM16 writes the 16-bit PCM of sgb_batch_fetch_pcm16,
+ * normalised over the row's len_c source samples (same kernel, same bits), so cropping keeps the normalisation of
+ * the whole row.
+ *
+ * Stream contract: nothing here waits on the host.  The library records an event on the caller's stream and
+ * makes its own stream wait for it (the destination is free), runs the copy, records an event and makes the
+ * caller's stream wait for that: work the caller queues on `stream` afterwards sees the rows.  Later runs of the
+ * same handle are queued behind the export on the handle's stream, so they cannot overwrite the source first.
+ * `stream` may come from another CUDA runtime in the process (torch's: torch.cuda.Stream.cuda_stream): both use
+ * the device's primary context.
+ *
+ * Every argument is checked before anything is queued (SGB_ERR_INVALID): `dst` must be device (or managed)
+ * memory of the batch's device, aligned to its element type; offsets and capacities non-negative, every row
+ * inside [0, dst_elems), no two rows overlapping.  A handle without a completed run gives SGB_ERR_STATE.
+ * There is no host path: without a device both calls return SGB_ERR_CUDA. */
+#define SGB_OUT_F32    0
+#define SGB_OUT_PCM16  1
+typedef struct sgb_device_out {
+  void          *dst;         /* device memory on the batch's device (float * or int16_t *)       */
+  int64_t        dst_elems;   /* elements available at dst (bounds check)                         */
+  const int64_t *dst_off;     /* host, n: first element of row c in dst                           */
+  const int64_t *cap;         /* host, n: elements written for row c (samples, then zeros)        */
+  int64_t       *out_written; /* host, n (may be NULL): min(len_c, cap_c)                         */
+  void          *stream;      /* caller's cudaStream_t (NULL = the legacy default stream)         */
+  int32_t        format;      /* SGB_OUT_F32 / SGB_OUT_PCM16                                      */
+  int32_t        reserved;
+} sgb_device_out;
+/* Every call of the last run (n = n_calls rows, row c = call c) -> caller-owned device memory. */
+int sgb_batch_export(sgb_batch *b, const sgb_device_out *o);
+/* The same over n float32 rows the caller already holds on `device` (row c = len[c] samples at src + src_off[c]):
+ * used to normalise to PCM16 a call assembled from several rounds, over the whole call. */
+int sgb_rows_export(int32_t device, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
+                    const sgb_device_out *o);
+
 /* Intermediate results (valid after run).  Sizes via the *_len calls. */
 int sgb_batch_syllable_len(sgb_batch *b, int32_t syl, int64_t *out_len);
 int sgb_batch_syllable_fetch(sgb_batch *b, int32_t syl, double *out, int64_t n);
@@ -252,7 +291,8 @@ int sgb_batch_set_tracks(sgb_batch *b, int32_t env, const double *rows, int32_t 
 /* Normal draws each voiced syllable consumed (valid after run_begin); n_syllables values. */
 int sgb_batch_z_used(sgb_batch *b, int32_t *out);
 /* sizeof() of the ABI structs, for bindings to verify their mirrors:
- * syllable, envelope, noise, bout, call, formant_ref, batch_desc, run_info, soundgen_args. */
+ * syllable, envelope, noise, bout, call, formant_ref, batch_desc, run_info, soundgen_args, device_out
+ * (cap >= 9; the 10th is written when cap >= 10). */
 int sgb_abi_sizes(int32_t *out, int32_t cap);
 /* The additive synthesis has two kernels: epochs with at least `rows` rows run on the tensor cores, the others on the
    FP32 pipe (default 224, or SGB_SYNTH / SGB_SYNTH_MIN_ROWS from the environment).  0 = tensor cores only, a huge value =

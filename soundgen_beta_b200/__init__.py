@@ -2,7 +2,8 @@
 reference's own function names.  All compute goes through libsoundgen_b200.so (CUDA,
 sm_100a); importing this package never falls back to a CPU implementation."""
 from .api import (ArgArray, Batch, BatchBuilder, FrontEnd, run_rounds, PipelinedBatches, SoundgenError, filter_sound, generateHarmonics, generateNoise,
-                  getRolloff, getSpectralEnvelope, pin_desc, soundgen, soundgen_batch)
+                  getRolloff, getSpectralEnvelope, pin_desc, rows_export, soundgen, soundgen_batch, soundgen_batch_device)
 
 __all__ = ['ArgArray', 'Batch', 'BatchBuilder', 'FrontEnd', 'run_rounds', 'PipelinedBatches', 'SoundgenError', 'filter_sound', 'generateHarmonics', 'generateNoise',
-           'getRolloff', 'getSpectralEnvelope', 'pin_desc', 'soundgen', 'soundgen_batch']
+           'getRolloff', 'getSpectralEnvelope', 'pin_desc', 'rows_export', 'soundgen', 'soundgen_batch',
+           'soundgen_batch_device']

@@ -10,6 +10,7 @@ SGB_OK = 0
 SGB_ERR_INVALID, SGB_ERR_CUDA, SGB_ERR_UNSUPPORTED = -1, -2, -3
 SGB_ERR_SYNTH, SGB_ERR_STREAM, SGB_ERR_STATE = -4, -5, -6
 SGB_CONTOUR_LOESS, SGB_CONTOUR_SPLINE = 0, 1
+SGB_OUT_F32, SGB_OUT_PCM16 = 0, 1
 
 SYL_DOUBLES = ['attackLen', 'nonlinBalance', 'jitterDep', 'jitterLen', 'vibratoFreq',
                'vibratoDep', 'shimmerDep', 'rolloff', 'rolloffOct', 'rolloffKHz', 'rolloffParab',
@@ -104,6 +105,11 @@ class SoundgenArgs(C.Structure):
                 ('u', C.c_void_p), ('u_len', C.c_void_p), ('n_u', i32), ('reserved1', i32)]
 
 
+class DeviceOut(C.Structure):
+    _fields_ = [('dst', C.c_void_p), ('dst_elems', i64), ('dst_off', C.c_void_p), ('cap', C.c_void_p),
+                ('out_written', C.c_void_p), ('stream', C.c_void_p), ('format', i32), ('reserved', i32)]
+
+
 T_NAMES = ['h2d', 'control', 'ampl', 'synth', 'compose', 'noise', 'assemble', 'envelope',
            'filter', 'finalize', 'd2h', 'total']
 
@@ -124,6 +130,7 @@ EXPORTS = ['sgb_version', 'sgb_last_error', 'sgb_device_count', 'sgb_set_device'
            'sgb_measure_fp32_peak',
            'sgb_batch_create', 'sgb_batch_destroy', 'sgb_batch_upload', 'sgb_batch_run',
            'sgb_batch_lengths', 'sgb_batch_fetch_f32', 'sgb_batch_fetch_f64', 'sgb_batch_fetch_pcm16', 'sgb_batch_status',
+           'sgb_batch_export', 'sgb_rows_export',
            'sgb_batch_syllable_len', 'sgb_batch_syllable_fetch', 'sgb_batch_noise_fetch',
            'sgb_batch_artefacts', 'sgb_batch_artefact_ints', 'sgb_batch_pitch_per_gc', 'sgb_batch_checksums', 'sgb_batch_debug_state',
            'sgb_get_rolloff', 'sgb_get_spectral_envelope', 'sgb_filter_len', 'sgb_filter',
@@ -172,6 +179,8 @@ def load():
     L.sgb_batch_fetch_f64.argtypes = [vp, vp, i64]
     L.sgb_batch_fetch_pcm16.argtypes = [vp, vp, i64]
     L.sgb_batch_status.argtypes = [vp, vp]
+    L.sgb_batch_export.argtypes = [vp, C.POINTER(DeviceOut)]
+    L.sgb_rows_export.argtypes = [i32, vp, vp, vp, i32, C.POINTER(DeviceOut)]
     L.sgb_batch_syllable_len.argtypes = [vp, i32, C.POINTER(i64)]
     L.sgb_batch_syllable_fetch.argtypes = [vp, i32, vp, i64]
     L.sgb_batch_noise_fetch.argtypes = [vp, i32, vp, i64]
@@ -213,9 +222,10 @@ def load():
     L.sgb_frontend_h2d_bytes.restype = i64
     L.sgb_rng_draw.argtypes = [C.c_uint32, i32, f64, f64, i32, vp, i32]
     L.sgb_smooth_contour.argtypes = [vp, vp, i32, i32, f64, i32, f64, i32, f64, i32, i32, vp]
-    sizes = (i32 * 9)()
-    L.sgb_abi_sizes(sizes, 9)
-    mine = [C.sizeof(t) for t in (Syllable, Envelope, Noise, Bout, Call, FormantRef, BatchDesc, RunInfo, SoundgenArgs)]
+    sizes = (i32 * 10)()
+    L.sgb_abi_sizes(sizes, 10)
+    mine = [C.sizeof(t) for t in (Syllable, Envelope, Noise, Bout, Call, FormantRef, BatchDesc, RunInfo, SoundgenArgs,
+                                  DeviceOut)]
     if list(sizes) != mine:
         raise RuntimeError('ctypes mirror out of date: library struct sizes %s, mirror %s' % (list(sizes), mine))
     _lib = L

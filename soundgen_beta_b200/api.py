@@ -659,6 +659,14 @@ class Batch:
         offs = np.concatenate(([0], np.cumsum(lens)))
         return [out[offs[i]:offs[i + 1]] for i in range(lens.size)]
 
+    def export(self, dst, dst_off, cap, stream=None, fmt='f32'):
+        """Writes every call of the last run into the CUDA tensor `dst` (float32 for fmt 'f32', int16 for 'pcm16'):
+        call c fills exactly cap[c] elements from element dst_off[c] of the flattened tensor, its first
+        min(len, cap) samples and then zeros.  Ordered on `stream` (a torch.cuda.Stream or a raw cudaStream_t; default
+        the current stream of dst's device) with no host synchronisation.  Returns the samples written per call."""
+        n = self.desc.n_calls if self.desc is not None else 0
+        return _export(lambda o: self.L.sgb_batch_export(self.h, C.byref(o)), n, dst, dst_off, cap, stream, fmt)
+
     def syllable(self, s):
         n = C.c_int64()
         _check(self.L.sgb_batch_syllable_len(self.h, s, C.byref(n)))
@@ -734,6 +742,136 @@ def soundgen_batch(list_of_kwargs, out_dtype=np.float32, u_dtype=np.float64):
     return outs, st
 
 
+_OUT_FORMATS = {'f32': (_abi.SGB_OUT_F32, 'float32'), 'pcm16': (_abi.SGB_OUT_PCM16, 'int16')}
+
+
+def _stream_handle(stream, dst):
+    import torch
+    if stream is None:
+        return torch.cuda.current_stream(dst.device).cuda_stream if dst.is_cuda else 0
+    return stream.cuda_stream if hasattr(stream, 'cuda_stream') else int(stream)
+
+
+def _export(call, n, dst, dst_off, cap, stream, fmt):
+    """Fills an sgb_device_out for the tensor `dst` and runs `call` on it; the library checks where dst lives."""
+    import torch
+    if fmt not in _OUT_FORMATS:
+        raise ValueError("fmt must be 'f32' or 'pcm16', not %r" % (fmt,))
+    code, tname = _OUT_FORMATS[fmt]
+    if dst.dtype != getattr(torch, tname):
+        raise ValueError('fmt %r writes %s, dst is %s' % (fmt, tname, dst.dtype))
+    if not dst.is_contiguous():
+        raise ValueError('dst must be contiguous')
+    off = np.ascontiguousarray(dst_off, dtype=np.int64)
+    cp = np.ascontiguousarray(cap, dtype=np.int64)
+    if off.shape != (n,) or cp.shape != (n,):
+        raise ValueError('dst_off and cap need one entry per row (%d)' % n)
+    written = np.zeros(n, dtype=np.int64)
+    o = _abi.DeviceOut()
+    o.dst, o.dst_elems = dst.data_ptr() or None, dst.numel()
+    o.dst_off, o.cap, o.out_written = _ptr(off), _ptr(cp), _ptr(written)
+    o.stream = _stream_handle(stream, dst) or None
+    o.format = code
+    _check(call(o))
+    return written
+
+
+def rows_export(device, src, src_off, lens, dst, dst_off, cap, stream=None, fmt='pcm16'):
+    """sgb_rows_export: the export over float32 rows the caller holds in the CUDA tensor `src` (row c = lens[c]
+    samples from element src_off[c]); with fmt 'pcm16' every row is normalised over its lens[c] samples."""
+    so = np.ascontiguousarray(src_off, dtype=np.int64)
+    ln = np.ascontiguousarray(lens, dtype=np.int64)
+    if not src.is_contiguous() or so.shape != ln.shape:
+        raise ValueError('src must be contiguous, src_off and lens of one length')
+    L = _abi.load()
+    return _export(lambda o: L.sgb_rows_export(int(device), src.data_ptr() or None, _ptr(so), _ptr(ln), ln.size,
+                                               C.byref(o)), ln.size, dst, dst_off, cap, stream, fmt)
+
+
+def _torch_out_dtype(dtype):
+    import torch
+    if dtype == torch.float32:
+        return 'f32'
+    if dtype == torch.int16:
+        return 'pcm16'
+    raise ValueError('dtype must be torch.float32 or torch.int16 (PCM16), not %r' % (dtype,))
+
+
+def soundgen_batch_device(calls, dtype=None, device=None, max_len=None, u_dtype=np.float64):
+    """soundgen_batch with the waveforms delivered on the GPU: returns (wave, lengths, status).
+    wave: [n_calls, T] tensor on the device, rows padded with zeros, T = max_len (longer calls are cropped) or else
+    the longest call; lengths: int64 CUDA tensor of the samples present per row; status: as soundgen_batch returns it.
+    dtype: torch.float32 (the samples soundgen() returns) or torch.int16 (16-bit PCM as seewave::savewav writes it,
+    normalised over the whole call, before any cropping).  device: CUDA device index (default: torch's current one).
+    The result is ordered on the device's current torch stream."""
+    import torch
+    fmt = _torch_out_dtype(torch.float32 if dtype is None else dtype)
+    if max_len is not None and int(max_len) < 0:
+        raise ValueError('max_len must be non-negative')
+    L = _abi.load()
+    if isinstance(device, (str, torch.device)):
+        device = torch.device(device).index
+    if device is None:
+        device = torch.cuda.current_device() if torch.cuda.is_available() else 0
+    device = int(device)
+    _check(L.sgb_set_device(device))       # the handles below are made on this thread's current device
+    fe = FrontEnd(u_dtype)
+    rounds = []
+    try:
+        for kw in calls:
+            fe.add(**kw)
+        n = fe.n_calls
+        # one handle per round: the next round would overwrite a handle's output, and T is known after the last one
+        while True:
+            desc, m = fe.round_begin()
+            if m == 0:
+                break
+            bt = Batch()
+            rounds.append(bt)
+            bt.upload(desc)
+            bt.run()
+            bt.round_calls = fe.round_calls().copy()
+            bt.seg_len = bt.lengths()
+        status = fe.status()
+    finally:
+        fe.close()
+    try:
+        total = np.zeros(n, dtype=np.int64)
+        for bt in rounds:
+            np.add.at(total, bt.round_calls, bt.seg_len)
+        T = int(max_len) if max_len is not None else int(total.max(initial=0))
+        dev = torch.device('cuda', device)
+        stream = torch.cuda.current_stream(dev)
+        rows = np.arange(n, dtype=np.int64)
+        last = np.full(n, -1)              # the last round each call took part in
+        for r, bt in enumerate(rounds):
+            last[bt.round_calls] = r
+        if fmt == 'f32':
+            wave = torch.empty((n, T), dtype=torch.float32, device=dev)
+            if np.any(last < 0):           # a call that never reached the device: its row is written by nobody
+                wave.zero_()
+            tgt, base, width = wave, rows * T, np.full(n, T, dtype=np.int64)
+        else:   # whole calls in float32 first (packed): PCM16 is normalised over the whole call
+            wave = torch.empty((n, T), dtype=torch.int16, device=dev)
+            base = (np.cumsum(total) - total).astype(np.int64)
+            tgt, width = torch.empty(int(total.sum()), dtype=torch.float32, device=dev), total
+        # a call's segment of round r lands behind its earlier segments; its last segment also writes the zero tail
+        done = np.zeros(n, dtype=np.int64)
+        for r, bt in enumerate(rounds):
+            ci = bt.round_calls
+            room = np.maximum(width[ci] - done[ci], 0)
+            cap = np.where(last[ci] == r, room, np.minimum(bt.seg_len, room))
+            bt.export(tgt, base[ci] + np.minimum(done[ci], width[ci]), cap, stream, 'f32')
+            done[ci] += bt.seg_len
+        if fmt == 'pcm16':
+            rows_export(device, tgt, base, total, wave, rows * T, np.full(n, T, dtype=np.int64), stream, 'pcm16')
+        lengths = torch.as_tensor(np.minimum(total, T), dtype=torch.int64).to(dev)
+    finally:
+        for bt in rounds:      # destroying a handle waits for its stream, i.e. for the export queued on it
+            bt.close()
+    return wave, lengths, status
+
+
 class PipelinedBatches:
     """Several sub-batches, each with its own handle / CUDA stream, driven as a three-stage software
     pipeline: one thread uploads (H2D copy engine), `runners` threads run the kernels (two, so that the
@@ -742,10 +880,14 @@ class PipelinedBatches:
     engine).  ctypes releases the GIL during the library calls.  Independent sounds need no ordering,
     so no work is skipped and nothing is shared between the sub-batches."""
 
-    def __init__(self, descs=None, runners=2, sources=None, fe_threads=2):
+    def __init__(self, descs=None, runners=2, sources=None, fe_threads=2, device_out=None):
         """`descs`: prebuilt batch descriptions, one per sub-batch -- or `sources`: one `ArgArray` per sub-batch, in
         which case every step starts from the argument lists: `fe_threads` threads run the library's host
-        front-end (`sgb_frontend_add_many` + `round_begin`) for a sub-batch before it is uploaded."""
+        front-end (`sgb_frontend_add_many` + `round_begin`) for a sub-batch before it is uploaded.
+        `device_out`: None (results are fetched to host memory) or dict(dtype=torch.float32 | torch.int16,
+        max_len=None | T, device=None | index): the fetch stage exports every sub-batch into CUDA tensors allocated
+        once, `results[i] = (wave [n_i, T], lengths)`, ordered on `streams[i]` (one consumer stream per sub-batch).
+        A step overwrites the tensors of the step before: consume them on `streams[i]` (or copy them) first."""
         self.sources = list(sources) if sources is not None else None
         if self.sources is not None:
             self.fes = [FrontEnd(src.u_dtype) for src in self.sources]
@@ -757,6 +899,36 @@ class PipelinedBatches:
         self.outs = [None] * len(self.descs)
         self.runners = max(1, int(runners))
         self.results = [None] * len(self.descs)
+        self.device_out = None
+        if device_out is not None:
+            import torch
+            do = dict(device_out)
+            self.device_out = dict(fmt=_torch_out_dtype(do.pop('dtype', torch.float32)), max_len=do.pop('max_len', None),
+                                   device=do.pop('device', None))
+            if do:
+                raise TypeError('device_out: unknown keys %s' % sorted(do))
+            if self.device_out['device'] is None:
+                self.device_out['device'] = torch.cuda.current_device()
+            dev = torch.device('cuda', int(self.device_out['device']))
+            self.streams = [torch.cuda.Stream(dev) for _ in self.descs]
+            self.waves = [None] * len(self.descs)
+
+    def _export(self, i):
+        """device_out: sub-batch i -> its [n_i, T] tensor, ordered on streams[i]"""
+        import torch
+        bt, s, do = self.batches[i], self.streams[i], self.device_out
+        lens = bt.lengths()
+        T = int(do['max_len']) if do['max_len'] is not None else int(lens.max(initial=0))
+        w = self.waves[i]
+        with torch.cuda.stream(s):
+            if w is None or w.shape != (lens.size, T):      # allocated once (again only if a longer call appears)
+                w = torch.empty((lens.size, T), dtype=torch.float32 if do['fmt'] == 'f32' else torch.int16,
+                                device=s.device)
+                self.waves[i] = w
+            n = lens.size
+            bt.export(w, np.arange(n, dtype=np.int64) * T, np.full(n, T, dtype=np.int64), s, do['fmt'])
+            lengths = torch.as_tensor(np.minimum(lens, T), dtype=torch.int64).to(s.device, non_blocking=True)
+        return w, lengths
 
     def _fetch(self, i, dtype):
         bt = self.batches[i]
@@ -862,7 +1034,7 @@ class PipelinedBatches:
                     done += 1
                     continue
                 if transfer:
-                    self.results[i] = self._fetch(i, dtype)
+                    self.results[i] = self._export(i) if self.device_out is not None else self._fetch(i, dtype)
                 free[i].release()
 
         th = [threading.Thread(target=guard(uploader))] + \

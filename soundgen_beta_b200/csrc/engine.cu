@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstring>
 #include <map>
+#include <mutex>
 #include <string>
 #include <vector>
 
@@ -155,6 +156,24 @@ struct HBuf {
   template <typename T> T *as() const { return reinterpret_cast<T *>(p); }
 };
 
+// Staging of the device-output exports (sgb_batch_export / sgb_rows_export): the per-row table and the (row, chunk)
+// grid travel from pinned host memory to the device.  A slot is reused only once the event recorded after its
+// kernel has passed, checked with cudaEventQuery: an export never waits on the host for an earlier one (which may
+// itself still wait on the caller's stream); a new slot is added while all are in flight.
+struct ExportSlot {
+  HBuf h;
+  DBuf d;
+  cudaEvent_t done = nullptr;
+};
+struct ExportCtx {
+  std::vector<ExportSlot *> slots;
+  cudaEvent_t ev_in = nullptr;
+  ~ExportCtx() {
+    for (auto s : slots) { s->h.release(); s->d.release(); if (s->done) cudaEventDestroy(s->done); delete s; }
+    if (ev_in) cudaEventDestroy(ev_in);
+  }
+};
+
 static int64_t align4(int64_t x) { return (x + 3) & ~(int64_t)3; }
 
 // seq(from, to, by) length: floor((to-from)/by + 1e-10) + 1
@@ -217,6 +236,7 @@ struct sgb_batch {
   struct Mark { volatile int *dst; } marks[16];
   bool keep_voiced = false;
   sgb_run_info info;
+  ExportCtx *xo = nullptr;           // device-output staging, made on the first export
 };
 
 // SGB_TRACE=1: a host callback after every stage records how far the stream got, readable without any
@@ -230,37 +250,70 @@ static void trace_mark(sgb_batch *b, int i) {
 
 // 16-bit PCM of every call's waveform as seewave::savewav writes it (soundgen.R:855-857, seewave.r:5192-5229
 // -> tuneR::normalize(unit = "16", level = min(1, max(x))), tuneR normalize.R): centre, scale the largest
-// magnitude to `level`, round(x * 32767).  One CTA per call; reductions in a fixed order (reproducible).
+// magnitude to `level`, round(x * 32767).  One CTA per row (the whole-row reductions come first); reductions in a
+// fixed order (reproducible).  Row r: statistics over its len[r] samples at src + src_off[r]; written: exactly
+// cap[r] elements from dst + dst_off[r], the first min(len, cap) samples and then zeros.  The host fetch passes
+// dst_off = src_off and cap = len.
 __global__ void __launch_bounds__(256)
-k_pcm16(const float *__restrict__ outp, const int64_t *__restrict__ off, const int64_t *__restrict__ len,
-        int16_t *__restrict__ pcm) {
+k_pcm16(const float *__restrict__ src, const int64_t *__restrict__ src_off, const int64_t *__restrict__ len,
+        const int64_t *__restrict__ dst_off, const int64_t *__restrict__ cap, int16_t *__restrict__ dst) {
   __shared__ double rs[8], rm[8], ra[8];
-  const int64_t n = len[blockIdx.x];
-  const float *x = outp + off[blockIdx.x];
-  int16_t *y = pcm + off[blockIdx.x];
-  if (n <= 0) return;
-  double sum = 0.0, mx = -INFINITY;
-  for (int64_t i = threadIdx.x; i < n; i += 256) { double v = (double)x[i]; sum += v; mx = fmax(mx, v); }
-  for (int o = 16; o > 0; o >>= 1) { sum += __shfl_xor_sync(0xffffffffu, sum, o); mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o)); }
-  if ((threadIdx.x & 31) == 0) { rs[threadIdx.x >> 5] = sum; rm[threadIdx.x >> 5] = mx; }
-  __syncthreads();
-  sum = 0.0; mx = -INFINITY;
-  for (int w = 0; w < 8; w++) { sum += rs[w]; mx = fmax(mx, rm[w]); }
-  const double mean = sum / (double)n;
-  double am = 0.0;
-  for (int64_t i = threadIdx.x; i < n; i += 256) am = fmax(am, fabs((double)x[i] - mean));
-  for (int o = 16; o > 0; o >>= 1) am = fmax(am, __shfl_xor_sync(0xffffffffu, am, o));
-  if ((threadIdx.x & 31) == 0) ra[threadIdx.x >> 5] = am;
-  __syncthreads();
-  am = 0.0;
-  for (int w = 0; w < 8; w++) am = fmax(am, ra[w]);
-  const double level = (mx <= 1.0) ? mx : 1.0;
+  const int64_t n = len[blockIdx.x], c = cap[blockIdx.x], m = n < c ? n : c;
+  const float *x = src + src_off[blockIdx.x];
+  int16_t *y = dst + dst_off[blockIdx.x];
+  double mean = 0.0, am = 0.0, level = 0.0;
+  if (n > 0) {                                   // uniform over the CTA
+    double sum = 0.0, mx = -INFINITY;
+    for (int64_t i = threadIdx.x; i < n; i += 256) { double v = (double)x[i]; sum += v; mx = fmax(mx, v); }
+    for (int o = 16; o > 0; o >>= 1) { sum += __shfl_xor_sync(0xffffffffu, sum, o); mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o)); }
+    if ((threadIdx.x & 31) == 0) { rs[threadIdx.x >> 5] = sum; rm[threadIdx.x >> 5] = mx; }
+    __syncthreads();
+    sum = 0.0; mx = -INFINITY;
+    for (int w = 0; w < 8; w++) { sum += rs[w]; mx = fmax(mx, rm[w]); }
+    mean = sum / (double)n;
+    for (int64_t i = threadIdx.x; i < n; i += 256) am = fmax(am, fabs((double)x[i] - mean));
+    for (int o = 16; o > 0; o >>= 1) am = fmax(am, __shfl_xor_sync(0xffffffffu, am, o));
+    if ((threadIdx.x & 31) == 0) ra[threadIdx.x >> 5] = am;
+    __syncthreads();
+    am = 0.0;
+    for (int w = 0; w < 8; w++) am = fmax(am, ra[w]);
+    level = (mx <= 1.0) ? mx : 1.0;
+  }
   const bool scale = fabs(am) > 1.5e-8;          // !isTRUE(all.equal(m, 0))
-  for (int64_t i = threadIdx.x; i < n; i += 256) {
+  for (int64_t i = threadIdx.x; i < m; i += 256) {
     double v = (double)x[i] - mean;
     if (scale) v = level * v / am;
     v = rint(v * 32767.0);
     y[i] = (int16_t)fmin(32767.0, fmax(-32768.0, v));
+  }
+  for (int64_t i = m + threadIdx.x; i < c; i += 256) y[i] = 0;
+}
+
+// Float32 rows into caller-owned device memory.  Rows run from 50 ms to many seconds, so the grid is a host-built
+// table of (row, chunk) pairs, EXPORT_CHUNK elements each, not one CTA per row.  Chunk k of row r writes elements
+// [k * EXPORT_CHUNK, min(cap, (k + 1) * EXPORT_CHUNK)) of the row: the source sample below min(len, cap), else 0.
+// Calls are packed back to back with no alignment, so neither side is 16-byte aligned in general: scalar accesses,
+// every thread's 32 loads in flight before its stores.
+constexpr int EXPORT_THREADS = 256, EXPORT_PER_THREAD = 32, EXPORT_CHUNK = EXPORT_THREADS * EXPORT_PER_THREAD;
+__global__ void __launch_bounds__(EXPORT_THREADS)
+k_export_f32(const float *__restrict__ src, const int64_t *__restrict__ src_off, const int64_t *__restrict__ len,
+             const int64_t *__restrict__ dst_off, const int64_t *__restrict__ cap, const int2 *__restrict__ tab,
+             float *__restrict__ dst) {
+  const int2 t = tab[blockIdx.x];
+  const int64_t c = cap[t.x], n = len[t.x], m = n < c ? n : c;
+  const int64_t b0 = (int64_t)t.y * EXPORT_CHUNK + threadIdx.x;
+  const float *x = src + src_off[t.x];
+  float *y = dst + dst_off[t.x];
+  float v[EXPORT_PER_THREAD];
+#pragma unroll
+  for (int k = 0; k < EXPORT_PER_THREAD; k++) {
+    const int64_t i = b0 + (int64_t)k * EXPORT_THREADS;
+    v[k] = i < m ? __ldcs(x + i) : 0.0f;         // read once: streaming load
+  }
+#pragma unroll
+  for (int k = 0; k < EXPORT_PER_THREAD; k++) {
+    const int64_t i = b0 + (int64_t)k * EXPORT_THREADS;
+    if (i < c) y[i] = v[k];
   }
 }
 
@@ -391,6 +444,7 @@ void sgb_batch_destroy(sgb_batch *b) {
   b->p_pc.release();
   b->h_tot.release(); b->h_summary.release(); b->h_lay.release(); b->h_calltab.release();
   b->d_pcm.release(); b->d_calltab.release();
+  delete b->xo;                    // after wait_stream: no export of this handle is in flight
   delete b->rs;
   for (auto &e : b->ev) cudaEventDestroy(e);
   if (b->ev_wait) cudaEventDestroy(b->ev_wait);
@@ -1310,9 +1364,10 @@ int sgb_synth_min_rows_set(int32_t rows) { g_synth_min_rows_override = rows < 0 
 int sgb_abi_sizes(int32_t *out, int32_t cap) {
   const int32_t v[] = {(int32_t)sizeof(sgb_syllable), (int32_t)sizeof(sgb_envelope), (int32_t)sizeof(sgb_noise),
                        (int32_t)sizeof(sgb_bout), (int32_t)sizeof(sgb_call), (int32_t)sizeof(sgb_formant_ref),
-                       (int32_t)sizeof(sgb_batch_desc), (int32_t)sizeof(sgb_run_info), (int32_t)sizeof(sgb_soundgen_args)};
+                       (int32_t)sizeof(sgb_batch_desc), (int32_t)sizeof(sgb_run_info), (int32_t)sizeof(sgb_soundgen_args),
+                       (int32_t)sizeof(sgb_device_out)};
   if (!out || cap < 9) return fail(SGB_ERR_INVALID, "need room for 9 sizes");
-  for (int i = 0; i < 9; i++) out[i] = v[i];
+  for (int i = 0; i < 10 && i < cap; i++) out[i] = v[i];
   return SGB_OK;
 }
 
@@ -1374,14 +1429,167 @@ int sgb_batch_fetch_pcm16(sgb_batch *b, int16_t *out, int64_t n) {
   for (size_t c = 0; c < NC; c++) { h[c] = b->call_off[c]; h[NC + c] = b->call_len[c]; }
   CK(cudaEventRecord(b->ev[SGB_T_COUNT], st));
   CK(cudaMemcpyAsync(b->d_calltab.p, h, 16 * NC, cudaMemcpyHostToDevice, st));
-  if (NC > 0) k_pcm16<<<(unsigned)NC, 256, 0, st>>>(b->d_out.as<float>(), b->d_calltab.as<int64_t>(),
-                                                   b->d_calltab.as<int64_t>() + NC, b->d_pcm.as<int16_t>());
+  const int64_t *d_off = b->d_calltab.as<int64_t>(), *d_len = d_off + NC;
+  if (NC > 0) k_pcm16<<<(unsigned)NC, 256, 0, st>>>(b->d_out.as<float>(), d_off, d_len, d_off, d_len, b->d_pcm.as<int16_t>());
   if (need > 0) CK(cudaMemcpyAsync(out, b->d_pcm.p, (size_t)need * 2, cudaMemcpyDeviceToHost, st));
   CK(cudaEventRecord(b->ev[SGB_T_COUNT + 1], st));
   CK(wait_stream(b));
   CK(cudaGetLastError());
   CK(cudaEventElapsedTime(&b->info.ms[SGB_T_D2H], b->ev[SGB_T_COUNT], b->ev[SGB_T_COUNT + 1]));
   return SGB_OK;
+}
+
+// ---- device output (sgb_batch_export / sgb_rows_export) ----
+// Checks everything the host can check before anything is queued.  `src` (sgb_rows_export) is checked like dst.
+static int export_check(int device, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
+                        const sgb_device_out *o) {
+  if (!o) return fail(SGB_ERR_INVALID, "null sgb_device_out");
+  if (o->format != SGB_OUT_F32 && o->format != SGB_OUT_PCM16) return fail(SGB_ERR_INVALID, "unknown output format %d", o->format);
+  if (n < 0 || o->dst_elems < 0) return fail(SGB_ERR_INVALID, "negative row count or dst_elems");
+  if (n > 0 && (!o->dst_off || !o->cap || !len || (src && !src_off))) return fail(SGB_ERR_INVALID, "null row table");
+  auto on_device = [&](const void *p, const char *what) -> int {
+    cudaPointerAttributes a;
+    cudaError_t e = cudaPointerGetAttributes(&a, p);
+    if (e != cudaSuccess) { cudaGetLastError(); return fail(SGB_ERR_INVALID, "%s: not a CUDA allocation (%s)", what, cudaGetErrorString(e)); }
+    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
+      return fail(SGB_ERR_INVALID, "%s is host memory (pinned or pageable), not device memory", what);
+    if (a.device != device) return fail(SGB_ERR_INVALID, "%s is memory of device %d, not of device %d", what, a.device, device);
+    return SGB_OK;
+  };
+  std::vector<std::pair<int64_t, int64_t>> rows;
+  rows.reserve((size_t)n);
+  for (int32_t c = 0; c < n; c++) {
+    const int64_t off = o->dst_off[c], cp = o->cap[c];
+    if (off < 0 || cp < 0) return fail(SGB_ERR_INVALID, "row %d: negative offset or capacity", c);
+    if (cp > o->dst_elems || off > o->dst_elems - cp)
+      return fail(SGB_ERR_INVALID, "row %d: elements [%lld, %lld) outside dst (%lld elements)", c, (long long)off,
+                  (long long)(off + cp), (long long)o->dst_elems);
+    if (len[c] < 0 || (src && src_off[c] < 0)) return fail(SGB_ERR_INVALID, "row %d: negative source offset or length", c);
+    if (cp > 0) rows.push_back({off, cp});
+  }
+  std::sort(rows.begin(), rows.end());
+  for (size_t i = 1; i < rows.size(); i++)
+    if (rows[i - 1].first + rows[i - 1].second > rows[i].first)
+      return fail(SGB_ERR_INVALID, "rows overlap in dst at element %lld", (long long)rows[i].first);
+  if (!rows.empty()) {
+    if (!o->dst) return fail(SGB_ERR_INVALID, "null dst");
+    const size_t esz = o->format == SGB_OUT_F32 ? 4 : 2;
+    if ((uintptr_t)o->dst % esz) return fail(SGB_ERR_INVALID, "dst is not aligned to its element type");
+    int rc = on_device(o->dst, "dst");
+    if (rc != SGB_OK) return rc;
+  }
+  if (src) {
+    if ((uintptr_t)src % 4) return fail(SGB_ERR_INVALID, "src is not aligned to float");
+    int rc = on_device(src, "src");
+    if (rc != SGB_OK) return rc;
+  }
+  return SGB_OK;
+}
+
+// Queues the export on `st` (the handle's stream, or the device's export stream) ordered against the caller's
+// stream as the header describes.  Arguments were checked by export_check.
+static int export_queue(ExportCtx &X, cudaStream_t st, const float *src, const int64_t *src_off, const int64_t *len,
+                        int32_t n, const sgb_device_out *o) {
+  cudaStream_t user = (cudaStream_t)o->stream;
+  if (!X.ev_in) CK(cudaEventCreateWithFlags(&X.ev_in, cudaEventDisableTiming));
+  ExportSlot *S = nullptr;
+  for (auto s : X.slots) {
+    cudaError_t q = cudaEventQuery(s->done);
+    if (q == cudaSuccess) { S = s; break; }
+    if (q != cudaErrorNotReady) CK(q);
+    cudaGetLastError();          // cudaErrorNotReady is not an error to carry forward
+  }
+  if (!S) {
+    S = new ExportSlot();
+    cudaError_t e = cudaEventCreateWithFlags(&S->done, cudaEventDisableTiming);
+    if (e != cudaSuccess) { delete S; CK(e); }
+    X.slots.push_back(S);
+  }
+  // row table: src_off, len, dst_off, cap (n each), then the (row, chunk) grid of the f32 kernel
+  std::vector<int2> grid;
+  if (o->format == SGB_OUT_F32) {
+    for (int32_t c = 0; c < n; c++)
+      for (int64_t k = 0; k * EXPORT_CHUNK < o->cap[c]; k++) grid.push_back(make_int2(c, (int)k));
+  }
+  const size_t tab_bytes = 32 * (size_t)n, bytes = tab_bytes + sizeof(int2) * grid.size();
+  CK(S->h.ensure(std::max<size_t>(bytes, 16)));
+  CK(S->d.ensure(std::max<size_t>(bytes, 16)));
+  int64_t *h = S->h.as<int64_t>();
+  for (int32_t c = 0; c < n; c++) {
+    h[c] = src_off[c]; h[n + c] = len[c]; h[2 * (size_t)n + c] = o->dst_off[c]; h[3 * (size_t)n + c] = o->cap[c];
+  }
+  if (!grid.empty()) memcpy(reinterpret_cast<char *>(S->h.p) + tab_bytes, grid.data(), sizeof(int2) * grid.size());
+  const int64_t *d = S->d.as<int64_t>();
+  CK(cudaEventRecord(X.ev_in, user));                // the destination is free once the caller's stream gets here
+  CK(cudaStreamWaitEvent(st, X.ev_in, 0));
+  if (bytes) CK(cudaMemcpyAsync(S->d.p, S->h.p, bytes, cudaMemcpyHostToDevice, st));
+  if (o->format == SGB_OUT_F32) {
+    if (!grid.empty())
+      k_export_f32<<<(unsigned)grid.size(), EXPORT_THREADS, 0, st>>>(
+          src, d, d + n, d + 2 * (size_t)n, d + 3 * (size_t)n,
+          reinterpret_cast<const int2 *>(reinterpret_cast<const char *>(S->d.p) + tab_bytes), (float *)o->dst);
+    CKL("k_export_f32");
+  } else {
+    if (n > 0)
+      k_pcm16<<<(unsigned)n, 256, 0, st>>>(src, d, d + n, d + 2 * (size_t)n, d + 3 * (size_t)n, (int16_t *)o->dst);
+    CKL("k_pcm16");
+  }
+  CK(cudaEventRecord(S->done, st));
+  CK(cudaStreamWaitEvent(user, S->done, 0));        // the caller's later work sees the rows
+  if (o->out_written)
+    for (int32_t c = 0; c < n; c++) o->out_written[c] = std::min(len[c], o->cap[c]);
+  return SGB_OK;
+}
+
+int sgb_batch_export(sgb_batch *b, const sgb_device_out *o) {
+  if (!b) return fail(SGB_ERR_INVALID, "null batch");
+  if (!b->have_run) return fail(SGB_ERR_STATE, "no completed run");
+  CK(cudaSetDevice(b->device));
+  const int32_t n = (int32_t)b->call_len.size();
+  int rc = export_check(b->device, nullptr, nullptr, b->call_len.data(), n, o);
+  if (rc != SGB_OK) return rc;
+  if (!b->xo) b->xo = new ExportCtx();
+  // queued on the handle's stream: the next run of this handle (same stream) cannot overwrite d_out first
+  return export_queue(*b->xo, b->st, b->d_out.as<float>(), b->call_off.data(), b->call_len.data(), n, o);
+}
+
+// one export stream + staging per device for rows the caller holds (no handle); exports from several host threads
+// to the same device take turns on its lock while they queue (nothing inside waits on the device)
+struct DeviceExport {
+  std::mutex mu;
+  cudaStream_t st = nullptr;
+  ExportCtx x;
+};
+static std::mutex g_dev_export_mu;
+static std::map<int, DeviceExport *> g_dev_export;     // kept for the life of the process
+
+int sgb_rows_export(int32_t device, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
+                    const sgb_device_out *o) {
+  int nd = 0;
+  if (cudaGetDeviceCount(&nd) != cudaSuccess || nd < 1) {
+    cudaGetLastError();
+    return fail(SGB_ERR_CUDA, "no CUDA device available (this library has no CPU fallback)");
+  }
+  if (device < 0 || device >= nd) return fail(SGB_ERR_INVALID, "device %d of %d", device, nd);
+  if (n > 0 && !src) return fail(SGB_ERR_INVALID, "null src");
+  CK(cudaSetDevice(device));
+  int rc = export_check(device, n > 0 ? src : nullptr, src_off, len, n, o);
+  if (rc != SGB_OK) return rc;
+  DeviceExport *D;
+  {
+    std::lock_guard<std::mutex> g(g_dev_export_mu);
+    auto it = g_dev_export.find(device);
+    if (it == g_dev_export.end()) {
+      D = new DeviceExport();
+      cudaError_t e = cudaStreamCreateWithFlags(&D->st, cudaStreamNonBlocking);
+      if (e != cudaSuccess) { delete D; CK(e); }
+      g_dev_export[device] = D;
+    } else {
+      D = it->second;
+    }
+  }
+  std::lock_guard<std::mutex> g(D->mu);
+  return export_queue(D->x, D->st, src, src_off, len, n, o);
 }
 
 // Diagnostic for a stuck run (callable from another thread): out[0] = which wait the handle's host thread
