@@ -254,6 +254,40 @@ int sgb_batch_export(sgb_batch *b, const sgb_device_out *o);
 int sgb_rows_export(int32_t device, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
                     const sgb_device_out *o);
 
+/* Spectrograms on the device, into caller-owned device memory (K9).  For a row x of L samples, window length wl
+ * and hop h = wl - overlap*wl/100 (may be fractional):
+ *   frames   k = 0 .. nc-1 start at the 1-based sample floor(1 + k*h), nc = length(seq(1, max(1, L - wl), h))
+ *            (soundgen.R:744-746), nc = 0 when L = 0; samples past L read as 0 (one zero-padded frame when L <= wl);
+ *   spectrum X_k(j) = (1/wl) sum_n x[s_k - 1 + n] w(n) exp(-2 pi i n j / wl), j = 0 .. wl/2 - 1 (seewave's stft as
+ *            soundgen's filter calls it), w = seewave's symmetric hamming.w or hanning.w;
+ *   power    P_k(j) = |X_k(j)|^2;  bands (optional): F_k(b) = sum_j B_b(j) P_k(j) over the contiguous bins
+ *            [band_lo[b], band_lo[b] + band_len[b]) inside [0, wl/2), weights band_w in that order, row after row;
+ *            without bands F = P and n_feat = wl/2, else n_feat = n_bands;
+ *   dB       (optional) 10 log10(max(F, db_floor)).
+ * Layout as sgb_device_out describes it, with cap counted in frames: row c gets exactly cap[c] frames of n_feat
+ * floats from element dst_off[c] on, frame after frame; frames >= nc are zeros; out_written[c] = min(nc, cap[c]);
+ * a row with cap[c] = 0 is left alone (one call per sampling-rate group of a batch).  format must be SGB_OUT_F32.
+ * Frames 2m and 2m+1 share one complex FFT, always: a row's values do not depend on cap or on the other rows.
+ * Stream contract, pinned staging and argument checks are those of the exports.  A wl that cannot be planned or
+ * whose working set does not fit in shared memory gives SGB_ERR_UNSUPPORTED; a bad overlap (hop < 1), window,
+ * band, weight or db_floor gives SGB_ERR_INVALID. */
+#define SGB_WIN_HAMMING 0
+#define SGB_WIN_HANNING 1
+typedef struct sgb_spec_params {
+  int32_t wl, window;            /* even, >= 4; SGB_WIN_*                                           */
+  double  overlap;               /* percent; hop = wl - overlap*wl/100 must be >= 1                 */
+  int32_t n_bands, db;           /* n_bands = 0: no filterbank; db: 0 power, 1 10*log10             */
+  double  db_floor;              /* > 0 when db                                                     */
+  const int32_t *band_lo, *band_len;  const float *band_w;   /* host, n_bands rows (CSR)            */
+} sgb_spec_params;
+/* nc of a row of `len` samples (0 when len = 0), or -1 for a bad wl / overlap. */
+int64_t sgb_spec_frames(int64_t len, int32_t wl, double overlap);
+/* Every call of the last run (row c = call c). */
+int sgb_batch_spectrogram(sgb_batch *b, const sgb_spec_params *p, const sgb_device_out *o);
+/* n float32 rows the caller holds on `device` (row c = len[c] samples at src + src_off[c]). */
+int sgb_rows_spectrogram(int32_t device, const float *src, const int64_t *src_off, const int64_t *len,
+                         int32_t n, const sgb_spec_params *p, const sgb_device_out *o);
+
 /* Intermediate results (valid after run).  Sizes via the *_len calls. */
 int sgb_batch_syllable_len(sgb_batch *b, int32_t syl, int64_t *out_len);
 int sgb_batch_syllable_fetch(sgb_batch *b, int32_t syl, double *out, int64_t n);
@@ -291,8 +325,8 @@ int sgb_batch_set_tracks(sgb_batch *b, int32_t env, const double *rows, int32_t 
 /* Normal draws each voiced syllable consumed (valid after run_begin); n_syllables values. */
 int sgb_batch_z_used(sgb_batch *b, int32_t *out);
 /* sizeof() of the ABI structs, for bindings to verify their mirrors:
- * syllable, envelope, noise, bout, call, formant_ref, batch_desc, run_info, soundgen_args, device_out
- * (cap >= 9; the 10th is written when cap >= 10). */
+ * syllable, envelope, noise, bout, call, formant_ref, batch_desc, run_info, soundgen_args, device_out, spec_params
+ * (cap >= 9; the 10th and 11th are written when cap allows). */
 int sgb_abi_sizes(int32_t *out, int32_t cap);
 /* The additive synthesis has two kernels: epochs with at least `rows` rows run on the tensor cores, the others on the
    FP32 pipe (default 224, or SGB_SYNTH / SGB_SYNTH_MIN_ROWS from the environment).  0 = tensor cores only, a huge value =

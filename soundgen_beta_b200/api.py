@@ -667,6 +667,18 @@ class Batch:
         n = self.desc.n_calls if self.desc is not None else 0
         return _export(lambda o: self.L.sgb_batch_export(self.h, C.byref(o)), n, dst, dst_off, cap, stream, fmt)
 
+    def spectrogram(self, dst, dst_off, cap, wl, overlap=75, window='hamming', bands=None, db=False, db_floor=1e-10,
+                    stream=None):
+        """Spectrogram of every call of the last run (row c = call c) into the float32 CUDA tensor `dst`: call c fills
+        exactly cap[c] frames of n_feat floats from element dst_off[c] of the flattened tensor, its first min(nc, cap)
+        frames and then zeros (see sgb_batch_spectrogram for the frame and spectrum definitions).  bands: None (power,
+        n_feat = wl / 2) or a dense [n_bands, wl / 2] filterbank whose rows each have contiguous support (n_feat =
+        n_bands), e.g. mel_filterbank(); db: 10 log10(max(F, db_floor)).  Ordered on `stream` like export().
+        Returns the frames written per call."""
+        n = self.desc.n_calls if self.desc is not None else 0
+        return _spectrogram(lambda p, o: self.L.sgb_batch_spectrogram(self.h, C.byref(p), C.byref(o)), n, dst, dst_off,
+                            cap, wl, overlap, window, bands, db, db_floor, stream)
+
     def syllable(self, s):
         n = C.c_int64()
         _check(self.L.sgb_batch_syllable_len(self.h, s, C.byref(n)))
@@ -786,6 +798,170 @@ def rows_export(device, src, src_off, lens, dst, dst_off, cap, stream=None, fmt=
     L = _abi.load()
     return _export(lambda o: L.sgb_rows_export(int(device), src.data_ptr() or None, _ptr(so), _ptr(ln), ln.size,
                                                C.byref(o)), ln.size, dst, dst_off, cap, stream, fmt)
+
+
+_WINDOWS = {'hamming': _abi.SGB_WIN_HAMMING, 'hanning': _abi.SGB_WIN_HANNING}
+
+
+def bands_csr(bands, n_bins):
+    """A dense filterbank [n_bands, n_bins] as the library takes it: (lo, len, weights), row b's weights on the
+    contiguous bins [lo[b], lo[b] + len[b]).  A row whose nonzero weights are not contiguous raises ValueError."""
+    B = np.asarray(bands, dtype=np.float32)
+    if B.ndim != 2 or B.shape[0] < 1 or B.shape[1] != n_bins:
+        raise ValueError('bands must be a [n_bands >= 1, %d] array, not %r' % (n_bins, B.shape))
+    lo = np.zeros(B.shape[0], dtype=np.int32)
+    ln = np.zeros(B.shape[0], dtype=np.int32)
+    w = []
+    for b, row in enumerate(B):
+        nz = np.flatnonzero(row)
+        if nz.size == 0:
+            continue
+        a, e = int(nz[0]), int(nz[-1]) + 1
+        if nz.size != e - a:
+            raise ValueError('band %d: weights on non-contiguous bins (%d nonzero in [%d, %d))' % (b, nz.size, a, e))
+        lo[b], ln[b] = a, e - a
+        w.append(row[a:e])
+    return lo, ln, (np.concatenate(w) if w else np.zeros(1, dtype=np.float32))
+
+
+def _spec_params(wl, overlap, window, bands, db, db_floor):
+    """sgb_spec_params for the arguments; also returns the arrays it points into (keep them alive)."""
+    if window not in _WINDOWS:
+        raise ValueError("window must be 'hamming' or 'hanning', not %r" % (window,))
+    p = _abi.SpecParams()
+    p.wl, p.window, p.overlap = int(wl), _WINDOWS[window], float(overlap)
+    p.db, p.db_floor = int(bool(db)), float(db_floor)
+    keep = None
+    if bands is not None:
+        keep = bands_csr(bands, int(wl) // 2)
+        p.n_bands = keep[0].size
+        p.band_lo, p.band_len, p.band_w = (_ptr(a) for a in keep)
+    return p, keep
+
+
+def _spectrogram(call, n, dst, dst_off, cap, wl, overlap, window, bands, db, db_floor, stream):
+    p, keep = _spec_params(wl, overlap, window, bands, db, db_floor)
+    written = _export(lambda o: call(p, o), n, dst, dst_off, cap, stream, 'f32')
+    del keep
+    return written
+
+
+def rows_spectrogram(device, src, src_off, lens, dst, dst_off, cap, wl, overlap=75, window='hamming', bands=None,
+                     db=False, db_floor=1e-10, stream=None):
+    """sgb_rows_spectrogram: Batch.spectrogram over float32 rows the caller holds in the CUDA tensor `src` (row c =
+    lens[c] samples from element src_off[c]).  Returns the frames written per row."""
+    import torch
+    so = np.ascontiguousarray(src_off, dtype=np.int64)
+    ln = np.ascontiguousarray(lens, dtype=np.int64)
+    if not src.is_contiguous() or src.dtype != torch.float32 or so.shape != ln.shape or so.ndim != 1:
+        raise ValueError('src must be a contiguous float32 tensor, src_off and lens of one length')
+    L = _abi.load()
+    return _spectrogram(lambda p, o: L.sgb_rows_spectrogram(int(device), src.data_ptr() or None, _ptr(so), _ptr(ln),
+                                                            ln.size, C.byref(p), C.byref(o)),
+                        ln.size, dst, dst_off, cap, wl, overlap, window, bands, db, db_floor, stream)
+
+
+def _hz_to_mel(f, mel_scale):
+    f = np.asarray(f, dtype=np.float64)
+    if mel_scale == 'htk':
+        return 2595.0 * np.log10(1.0 + f / 700.0)
+    f_sp, min_log_hz = 200.0 / 3, 1000.0
+    min_log_mel, logstep = min_log_hz / f_sp, math.log(6.4) / 27.0
+    return np.where(f >= min_log_hz, min_log_mel + np.log(np.maximum(f, min_log_hz) / min_log_hz) / logstep, f / f_sp)
+
+
+def _mel_to_hz(m, mel_scale):
+    m = np.asarray(m, dtype=np.float64)
+    if mel_scale == 'htk':
+        return 700.0 * (10.0 ** (m / 2595.0) - 1.0)
+    f_sp, min_log_hz = 200.0 / 3, 1000.0
+    min_log_mel, logstep = min_log_hz / f_sp, math.log(6.4) / 27.0
+    return np.where(m >= min_log_mel, min_log_hz * np.exp(logstep * (m - min_log_mel)), f_sp * m)
+
+
+def mel_filterbank(samplingRate, wl, n_mels, fmin=0, fmax=None, mel_scale='htk', norm=None):
+    """Triangular mel filterbank over the wl / 2 bins of a wl-point spectrum (bin j at j * samplingRate / wl), as a
+    [n_mels, wl / 2] float64 array: torchaudio.functional.melscale_fbanks(wl // 2 + 1, fmin, fmax, n_mels,
+    samplingRate, norm, mel_scale)[:wl // 2].T, without the dependency.  fmax defaults to samplingRate // 2.
+    mel_scale: 'htk' or 'slaney'; norm: None or 'slaney' (each band scaled to unit area in Hz)."""
+    if mel_scale not in ('htk', 'slaney'):
+        raise ValueError("mel_scale must be 'htk' or 'slaney', not %r" % (mel_scale,))
+    if norm not in (None, 'slaney'):
+        raise ValueError("norm must be None or 'slaney', not %r" % (norm,))
+    wl, n_mels = int(wl), int(n_mels)
+    if wl < 4 or wl % 2 or n_mels < 1 or not samplingRate > 0:
+        raise ValueError('need an even wl >= 4, n_mels >= 1 and a positive samplingRate')
+    fmax = float(samplingRate // 2) if fmax is None else float(fmax)
+    if not 0 <= fmin < fmax:
+        raise ValueError('need 0 <= fmin < fmax (%r, %r)' % (fmin, fmax))
+    freqs = np.arange(wl // 2, dtype=np.float64) * float(samplingRate) / wl
+    m = np.linspace(_hz_to_mel(float(fmin), mel_scale), _hz_to_mel(fmax, mel_scale), n_mels + 2)
+    f_pts = _mel_to_hz(m, mel_scale)
+    f_diff = np.diff(f_pts)
+    slopes = f_pts[None, :] - freqs[:, None]
+    down = -slopes[:, :-2] / f_diff[:-1]
+    up = slopes[:, 2:] / f_diff[1:]
+    fb = np.maximum(0.0, np.minimum(down, up))
+    if norm == 'slaney':
+        fb = fb * (2.0 / (f_pts[2:n_mels + 2] - f_pts[:n_mels]))[None, :]
+    return np.ascontiguousarray(fb.T)
+
+
+def spectrogram_device(wave, lengths, samplingRate, windowLength=50, overlap=75, window='hamming', n_mels=None, fmin=0,
+                       fmax=None, mel_scale='htk', norm=None, db=False, db_floor=1e-10, max_frames=None, stream=None):
+    """Power (n_mels None) or mel spectrograms of the [n, T] float32 CUDA tensor `wave` that soundgen_batch_device
+    returns, row c = its first lengths[c] samples.  Returns (spec, frames): spec [n, F, n_feat] float32 on the same
+    device, frame k of row c at spec[c, k] (zeros past the row's frames), F = max_frames or the most frames of any
+    row; frames: int64 CUDA tensor of the frames present per row.  n_feat = wl / 2 bins, or n_mels.
+    Each row's window is wl = floor(windowLength / 1000 * sr / 2) * 2 points (soundgen.R:317) at its sampling rate
+    sr: samplingRate is one value or one per row, and must be the rate the row was synthesised at.  A linear
+    spectrogram needs one wl for all rows; mel features may mix rates (one library call per rate).
+    lengths may be host or CUDA; a CUDA tensor is read back once, which synchronises with its stream.
+    The result is ordered on `stream` (default: the device's current torch stream), with no other host wait."""
+    import torch
+    if not (torch.is_tensor(wave) and wave.is_cuda and wave.dtype == torch.float32 and wave.dim() == 2):
+        raise ValueError('wave must be a 2-D float32 CUDA tensor')
+    if window not in _WINDOWS:
+        raise ValueError("window must be 'hamming' or 'hanning', not %r" % (window,))
+    n, T = wave.shape
+    lens = (lengths.cpu().numpy() if torch.is_tensor(lengths) else np.asarray(lengths)).astype(np.int64).reshape(-1)
+    if lens.shape != (n,) or np.any(lens < 0) or np.any(lens > T):
+        raise ValueError('lengths needs one value in [0, %d] per row (%d)' % (T, n))
+    sr = np.broadcast_to(np.asarray(samplingRate, dtype=np.float64).reshape(-1), (n,)) if n else np.zeros(0)
+    if not np.all(np.isfinite(sr) & (sr > 0)):
+        raise ValueError('samplingRate must be positive')
+    wl = (np.floor(windowLength / 1000 * sr / 2) * 2).astype(np.int64)
+    if max_frames is not None and int(max_frames) < 0:
+        raise ValueError('max_frames must be non-negative')
+    if n_mels is None:
+        if np.unique(wl).size > 1:
+            raise ValueError('a linear spectrogram needs one window length for all rows, not %s' % np.unique(wl))
+        groups = [(np.arange(n), None)]
+        n_feat = int(wl[0]) // 2 if n else 0
+    else:
+        if int(n_mels) < 1:
+            raise ValueError('n_mels must be positive')
+        groups = [(np.flatnonzero(sr == r), r) for r in np.unique(sr)]
+        n_feat = int(n_mels)
+    L = _abi.load()
+    nc = np.array([L.sgb_spec_frames(int(l), int(w), float(overlap)) for l, w in zip(lens, wl)], dtype=np.int64)
+    if np.any(nc < 0):
+        raise SoundgenError(_abi.SGB_ERR_UNSUPPORTED, 'window of %s points / overlap %r cannot be analysed'
+                            % (np.unique(wl[nc < 0]), overlap))
+    F = int(max_frames) if max_frames is not None else int(nc.max(initial=0))
+    spec = torch.empty((n, F, n_feat), dtype=torch.float32, device=wave.device)
+    if n and F and n_feat:
+        src = wave.contiguous()
+        rows = np.arange(n, dtype=np.int64)
+        for idx, r in groups:
+            w = int(wl[idx[0]])
+            bands = None if r is None else mel_filterbank(r, w, n_feat, fmin, fmax, mel_scale, norm)
+            cap = np.zeros(n, dtype=np.int64)
+            cap[idx] = F
+            rows_spectrogram(wave.device.index, src, rows * T, lens, spec, rows * F * n_feat, cap, w, overlap, window,
+                             bands, db, db_floor, stream)
+    frames = torch.as_tensor(np.minimum(nc, F), dtype=torch.int64).to(wave.device)
+    return spec, frames
 
 
 def _torch_out_dtype(dtype):

@@ -9,6 +9,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <map>
 #include <mutex>
 #include <string>
@@ -48,6 +49,10 @@ cudaError_t launch_stft(int mode, int u_is_float, int spec, const FftSeg *, int,
                         const float2 *, const float *, const float *, const void *, const float *, float *, int *,
                         size_t, cudaStream_t);
 int stft_spec_of(int n, const int *radix, int npass);
+size_t spectrogram_smem_bytes(int n, double h_in, int n_bands, int64_t n_w);
+cudaError_t launch_spectrogram(const FftSeg *, int, const SpecRow *, const FftPlan &, const float2 *, const float *,
+                               const float *, int, const int32_t *, const float *, int, int, float, float *, size_t,
+                               cudaStream_t);
 void launch_noise_final(const sgb_noise *, int, const NoiseLayout *, const double *, const double *, const int *, int,
                         const float *, float *, void *, double *, const int64_t *, int, cudaStream_t);
 size_t contour_tab_bytes();
@@ -744,9 +749,9 @@ struct PlanTable {
     pl.h_in = n - (overlap * n / 100.0);
     pl.h_out = n * (100.0 - overlap) / 100.0;
     const size_t t0 = tw.size(), w0 = win.size();
-    pl.tw_off = (int64_t)t0; pl.wa_off = (int64_t)w0; pl.ws_off = (int64_t)w0 + n;
+    pl.tw_off = (int64_t)t0; pl.wa_off = (int64_t)w0; pl.ws_off = (int64_t)w0 + n; pl.wh_off = (int64_t)w0 + 2 * n;
     tw.resize(t0 + n);
-    win.resize(w0 + 2 * (size_t)n);
+    win.resize(w0 + 3 * (size_t)n);
     const double two_pi = 2.0 * 3.141592653589793;
     double W0 = 0.0;
     std::vector<double> hann(n);
@@ -759,6 +764,7 @@ struct PlanTable {
       win[w0 + i] = (float)((0.54 - 0.46 * c) / (double)n);
     }
     for (int i = 0; i < n; i++) win[w0 + n + i] = (float)(hann[i] * pl.h_out / (W0 * (double)n));
+    for (int i = 0; i < n; i++) win[w0 + 2 * n + i] = (float)(hann[i] / (double)n);
     plans.push_back(pl);
     idx[key] = (int)plans.size() - 1;
     return (int)plans.size() - 1;
@@ -1365,9 +1371,9 @@ int sgb_abi_sizes(int32_t *out, int32_t cap) {
   const int32_t v[] = {(int32_t)sizeof(sgb_syllable), (int32_t)sizeof(sgb_envelope), (int32_t)sizeof(sgb_noise),
                        (int32_t)sizeof(sgb_bout), (int32_t)sizeof(sgb_call), (int32_t)sizeof(sgb_formant_ref),
                        (int32_t)sizeof(sgb_batch_desc), (int32_t)sizeof(sgb_run_info), (int32_t)sizeof(sgb_soundgen_args),
-                       (int32_t)sizeof(sgb_device_out)};
+                       (int32_t)sizeof(sgb_device_out), (int32_t)sizeof(sgb_spec_params)};
   if (!out || cap < 9) return fail(SGB_ERR_INVALID, "need room for 9 sizes");
-  for (int i = 0; i < 10 && i < cap; i++) out[i] = v[i];
+  for (int i = 0; i < 11 && i < cap; i++) out[i] = v[i];
   return SGB_OK;
 }
 
@@ -1439,12 +1445,14 @@ int sgb_batch_fetch_pcm16(sgb_batch *b, int16_t *out, int64_t n) {
   return SGB_OK;
 }
 
-// ---- device output (sgb_batch_export / sgb_rows_export) ----
-// Checks everything the host can check before anything is queued.  `src` (sgb_rows_export) is checked like dst.
+// ---- device output (sgb_batch_export / sgb_rows_export, sgb_batch_spectrogram / sgb_rows_spectrogram) ----
+// Checks everything the host can check before anything is queued.  `src` (the rows entries) is checked like dst.
+// Row c occupies cap[c] * unit elements of dst (unit: floats per frame of a spectrogram, 1 for the exports).
 static int export_check(int device, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
-                        const sgb_device_out *o) {
+                        const sgb_device_out *o, int64_t unit, bool pcm16_ok) {
   if (!o) return fail(SGB_ERR_INVALID, "null sgb_device_out");
-  if (o->format != SGB_OUT_F32 && o->format != SGB_OUT_PCM16) return fail(SGB_ERR_INVALID, "unknown output format %d", o->format);
+  if (o->format != SGB_OUT_F32 && !(pcm16_ok && o->format == SGB_OUT_PCM16))
+    return fail(SGB_ERR_INVALID, "unsupported output format %d", o->format);
   if (n < 0 || o->dst_elems < 0) return fail(SGB_ERR_INVALID, "negative row count or dst_elems");
   if (n > 0 && (!o->dst_off || !o->cap || !len || (src && !src_off))) return fail(SGB_ERR_INVALID, "null row table");
   auto on_device = [&](const void *p, const char *what) -> int {
@@ -1461,11 +1469,11 @@ static int export_check(int device, const float *src, const int64_t *src_off, co
   for (int32_t c = 0; c < n; c++) {
     const int64_t off = o->dst_off[c], cp = o->cap[c];
     if (off < 0 || cp < 0) return fail(SGB_ERR_INVALID, "row %d: negative offset or capacity", c);
-    if (cp > o->dst_elems || off > o->dst_elems - cp)
-      return fail(SGB_ERR_INVALID, "row %d: elements [%lld, %lld) outside dst (%lld elements)", c, (long long)off,
-                  (long long)(off + cp), (long long)o->dst_elems);
+    if (off > o->dst_elems || cp > (o->dst_elems - off) / unit)
+      return fail(SGB_ERR_INVALID, "row %d: elements [%lld, %lld x %lld more) outside dst (%lld elements)", c,
+                  (long long)off, (long long)cp, (long long)unit, (long long)o->dst_elems);
     if (len[c] < 0 || (src && src_off[c] < 0)) return fail(SGB_ERR_INVALID, "row %d: negative source offset or length", c);
-    if (cp > 0) rows.push_back({off, cp});
+    if (cp > 0) rows.push_back({off, cp * unit});
   }
   std::sort(rows.begin(), rows.end());
   for (size_t i = 1; i < rows.size(); i++)
@@ -1486,10 +1494,11 @@ static int export_check(int device, const float *src, const int64_t *src_off, co
   return SGB_OK;
 }
 
-// Queues the export on `st` (the handle's stream, or the device's export stream) ordered against the caller's
-// stream as the header describes.  Arguments were checked by export_check.
-static int export_queue(ExportCtx &X, cudaStream_t st, const float *src, const int64_t *src_off, const int64_t *len,
-                        int32_t n, const sgb_device_out *o) {
+// Queues work on `st` (the handle's stream, or the device's export stream) ordered against the caller's stream as
+// the header describes.  fill(h) writes `bytes` of host-built tables into a pinned staging slot; launch(d) queues
+// the kernels on their device copy.  Arguments were checked by export_check.
+static int export_queue(ExportCtx &X, cudaStream_t st, const sgb_device_out *o, size_t bytes,
+                        const std::function<void(char *)> &fill, const std::function<int(const char *)> &launch) {
   cudaStream_t user = (cudaStream_t)o->stream;
   if (!X.ev_in) CK(cudaEventCreateWithFlags(&X.ev_in, cudaEventDisableTiming));
   ExportSlot *S = nullptr;
@@ -1505,6 +1514,21 @@ static int export_queue(ExportCtx &X, cudaStream_t st, const float *src, const i
     if (e != cudaSuccess) { delete S; CK(e); }
     X.slots.push_back(S);
   }
+  CK(S->h.ensure(std::max<size_t>(bytes, 16)));
+  CK(S->d.ensure(std::max<size_t>(bytes, 16)));
+  fill(reinterpret_cast<char *>(S->h.p));
+  CK(cudaEventRecord(X.ev_in, user));                // the destination is free once the caller's stream gets here
+  CK(cudaStreamWaitEvent(st, X.ev_in, 0));
+  if (bytes) CK(cudaMemcpyAsync(S->d.p, S->h.p, bytes, cudaMemcpyHostToDevice, st));
+  const int rc = launch(reinterpret_cast<const char *>(S->d.p));
+  CK(cudaEventRecord(S->done, st));                  // the slot is reused only after its copy has been read
+  if (rc != SGB_OK) return rc;
+  CK(cudaStreamWaitEvent(user, S->done, 0));        // the caller's later work sees the rows
+  return SGB_OK;
+}
+
+static int export_rows(ExportCtx &X, cudaStream_t st, const float *src, const int64_t *src_off, const int64_t *len,
+                       int32_t n, const sgb_device_out *o) {
   // row table: src_off, len, dst_off, cap (n each), then the (row, chunk) grid of the f32 kernel
   std::vector<int2> grid;
   if (o->format == SGB_OUT_F32) {
@@ -1512,32 +1536,41 @@ static int export_queue(ExportCtx &X, cudaStream_t st, const float *src, const i
       for (int64_t k = 0; k * EXPORT_CHUNK < o->cap[c]; k++) grid.push_back(make_int2(c, (int)k));
   }
   const size_t tab_bytes = 32 * (size_t)n, bytes = tab_bytes + sizeof(int2) * grid.size();
-  CK(S->h.ensure(std::max<size_t>(bytes, 16)));
-  CK(S->d.ensure(std::max<size_t>(bytes, 16)));
-  int64_t *h = S->h.as<int64_t>();
-  for (int32_t c = 0; c < n; c++) {
-    h[c] = src_off[c]; h[n + c] = len[c]; h[2 * (size_t)n + c] = o->dst_off[c]; h[3 * (size_t)n + c] = o->cap[c];
-  }
-  if (!grid.empty()) memcpy(reinterpret_cast<char *>(S->h.p) + tab_bytes, grid.data(), sizeof(int2) * grid.size());
-  const int64_t *d = S->d.as<int64_t>();
-  CK(cudaEventRecord(X.ev_in, user));                // the destination is free once the caller's stream gets here
-  CK(cudaStreamWaitEvent(st, X.ev_in, 0));
-  if (bytes) CK(cudaMemcpyAsync(S->d.p, S->h.p, bytes, cudaMemcpyHostToDevice, st));
-  if (o->format == SGB_OUT_F32) {
-    if (!grid.empty())
-      k_export_f32<<<(unsigned)grid.size(), EXPORT_THREADS, 0, st>>>(
-          src, d, d + n, d + 2 * (size_t)n, d + 3 * (size_t)n,
-          reinterpret_cast<const int2 *>(reinterpret_cast<const char *>(S->d.p) + tab_bytes), (float *)o->dst);
-    CKL("k_export_f32");
-  } else {
-    if (n > 0)
-      k_pcm16<<<(unsigned)n, 256, 0, st>>>(src, d, d + n, d + 2 * (size_t)n, d + 3 * (size_t)n, (int16_t *)o->dst);
-    CKL("k_pcm16");
-  }
-  CK(cudaEventRecord(S->done, st));
-  CK(cudaStreamWaitEvent(user, S->done, 0));        // the caller's later work sees the rows
+  auto fill = [&](char *hp) {
+    int64_t *h = reinterpret_cast<int64_t *>(hp);
+    for (int32_t c = 0; c < n; c++) {
+      h[c] = src_off[c]; h[n + c] = len[c]; h[2 * (size_t)n + c] = o->dst_off[c]; h[3 * (size_t)n + c] = o->cap[c];
+    }
+    if (!grid.empty()) memcpy(hp + tab_bytes, grid.data(), sizeof(int2) * grid.size());
+  };
+  auto launch = [&](const char *dp) -> int {
+    const int64_t *d = reinterpret_cast<const int64_t *>(dp);
+    if (o->format == SGB_OUT_F32) {
+      if (!grid.empty())
+        k_export_f32<<<(unsigned)grid.size(), EXPORT_THREADS, 0, st>>>(
+            src, d, d + n, d + 2 * (size_t)n, d + 3 * (size_t)n, reinterpret_cast<const int2 *>(dp + tab_bytes),
+            (float *)o->dst);
+      CKL("k_export_f32");
+    } else {
+      if (n > 0)
+        k_pcm16<<<(unsigned)n, 256, 0, st>>>(src, d, d + n, d + 2 * (size_t)n, d + 3 * (size_t)n, (int16_t *)o->dst);
+      CKL("k_pcm16");
+    }
+    return SGB_OK;
+  };
+  int rc = export_queue(X, st, o, bytes, fill, launch);
+  if (rc != SGB_OK) return rc;
   if (o->out_written)
     for (int32_t c = 0; c < n; c++) o->out_written[c] = std::min(len[c], o->cap[c]);
+  return SGB_OK;
+}
+
+static int no_device() {
+  int nd = 0;
+  if (cudaGetDeviceCount(&nd) != cudaSuccess || nd < 1) {
+    cudaGetLastError();
+    return fail(SGB_ERR_CUDA, "no CUDA device available (this library has no CPU fallback)");
+  }
   return SGB_OK;
 }
 
@@ -1546,11 +1579,11 @@ int sgb_batch_export(sgb_batch *b, const sgb_device_out *o) {
   if (!b->have_run) return fail(SGB_ERR_STATE, "no completed run");
   CK(cudaSetDevice(b->device));
   const int32_t n = (int32_t)b->call_len.size();
-  int rc = export_check(b->device, nullptr, nullptr, b->call_len.data(), n, o);
+  int rc = export_check(b->device, nullptr, nullptr, b->call_len.data(), n, o, 1, true);
   if (rc != SGB_OK) return rc;
   if (!b->xo) b->xo = new ExportCtx();
   // queued on the handle's stream: the next run of this handle (same stream) cannot overwrite d_out first
-  return export_queue(*b->xo, b->st, b->d_out.as<float>(), b->call_off.data(), b->call_len.data(), n, o);
+  return export_rows(*b->xo, b->st, b->d_out.as<float>(), b->call_off.data(), b->call_len.data(), n, o);
 }
 
 // one export stream + staging per device for rows the caller holds (no handle); exports from several host threads
@@ -1563,33 +1596,218 @@ struct DeviceExport {
 static std::mutex g_dev_export_mu;
 static std::map<int, DeviceExport *> g_dev_export;     // kept for the life of the process
 
-int sgb_rows_export(int32_t device, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
-                    const sgb_device_out *o) {
-  int nd = 0;
-  if (cudaGetDeviceCount(&nd) != cudaSuccess || nd < 1) {
-    cudaGetLastError();
-    return fail(SGB_ERR_CUDA, "no CUDA device available (this library has no CPU fallback)");
+static int device_export(int device, DeviceExport **out) {
+  std::lock_guard<std::mutex> g(g_dev_export_mu);
+  auto it = g_dev_export.find(device);
+  if (it == g_dev_export.end()) {
+    DeviceExport *D = new DeviceExport();
+    cudaError_t e = cudaStreamCreateWithFlags(&D->st, cudaStreamNonBlocking);
+    if (e != cudaSuccess) { delete D; CK(e); }
+    g_dev_export[device] = D;
+    *out = D;
+  } else {
+    *out = it->second;
   }
+  return SGB_OK;
+}
+
+static int rows_device_check(int32_t device, const float *src, int32_t n) {
+  int rc = no_device();
+  if (rc != SGB_OK) return rc;
+  int nd = 0;
+  CK(cudaGetDeviceCount(&nd));
   if (device < 0 || device >= nd) return fail(SGB_ERR_INVALID, "device %d of %d", device, nd);
   if (n > 0 && !src) return fail(SGB_ERR_INVALID, "null src");
   CK(cudaSetDevice(device));
-  int rc = export_check(device, n > 0 ? src : nullptr, src_off, len, n, o);
+  return SGB_OK;
+}
+
+int sgb_rows_export(int32_t device, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
+                    const sgb_device_out *o) {
+  int rc = rows_device_check(device, src, n);
+  if (rc != SGB_OK) return rc;
+  rc = export_check(device, n > 0 ? src : nullptr, src_off, len, n, o, 1, true);
   if (rc != SGB_OK) return rc;
   DeviceExport *D;
-  {
-    std::lock_guard<std::mutex> g(g_dev_export_mu);
-    auto it = g_dev_export.find(device);
-    if (it == g_dev_export.end()) {
-      D = new DeviceExport();
-      cudaError_t e = cudaStreamCreateWithFlags(&D->st, cudaStreamNonBlocking);
-      if (e != cudaSuccess) { delete D; CK(e); }
-      g_dev_export[device] = D;
-    } else {
-      D = it->second;
-    }
-  }
+  if ((rc = device_export(device, &D)) != SGB_OK) return rc;
   std::lock_guard<std::mutex> g(D->mu);
-  return export_queue(D->x, D->st, src, src_off, len, n, o);
+  return export_rows(D->x, D->st, src, src_off, len, n, o);
+}
+
+// ---- spectrograms (K9) ----
+// nc = length(seq(1, max(1, len - wl), h)) in 64 bits (seq_by_count), 0 for an empty row
+static int64_t spec_nc(int64_t len, int wl, double h) {
+  if (len <= 0) return 0;
+  const double to = std::max<double>(1.0, (double)(len - wl));
+  if (to == 1.0) return 1;
+  return (int64_t)std::floor((to - 1.0) / h + 1e-10) + 1;
+}
+
+static int spec_geometry(int32_t wl, double overlap, double *h) {
+  if (wl < 4 || (wl & 1)) return fail(SGB_ERR_UNSUPPORTED, "window of %d points (odd or < 4) is not supported", wl);
+  if (!(overlap >= 0.0 && overlap < 100.0)) return fail(SGB_ERR_INVALID, "overlap %g out of [0, 100)", overlap);
+  *h = wl - (overlap * wl / 100.0);
+  if (!(*h >= 1.0)) return fail(SGB_ERR_INVALID, "hop %g of a %d-point window is below one sample", *h, wl);
+  return SGB_OK;
+}
+
+int64_t sgb_spec_frames(int64_t len, int32_t wl, double overlap) {
+  double h;
+  if (len < 0 || spec_geometry(wl, overlap, &h) != SGB_OK) return -1;
+  return spec_nc(len, wl, h);
+}
+
+// Everything a spectrogram call queues, built and checked on the host before anything is queued.
+struct SpecJob {
+  PlanTable PT;
+  FftPlan pl;
+  int n_feat = 0, n_w = 0;
+  size_t smem = 0;
+  std::vector<SpecRow> rows;
+  std::vector<FftSeg> segs;
+  std::vector<int32_t> band_tab;       // lo, len, first weight (n_bands each)
+};
+
+// the parameters alone (no device needed)
+static int spec_params(const sgb_spec_params *p, SpecJob &J) {
+  if (!p) return fail(SGB_ERR_INVALID, "null sgb_spec_params");
+  double h;
+  int rc = spec_geometry(p->wl, p->overlap, &h);
+  if (rc != SGB_OK) return rc;
+  if (p->window != SGB_WIN_HAMMING && p->window != SGB_WIN_HANNING) return fail(SGB_ERR_INVALID, "unknown window %d", p->window);
+  if (p->db != 0 && p->db != 1) return fail(SGB_ERR_INVALID, "db must be 0 or 1, not %d", p->db);
+  if (p->db && !(p->db_floor > 0.0 && std::isfinite(p->db_floor) && (float)p->db_floor > 0.0f))
+    return fail(SGB_ERR_INVALID, "db_floor %g: a positive finite float is needed", p->db_floor);
+  const int nr = p->wl / 2;
+  if (p->n_bands < 0) return fail(SGB_ERR_INVALID, "negative n_bands");
+  if (p->n_bands > 0) {
+    if (!p->band_lo || !p->band_len || !p->band_w) return fail(SGB_ERR_INVALID, "null band table");
+    J.band_tab.resize(3 * (size_t)p->n_bands);
+    int64_t nw = 0;
+    for (int b = 0; b < p->n_bands; b++) {
+      const int32_t lo = p->band_lo[b], ln = p->band_len[b];
+      if (lo < 0 || ln < 0 || lo > nr || ln > nr - lo)
+        return fail(SGB_ERR_INVALID, "band %d: bins [%d, %d + %d) outside [0, %d)", b, lo, lo, ln, nr);
+      for (int j = 0; j < ln; j++)
+        if (!std::isfinite(p->band_w[nw + j])) return fail(SGB_ERR_INVALID, "band %d: weight %d is not finite", b, j);
+      if (nw + ln > (int64_t)INT32_MAX) return fail(SGB_ERR_UNSUPPORTED, "band weights do not fit in shared memory");
+      J.band_tab[b] = lo; J.band_tab[p->n_bands + b] = ln; J.band_tab[2 * (size_t)p->n_bands + b] = (int32_t)nw;
+      nw += ln;
+    }
+    J.n_w = (int)nw;
+  }
+  J.n_feat = p->n_bands ? p->n_bands : nr;
+  J.smem = spectrogram_smem_bytes(p->wl, h, p->n_bands, J.n_w);
+  if (J.smem > 226 * 1024) return fail(SGB_ERR_UNSUPPORTED, "window and bands too large for shared memory (%zu bytes)", J.smem);
+  const int pi = J.PT.get(p->wl, p->overlap);
+  if (pi < 0) return fail(SGB_ERR_UNSUPPORTED, "cannot factor window length %d", p->wl);
+  J.pl = J.PT.plans[pi];
+  return SGB_OK;
+}
+
+// the rows and the destination, after spec_params
+static int spec_rows(const sgb_spec_params *p, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
+                     const sgb_device_out *o, int device, SpecJob &J) {
+  const double h = J.pl.h_in;
+  int rc = export_check(device, src, src_off, len, n, o, J.n_feat, false);
+  if (rc != SGB_OK) return rc;
+  // rows: the first min(nc, cap) frames are computed, frame pairs completed (a pair is one FFT); the rest are zeros
+  std::vector<FftJob> jobs;
+  J.rows.resize((size_t)n);
+  for (int32_t c = 0; c < n; c++) {
+    if (len[c] > INT32_MAX || o->cap[c] > INT32_MAX)
+      return fail(SGB_ERR_INVALID, "row %d: %lld samples, %lld frames (at most 2^31 - 1 each)", c, (long long)len[c],
+                  (long long)o->cap[c]);
+    SpecRow &R = J.rows[c];
+    R.src_off = src_off[c]; R.dst_off = o->dst_off[c]; R.len = len[c]; R.cap = o->cap[c];
+    R.nc = spec_nc(len[c], p->wl, h);
+    FftJob fj;
+    memset(&fj, 0, sizeof fj);
+    fj.plan = 0;
+    fj.nc = (int32_t)std::min(R.nc, R.cap + (R.cap & 1));
+    jobs.push_back(fj);
+  }
+  std::vector<SegGroup> groups;
+  make_segs(jobs, J.PT.plans, 0, J.segs, groups);
+  const int zf = std::max(1, 8192 / J.n_feat);        // zero-tail segments: about 8192 floats each
+  for (int32_t c = 0; c < n; c++)
+    for (int64_t k = J.rows[c].nc; k < J.rows[c].cap; k += zf) {
+      FftSeg sg; sg.job = c; sg.ka = (int32_t)k; sg.kb = (int32_t)std::min<int64_t>(J.rows[c].cap, k + zf); sg.pad = 0;
+      J.segs.push_back(sg);
+    }
+  if (J.segs.size() > (size_t)INT32_MAX) return fail(SGB_ERR_UNSUPPORTED, "too many segments");
+  return SGB_OK;
+}
+
+static int spec_queue(ExportCtx &X, cudaStream_t st, const float *src, const SpecJob &J, const sgb_spec_params *p,
+                      const sgb_device_out *o) {
+  const int N = J.pl.n, nb = p->n_bands;
+  auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
+  const size_t o_rows = 0, o_segs = up16(o_rows + sizeof(SpecRow) * J.rows.size());
+  const size_t o_tw = up16(o_segs + sizeof(FftSeg) * J.segs.size()), o_win = up16(o_tw + sizeof(float2) * N);
+  const size_t o_band = up16(o_win + sizeof(float) * N), o_w = up16(o_band + sizeof(int32_t) * J.band_tab.size());
+  const size_t bytes = o_w + sizeof(float) * J.n_w;
+  const int64_t w_off = p->window == SGB_WIN_HANNING ? J.pl.wh_off : J.pl.wa_off;
+  auto fill = [&](char *h) {
+    if (!J.rows.empty()) memcpy(h + o_rows, J.rows.data(), sizeof(SpecRow) * J.rows.size());
+    if (!J.segs.empty()) memcpy(h + o_segs, J.segs.data(), sizeof(FftSeg) * J.segs.size());
+    memcpy(h + o_tw, J.PT.tw.data() + J.pl.tw_off, sizeof(float2) * N);
+    memcpy(h + o_win, J.PT.win.data() + w_off, sizeof(float) * N);
+    if (nb) {
+      memcpy(h + o_band, J.band_tab.data(), sizeof(int32_t) * J.band_tab.size());
+      memcpy(h + o_w, p->band_w, sizeof(float) * J.n_w);
+    }
+  };
+  auto launch = [&](const char *d) -> int {
+    cudaError_t e = launch_spectrogram(reinterpret_cast<const FftSeg *>(d + o_segs), (int)J.segs.size(),
+                                       reinterpret_cast<const SpecRow *>(d + o_rows), J.pl,
+                                       reinterpret_cast<const float2 *>(d + o_tw), reinterpret_cast<const float *>(d + o_win),
+                                       src, nb, reinterpret_cast<const int32_t *>(d + o_band),
+                                       reinterpret_cast<const float *>(d + o_w), J.n_w, p->db, (float)p->db_floor,
+                                       (float *)o->dst, J.smem, st);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return fail(SGB_ERR_CUDA, "k_spectrogram launch failed (%zu segments, %zu bytes of shared memory): %s",
+                  J.segs.size(), J.smem, cudaGetErrorString(e));
+    }
+    return SGB_OK;
+  };
+  int rc = export_queue(X, st, o, bytes, fill, launch);
+  if (rc != SGB_OK) return rc;
+  if (o->out_written)
+    for (size_t c = 0; c < J.rows.size(); c++) o->out_written[c] = std::min(J.rows[c].nc, J.rows[c].cap);
+  return SGB_OK;
+}
+
+int sgb_batch_spectrogram(sgb_batch *b, const sgb_spec_params *p, const sgb_device_out *o) {
+  SpecJob J;
+  int rc = spec_params(p, J);
+  if (rc != SGB_OK) return rc;
+  if ((rc = no_device()) != SGB_OK) return rc;
+  if (!b) return fail(SGB_ERR_INVALID, "null batch");
+  if (!b->have_run) return fail(SGB_ERR_STATE, "no completed run");
+  CK(cudaSetDevice(b->device));
+  const int32_t n = (int32_t)b->call_len.size();
+  rc = spec_rows(p, nullptr, b->call_off.data(), b->call_len.data(), n, o, b->device, J);
+  if (rc != SGB_OK) return rc;
+  if (!b->xo) b->xo = new ExportCtx();
+  // on the handle's stream, like the export: the handle's next run cannot overwrite the rows first
+  return spec_queue(*b->xo, b->st, b->d_out.as<float>(), J, p, o);
+}
+
+int sgb_rows_spectrogram(int32_t device, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
+                         const sgb_spec_params *p, const sgb_device_out *o) {
+  SpecJob J;
+  int rc = spec_params(p, J);
+  if (rc != SGB_OK) return rc;
+  if ((rc = rows_device_check(device, src, n)) != SGB_OK) return rc;
+  if (n > 0 && !src_off) return fail(SGB_ERR_INVALID, "null src_off");
+  rc = spec_rows(p, n > 0 ? src : nullptr, src_off, len, n, o, device, J);
+  if (rc != SGB_OK) return rc;
+  DeviceExport *D;
+  if ((rc = device_export(device, &D)) != SGB_OK) return rc;
+  std::lock_guard<std::mutex> g(D->mu);
+  return spec_queue(D->x, D->st, src, J, p, o);
 }
 
 // Diagnostic for a stuck run (callable from another thread): out[0] = which wait the handle's host thread

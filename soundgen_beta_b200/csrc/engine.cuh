@@ -124,6 +124,7 @@ struct FftPlan {
   int64_t tw_off;            // float2[n]: exp(-2*pi*i*t/n)
   int64_t wa_off;            // float[n]: analysis window (Hamming) / n
   int64_t ws_off;            // float[n]: synthesis window (Hanning) * h / (sum(win^2) * n)
+  int64_t wh_off;            // float[n]: Hanning analysis window / n (K9)
   double h_in;               // wl - overlap*wl/100  (frame starts 1 + k*h_in)
   double h_out;              // wl*(100-overlap)/100 (OLA offsets k*h_out)
 };
@@ -144,6 +145,14 @@ struct FftJob {              // one sound (bout to filter, or noise segment to g
 };
 
 struct FftSeg { int32_t job, ka, kb, pad; };
+
+struct SpecRow {             // one row of a spectrogram (K9); nc and cap count frames
+  int64_t src_off;           // floats into the source
+  int64_t dst_off;           // floats into the destination
+  int64_t len;               // samples
+  int64_t nc;                // frames of the row
+  int64_t cap;               // frames written (the first min(nc, cap) computed, the rest zeros)
+};
 
 
 // Ordered-int encoding so that atomicMax on int implements a signed float max.

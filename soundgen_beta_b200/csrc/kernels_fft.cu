@@ -207,12 +207,18 @@ __device__ __forceinline__ void pass_ct(XIn x, float2 *__restrict__ y, const flo
   }
 }
 
+// Bin kk of each of the two real frames packed as Z = A + iB: zk = Z[kk], zm = Z[(N - kk) mod N].
+__device__ __forceinline__ void pair_split(float2 zk, float2 zm, float2 *XA, float2 *XB) {
+  *XA = make_float2(0.5f * (zk.x + zm.x), 0.5f * (zk.y - zm.y));      // (zk + conj(zm)) / 2
+  *XB = make_float2(0.5f * (zk.y + zm.y), -0.5f * (zk.x - zm.x));     // (zk - conj(zm)) / (2i)
+}
+
 // Spectrum of one bin pair of the two packed frames (seewave.r:7806, soundgen.R:790-795, seewave.r:3470-3474):
 // zk = Z[kk], zm = Z[N - kk], 0 < kk < N/2.  Returns the packed filtered pair for the inverse transform.
 __device__ __forceinline__ void spec_pair(float2 zk, float2 zm, float ea, float eb, float2 *outk, float2 *outm,
                                           float *nyqA, float *nyqB) {
-  const float2 XA = make_float2(0.5f * (zk.x + zm.x), 0.5f * (zk.y - zm.y));      // (zk + conj(zm)) / 2
-  const float2 XB = make_float2(0.5f * (zk.y + zm.y), -0.5f * (zk.x - zm.x));     // (zk - conj(zm)) / (2i)
+  float2 XA, XB;
+  pair_split(zk, zm, &XA, &XB);
   const float2 FA = make_float2(ea * XA.x, ea * XA.y), FB = make_float2(eb * XB.x, eb * XB.y);
   *outk = make_float2(FA.x - FB.y, FA.y + FB.x);            // FA + i FB
   *outm = make_float2(FA.x + FB.y, FB.x - FA.y);            // conj(FA) + i conj(FB)
@@ -1109,4 +1115,140 @@ cudaError_t launch_stft(int mode, int u_is_float, int spec, const FftSeg *segs, 
     default: return launch_spec<0>(mode, u_is_float, segs, n_segs, jobs, plans, tw, win, in_f, in_u, env, out, maxpool, smem, st);
   }
 #undef SGB_CASE
+}
+
+// ---------------------------------------------------------------------------------------------------
+// K9: power / banded / dB spectrogram of float32 rows into caller-owned memory (sgb_batch_spectrogram,
+// sgb_rows_spectrogram).  The forward half of K2: frames start at R's truncated 1 + k h (frame_in_start), two real
+// frames share one complex FFT, a pair's input is staged by one TMA bulk copy into a double buffer while the
+// previous pair is transformed.  Epilogue: split the two spectra, |X|^2, optional projection onto contiguous bands
+// (weights staged in shared memory), optional 10 log10(max(F, floor)), coalesced stores at any dst alignment.
+// A CTA walks one segment: frames [ka, kb) of one row (ka even), or, when ka >= nc, the zero tail [ka, kb).
+// Frame 2m is always transformed together with frame 2m + 1 (when that frame exists, whether or not it is stored),
+// so a row's bits do not depend on its segmentation, on its capacity or on the other rows of the launch.
+__global__ void __launch_bounds__(STFT_THREADS)
+k_spectrogram(const FftSeg *__restrict__ segs, const SpecRow *__restrict__ rows, const FftPlan pl,
+              const float2 *__restrict__ twg, const float *__restrict__ win, const float *__restrict__ src,
+              int n_bands, const int32_t *__restrict__ band_tab, const float *__restrict__ band_w, int n_w, int db,
+              float db_floor, float *__restrict__ dst) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ uint64_t bars[2];
+  const FftSeg sg = segs[blockIdx.x];
+  const SpecRow R = rows[sg.job];
+  const int N = pl.n, nr = N / 2, nf = n_bands ? n_bands : nr;
+  float *out = dst + R.dst_off;
+  if (sg.ka >= R.nc) {                      // zero tail: frames [ka, kb) of the row, no transform
+    const int64_t a = (int64_t)sg.ka * nf, e = (int64_t)sg.kb * nf;
+    for (int64_t i = a + threadIdx.x; i < e; i += STFT_THREADS) __stcs(out + i, 0.0f);
+    return;
+  }
+  const int stage_len = (N + (int)ceil(pl.h_in) + 12) & ~3;
+  float2 *bufA = reinterpret_cast<float2 *>(smem_raw);
+  float2 *bufB = bufA + N;
+  float2 *tw = bufB + N;
+  float *stage0 = reinterpret_cast<float *>(tw + N);
+  float *stage1 = stage0 + stage_len;
+  int32_t *blo = reinterpret_cast<int32_t *>(stage1 + stage_len), *blen = blo + n_bands, *boff = blen + n_bands;
+  float *bw = reinterpret_cast<float *>(boff + n_bands);
+  for (int i = threadIdx.x; i < N; i += STFT_THREADS) tw[i] = twg[i];
+  for (int i = threadIdx.x; i < 3 * n_bands; i += STFT_THREADS) blo[i] = band_tab[i];
+  for (int i = threadIdx.x; i < n_w; i += STFT_THREADS) bw[i] = band_w[i];
+  const float *x = src + R.src_off;
+  // a row shorter than the window has one frame, read past the row's end as zeros: plain loads, no TMA
+  const bool short_row = R.len < N;
+  if (short_row) {
+    for (int i = threadIdx.x; i < N; i += STFT_THREADS) stage0[i] = (i < R.len) ? x[i] : 0.0f;
+  } else if (threadIdx.x == 0) {
+    mbar_init(&bars[0], 1);
+    mbar_init(&bars[1], 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  __syncthreads();
+
+  // frames k, k+1 need input [s_k, s_{k+1} + N); the copy is widened to 16-byte boundaries of the address, which
+  // stay inside the allocation (allocations are aligned far coarser than that)
+  uint32_t phase[2] = {0u, 0u};
+  auto stage_shift = [&](int k) { return (int)(((uintptr_t)(x + frame_in_start(pl, k)) & 15u) >> 2); };
+  auto issue_load = [&](int k, int buf) {
+    const int sA = frame_in_start(pl, k), sB = frame_in_start(pl, min(k + 1, (int)R.nc - 1));
+    const int d = stage_shift(k);
+    int cnt = (d + sB - sA + N + 3) & ~3;
+    if (cnt > stage_len) cnt = stage_len;
+    const uint32_t bytes = (uint32_t)cnt * 4u;
+    mbar_expect_tx(&bars[buf], bytes);
+    tma_load_1d(buf ? stage1 : stage0, x + sA - d, bytes, &bars[buf]);
+  };
+  if (!short_row && threadIdx.x == 0) issue_load(sg.ka, 0);
+
+  int cur = 0;
+  for (int k = sg.ka; k < sg.kb; k += 2) {
+    const bool hasB = k + 1 < R.nc;
+    const bool keepA = k < R.cap, keepB = hasB && k + 1 < R.cap;
+    const float *st = stage0;
+    int d = 0;
+    if (!short_row) {
+      if (!mbar_wait(&bars[cur], phase[cur])) return;   // sets g_stft_timeout
+      phase[cur] ^= 1u;
+      if (threadIdx.x == 0 && k + 2 < sg.kb) issue_load(k + 2, cur ^ 1);
+      st = cur ? stage1 : stage0;
+      d = stage_shift(k);
+    }
+    WinIn W;
+    W.a = st + d; W.b = st + d + (hasB ? frame_in_start(pl, k + 1) - frame_in_start(pl, k) : 0);
+    W.w = win; W.off = 0; W.hasB = hasB;
+    OlaOut O0 = {};
+    float2 *Z;
+    if (pl.radix[0] <= 5 || pl.radix[0] == 8) {
+      Z = fft_run<-1, true, false>(bufA, bufB, pl, tw, W, O0);
+    } else {   // a large prime first radix reads every input (r + 1) / 2 times: window the frames once
+      for (int i = threadIdx.x; i < N; i += STFT_THREADS) bufA[i] = W[i];
+      __syncthreads();
+      Z = fft_run<-1, false, false>(bufA, bufB, pl, tw, W, O0);
+    }
+    // all generic-proxy reads of this staging buffer are done: make it safe for the next TMA write
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    float *oA = out + (int64_t)k * nf, *oB = oA + nf;
+    float *P = reinterpret_cast<float *>(Z == bufA ? bufB : bufA);      // power of frame A, then of frame B
+    for (int kk = threadIdx.x; kk < nr; kk += STFT_THREADS) {
+      float2 XA, XB;
+      pair_split(Z[kk], Z[kk ? N - kk : 0], &XA, &XB);
+      const float pa = XA.x * XA.x + XA.y * XA.y, pb = XB.x * XB.x + XB.y * XB.y;
+      if (n_bands) {
+        P[kk] = pa; P[nr + kk] = pb;
+      } else {
+        if (keepA) __stcs(oA + kk, db ? 10.0f * log10f(fmaxf(pa, db_floor)) : pa);
+        if (keepB) __stcs(oB + kk, db ? 10.0f * log10f(fmaxf(pb, db_floor)) : pb);
+      }
+    }
+    if (n_bands) {
+      __syncthreads();
+      for (int i = threadIdx.x; i < 2 * n_bands; i += STFT_THREADS) {
+        const int f = i >= n_bands, b = i - f * n_bands;
+        if (!(f ? keepB : keepA)) continue;
+        const float *pp = P + f * nr + blo[b], *ww = bw + boff[b];
+        float acc = 0.0f;
+        for (int j = 0; j < blen[b]; j++) acc = fmaf(ww[j], pp[j], acc);
+        __stcs((f ? oB : oA) + b, db ? 10.0f * log10f(fmaxf(acc, db_floor)) : acc);
+      }
+    }
+    __syncthreads();
+    cur ^= 1;
+  }
+}
+
+size_t spectrogram_smem_bytes(int n, double h_in, int n_bands, int64_t n_w) {
+  const int stage_len = (n + (int)ceil(h_in) + 12) & ~3;
+  return (size_t)24 * n + 8 * (size_t)stage_len + 12 * (size_t)n_bands + 4 * (size_t)n_w;
+}
+
+cudaError_t launch_spectrogram(const FftSeg *segs, int n_segs, const SpecRow *rows, const FftPlan &pl, const float2 *tw,
+                               const float *win, const float *src, int n_bands, const int32_t *band_tab,
+                               const float *band_w, int n_w, int db, float db_floor, float *dst, size_t smem,
+                               cudaStream_t st) {
+  if (n_segs <= 0) return cudaSuccess;
+  cudaError_t e = ensure_smem(k_spectrogram, nullptr, smem);
+  if (e != cudaSuccess) return e;
+  k_spectrogram<<<n_segs, STFT_THREADS, smem, st>>>(segs, rows, pl, tw, win, src, n_bands, band_tab, band_w, n_w, db,
+                                                    db_floor, dst);
+  return cudaGetLastError();
 }
