@@ -288,6 +288,38 @@ int sgb_batch_spectrogram(sgb_batch *b, const sgb_spec_params *p, const sgb_devi
 int sgb_rows_spectrogram(int32_t device, const float *src, const int64_t *src_off, const int64_t *len,
                          int32_t n, const sgb_spec_params *p, const sgb_device_out *o);
 
+/* Similarity of spectrogram rows on the device (K10), one float64 score per pair into caller-owned device memory.
+ * Pair c compares row a_c (a_frames[c] frames of n_feat floats, frame after frame, from element a_off[c] of a) with
+ * row b_c (likewise in b); pairs may share rows.  With N = max(n_a, n_b), the frames past the shorter row read as
+ * `pad` in every feature:
+ *   SGB_CMP_COR     Pearson correlation over the N * n_feat cells (two-pass, FP64);
+ *   SGB_CMP_COSINE  <a, b> / (|a| |b|) over the same cells (FP64);
+ *   SGB_CMP_DTW     -D(n_a, n_b) / (n_a + n_b), no padding: cell cost d(i, j) = |a_i - b_j|_2 over the features (FP32),
+ *                   step pattern symmetric2 of R's dtw package, D(1, 1) = d(1, 1) and
+ *                   D(i, j) = min(D(i-1, j-1) + 2 d, D(i-1, j) + d, D(i, j-1) + d) (FP64).
+ * Higher is more similar.  A row with 0 frames gives NaN, and so does a constant side (cor) or an all-zero side
+ * (cosine), as 0/0 does.  A pair's score does not depend on the other pairs, their order or their number.
+ * dst gets n scores (8-byte aligned device memory of `device`, dst_elems >= n); a and b must be device memory of
+ * `device` (checked when a row of that side has frames).  The stream contract and pinned staging are those of the
+ * exports: ordered after the work queued on `stream` so far, and the caller's later work on `stream` sees dst, with
+ * no host wait.  Refused before anything is queued: an unknown method, n_feat < 1, a non-finite pad, negative
+ * offsets or frames, a row outside a_elems / b_elems, or bad pointers give SGB_ERR_INVALID; a DTW row of more than
+ * SGB_CMP_DTW_MAX_FRAMES frames gives SGB_ERR_UNSUPPORTED (its wavefront lives in shared memory). */
+#define SGB_CMP_COR    0
+#define SGB_CMP_COSINE 1
+#define SGB_CMP_DTW    2
+#define SGB_CMP_DTW_MAX_FRAMES 4096
+typedef struct sgb_compare_params {
+  int32_t method, n_feat;        /* SGB_CMP_*; floats per frame                                     */
+  double  pad;                   /* value of the frames past the shorter row (cor, cosine)          */
+} sgb_compare_params;
+int sgb_rows_compare(int32_t device, const float *a, int64_t a_elems, const float *b, int64_t b_elems,
+                     const int64_t *a_off, const int64_t *a_frames, const int64_t *b_off, const int64_t *b_frames,
+                     int32_t n, const sgb_compare_params *p, double *dst, int64_t dst_elems, void *stream);
+/* default, low and high of a scalar argument of soundgen() as the front-end checks it (permittedValues,
+ * R/presets.R:22-79); SGB_ERR_INVALID for a name the front-end does not range-check. */
+int sgb_param_range(const char *name, double out3[3]);
+
 /* Intermediate results (valid after run).  Sizes via the *_len calls. */
 int sgb_batch_syllable_len(sgb_batch *b, int32_t syl, int64_t *out_len);
 int sgb_batch_syllable_fetch(sgb_batch *b, int32_t syl, double *out, int64_t n);
@@ -325,8 +357,8 @@ int sgb_batch_set_tracks(sgb_batch *b, int32_t env, const double *rows, int32_t 
 /* Normal draws each voiced syllable consumed (valid after run_begin); n_syllables values. */
 int sgb_batch_z_used(sgb_batch *b, int32_t *out);
 /* sizeof() of the ABI structs, for bindings to verify their mirrors:
- * syllable, envelope, noise, bout, call, formant_ref, batch_desc, run_info, soundgen_args, device_out, spec_params
- * (cap >= 9; the 10th and 11th are written when cap allows). */
+ * syllable, envelope, noise, bout, call, formant_ref, batch_desc, run_info, soundgen_args, device_out, spec_params,
+ * compare_params (cap >= 9; the 10th to 12th are written when cap allows). */
 int sgb_abi_sizes(int32_t *out, int32_t cap);
 /* The additive synthesis has two kernels: epochs with at least `rows` rows run on the tensor cores, the others on the
    FP32 pipe (default 224, or SGB_SYNTH / SGB_SYNTH_MIN_ROWS from the environment).  0 = tensor cores only, a huge value =

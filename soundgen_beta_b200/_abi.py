@@ -12,6 +12,8 @@ SGB_ERR_SYNTH, SGB_ERR_STREAM, SGB_ERR_STATE = -4, -5, -6
 SGB_CONTOUR_LOESS, SGB_CONTOUR_SPLINE = 0, 1
 SGB_OUT_F32, SGB_OUT_PCM16 = 0, 1
 SGB_WIN_HAMMING, SGB_WIN_HANNING = 0, 1
+SGB_CMP_COR, SGB_CMP_COSINE, SGB_CMP_DTW = 0, 1, 2
+SGB_CMP_DTW_MAX_FRAMES = 4096
 
 SYL_DOUBLES = ['attackLen', 'nonlinBalance', 'jitterDep', 'jitterLen', 'vibratoFreq',
                'vibratoDep', 'shimmerDep', 'rolloff', 'rolloffOct', 'rolloffKHz', 'rolloffParab',
@@ -116,6 +118,10 @@ class SpecParams(C.Structure):
                 ('band_lo', C.c_void_p), ('band_len', C.c_void_p), ('band_w', C.c_void_p)]
 
 
+class CompareParams(C.Structure):
+    _fields_ = [('method', i32), ('n_feat', i32), ('pad', f64)]
+
+
 T_NAMES = ['h2d', 'control', 'ampl', 'synth', 'compose', 'noise', 'assemble', 'envelope',
            'filter', 'finalize', 'd2h', 'total']
 
@@ -137,6 +143,7 @@ EXPORTS = ['sgb_version', 'sgb_last_error', 'sgb_device_count', 'sgb_set_device'
            'sgb_batch_create', 'sgb_batch_destroy', 'sgb_batch_upload', 'sgb_batch_run',
            'sgb_batch_lengths', 'sgb_batch_fetch_f32', 'sgb_batch_fetch_f64', 'sgb_batch_fetch_pcm16', 'sgb_batch_status',
            'sgb_batch_export', 'sgb_rows_export', 'sgb_spec_frames', 'sgb_batch_spectrogram', 'sgb_rows_spectrogram',
+           'sgb_rows_compare', 'sgb_param_range',
            'sgb_batch_syllable_len', 'sgb_batch_syllable_fetch', 'sgb_batch_noise_fetch',
            'sgb_batch_artefacts', 'sgb_batch_artefact_ints', 'sgb_batch_pitch_per_gc', 'sgb_batch_checksums', 'sgb_batch_debug_state',
            'sgb_get_rolloff', 'sgb_get_spectral_envelope', 'sgb_filter_len', 'sgb_filter',
@@ -191,6 +198,8 @@ def load():
     L.sgb_spec_frames.restype = i64
     L.sgb_batch_spectrogram.argtypes = [vp, C.POINTER(SpecParams), C.POINTER(DeviceOut)]
     L.sgb_rows_spectrogram.argtypes = [i32, vp, vp, vp, i32, C.POINTER(SpecParams), C.POINTER(DeviceOut)]
+    L.sgb_rows_compare.argtypes = [i32, vp, i64, vp, i64, vp, vp, vp, vp, i32, C.POINTER(CompareParams), vp, i64, vp]
+    L.sgb_param_range.argtypes = [C.c_char_p, vp]
     L.sgb_batch_syllable_len.argtypes = [vp, i32, C.POINTER(i64)]
     L.sgb_batch_syllable_fetch.argtypes = [vp, i32, vp, i64]
     L.sgb_batch_noise_fetch.argtypes = [vp, i32, vp, i64]
@@ -232,10 +241,10 @@ def load():
     L.sgb_frontend_h2d_bytes.restype = i64
     L.sgb_rng_draw.argtypes = [C.c_uint32, i32, f64, f64, i32, vp, i32]
     L.sgb_smooth_contour.argtypes = [vp, vp, i32, i32, f64, i32, f64, i32, f64, i32, i32, vp]
-    sizes = (i32 * 11)()
-    L.sgb_abi_sizes(sizes, 11)
+    sizes = (i32 * 12)()
+    L.sgb_abi_sizes(sizes, 12)
     mine = [C.sizeof(t) for t in (Syllable, Envelope, Noise, Bout, Call, FormantRef, BatchDesc, RunInfo, SoundgenArgs,
-                                  DeviceOut, SpecParams)]
+                                  DeviceOut, SpecParams, CompareParams)]
     if list(sizes) != mine:
         raise RuntimeError('ctypes mirror out of date: library struct sizes %s, mirror %s' % (list(sizes), mine))
     _lib = L

@@ -1048,6 +1048,183 @@ def soundgen_batch_device(calls, dtype=None, device=None, max_len=None, u_dtype=
     return wave, lengths, status
 
 
+_CMP_METHODS = {'cor': _abi.SGB_CMP_COR, 'cosine': _abi.SGB_CMP_COSINE, 'dtw': _abi.SGB_CMP_DTW}
+
+
+def _host_counts(x, n, hi, what):
+    import torch
+    v = (x.cpu().numpy() if torch.is_tensor(x) else np.asarray(x)).astype(np.int64).reshape(-1)
+    if v.shape != (n,) or np.any(v < 0) or np.any(v > hi):
+        raise ValueError('%s needs one value in [0, %d] per row (%d)' % (what, hi, n))
+    return v
+
+
+def compare_spectrograms(a, a_frames, b, b_frames, method='cor', pairs=None, pad=0.0, stream=None):
+    """Similarity of spectrogram rows on the device (K10, sgb_rows_compare): a [n, F, n_feat] and b [m, F', n_feat]
+    are float32 CUDA tensors as spectrogram_device returns them, a_frames / b_frames the frames present per row (host
+    or CUDA; a CUDA tensor is read back once).  Row c of a is scored against row pairs[c] of b (default: row 0 when
+    m == 1, else row c).  method: 'cor' (Pearson correlation), 'cosine' or 'dtw' (minus the normalised symmetric2 DTW
+    distance); for cor and cosine the frames past the shorter row of a pair read as `pad`.  Higher is more similar;
+    NaN for a row without frames, a constant side (cor) or an all-zero side (cosine).  Returns a float64 CUDA
+    tensor [n], ordered on `stream` (default: the device's current torch stream) with no host wait."""
+    import torch
+    if method not in _CMP_METHODS:
+        raise ValueError("method must be 'cor', 'cosine' or 'dtw', not %r" % (method,))
+    for t, nm in ((a, 'a'), (b, 'b')):
+        if not (torch.is_tensor(t) and t.is_cuda and t.dtype == torch.float32 and t.dim() == 3 and t.is_contiguous()):
+            raise ValueError('%s must be a contiguous [rows, frames, n_feat] float32 CUDA tensor' % nm)
+    if a.device != b.device:
+        raise ValueError('a and b must be on one device')
+    n, Fa, nf = a.shape
+    m, Fb, nfb = b.shape
+    if nf != nfb or nf < 1:
+        raise ValueError('a and b need the same n_feat >= 1, not %d and %d' % (nf, nfb))
+    af = _host_counts(a_frames, n, Fa, 'a_frames')
+    bf = _host_counts(b_frames, m, Fb, 'b_frames')
+    if pairs is None:
+        if m != 1 and m != n:
+            raise ValueError('pairs is needed when b has neither one row nor one row per row of a')
+        pairs = np.zeros(n) if m == 1 else np.arange(n)
+    pr = np.asarray(pairs).reshape(-1)
+    if pr.shape != (n,) or not np.all((pr >= 0) & (pr < m) & (pr == np.floor(pr))):
+        raise ValueError('pairs needs one row index of b in [0, %d) per row of a (%d)' % (m, n))
+    pr = pr.astype(np.int64)
+    p = _abi.CompareParams()
+    p.method, p.n_feat, p.pad = _CMP_METHODS[method], nf, float(pad)
+    a_off = np.arange(n, dtype=np.int64) * Fa * nf
+    b_off = np.ascontiguousarray(pr * Fb * nf)
+    b_fr = np.ascontiguousarray(bf[pr])
+    dst = torch.empty(n, dtype=torch.float64, device=a.device)
+    L = _abi.load()
+    _check(L.sgb_rows_compare(a.device.index, a.data_ptr() or None, a.numel(), b.data_ptr() or None, b.numel(),
+                              _ptr(a_off), _ptr(af), _ptr(b_off), _ptr(b_fr), n, C.byref(p), dst.data_ptr() or None,
+                              n, _stream_handle(stream, dst) or None))
+    return dst
+
+
+def param_range(name):
+    """(default, low, high) of a scalar soundgen() argument as the front-end range-checks it (permittedValues,
+    R/presets.R:22-79).  ValueError for a name it does not check."""
+    out = np.zeros(3)
+    if not isinstance(name, str) or _abi.load().sgb_param_range(name.encode(), _ptr(out)) != _abi.SGB_OK:
+        raise ValueError('%r is not a range-checked scalar argument of soundgen()' % (name,))
+    return float(out[0]), float(out[1]), float(out[2])
+
+
+# arguments match_pars does not search: the sampling rate and window set the analysis, temperature the draws, and
+# the counts of bouts and syllables change the structure of the call
+_NOT_SEARCHED = ('samplingRate', 'windowLength', 'temperature', 'repeatBout', 'nSyl')
+
+
+def _searched(pars):
+    pars = [pars] if isinstance(pars, str) else list(pars)
+    if not pars or len(set(pars)) != len(pars):
+        raise ValueError('pars must name one or more distinct arguments')
+    for nm in pars:
+        if nm in _NOT_SEARCHED:
+            raise ValueError('%s cannot be searched (not one of %s)' % (nm, ', '.join(_NOT_SEARCHED)))
+        param_range(nm)
+    return pars
+
+
+def wiggle_pars(values, pars, prob_mutation=0.25, step_variance=0.1, rng=None):
+    """One mutation of `values` (a dict holding every name of `pars`), drawn from the numpy Generator `rng` (or a
+    seed): each name of pars changes with probability prob_mutation, and one chosen at random when none did, to a
+    normal draw with mean its value and sd step_variance * (high - low), redrawn up to 100 times until it falls in
+    [low, high] of param_range, then clipped.  Returns a new dict; the other entries are copied unchanged."""
+    pars = _searched(pars)
+    if not 0.0 <= float(prob_mutation) <= 1.0 or not float(step_variance) > 0.0:
+        raise ValueError('need 0 <= prob_mutation <= 1 and step_variance > 0')
+    rng = rng if isinstance(rng, np.random.Generator) else np.random.default_rng(rng)
+    out = dict(values)
+    mutate = rng.random(len(pars)) < float(prob_mutation)
+    if not mutate.any():
+        mutate[rng.integers(len(pars))] = True
+    for nm, mu in zip(pars, mutate):
+        if not mu:
+            continue
+        _, lo, hi = param_range(nm)
+        mean, sd = float(values[nm]), float(step_variance) * (hi - lo)
+        for _ in range(100):
+            v = float(rng.normal(mean, sd))
+            if lo <= v <= hi:
+                break
+        out[nm] = min(max(v, lo), hi)
+    return out
+
+
+_DB_FLOOR = 1e-10
+
+
+def match_pars(target, samplingRate, pars, base=None, n_candidates=64, max_iter=50, prob_mutation=0.25,
+               step_variance=0.1, method='cor', min_delta=0.0, windowLength=40, overlap=50, n_mels=64, seed=0):
+    """Searches soundgen() arguments for a call that sounds like `target` (a 1-D float32 waveform, numpy or CUDA, at
+    samplingRate): a hill-climb in the manner of the reference's matchPars that tries n_candidates mutations of the
+    current best per step on the GPU.  base: the fixed arguments (temperature defaults to 0); pars: the scalar
+    arguments searched, starting from their values in base (or soundgen()'s defaults).  Each step draws the
+    candidates with wiggle_pars, synthesises them at samplingRate (soundgen_batch_device), takes their log-mel
+    spectrograms as the target's (spectrogram_device with windowLength, overlap, n_mels, db=True) and scores them
+    against it (compare_spectrograms with `method`; missing frames read as the dB floor, i.e. silence).  A candidate
+    with a non-zero status or a NaN score counts as -inf.  The best candidate replaces the current one when its score
+    beats the current score by more than min_delta.
+    Returns (best_kwargs, best_score, history): history[0] is the starting point, history[k] step k, each a dict with
+    'score' (the step's best), 'accepted', 'values' ([candidates, len(pars)] array of the values tried) and 'best'
+    (the current score after the step).  The same seed, inputs and n_candidates give the same history, bit for bit.
+    This is not R's matchPars: the draws come from numpy's generator, not R's stream, and the features are this
+    library's log-mel spectrograms, not tuneR::melfcc."""
+    import torch
+    pars = _searched(pars)
+    if method not in _CMP_METHODS:
+        raise ValueError("method must be 'cor', 'cosine' or 'dtw', not %r" % (method,))
+    if int(n_candidates) < 1 or int(max_iter) < 0:
+        raise ValueError('need n_candidates >= 1 and max_iter >= 0')
+    sr = float(samplingRate)
+    kw = dict(temperature=0)
+    kw.update(base or {})
+    if kw.get('samplingRate', sr) != sr:
+        raise ValueError('base sets samplingRate %r, the target is at %r' % (kw['samplingRate'], sr))
+    kw['samplingRate'] = sr
+    _, lo, hi = param_range('samplingRate')
+    if not lo <= sr <= hi and kw.get('invalidArgAction', 'adjust') != 'ignore':
+        raise ValueError("samplingRate %g is outside [%g, %g]: the front-end would not synthesise at it unless base "
+                         "sets invalidArgAction='ignore'" % (sr, lo, hi))
+    if torch.is_tensor(target):
+        dev = target.device if target.is_cuda else torch.device('cuda', torch.cuda.current_device())
+        x = target.to(dev, torch.float32)
+    else:
+        dev = torch.device('cuda', torch.cuda.current_device())
+        x = torch.as_tensor(np.asarray(target, dtype=np.float32), device=dev)
+    if x.dim() != 1:
+        raise ValueError('target must be a 1-D waveform')
+    spec_kw = dict(windowLength=windowLength, overlap=overlap, n_mels=int(n_mels), db=True, db_floor=_DB_FLOOR)
+    tgt, tgt_frames = spectrogram_device(x.reshape(1, -1).contiguous(), [x.numel()], sr, **spec_kw)
+    pad = 10.0 * math.log10(_DB_FLOOR)
+
+    def best_of(cands):
+        wave, lengths, status = soundgen_batch_device([dict(kw, **c) for c in cands], device=dev.index)
+        spec, frames = spectrogram_device(wave, lengths, sr, **spec_kw)
+        s = compare_spectrograms(spec, frames, tgt, tgt_frames, method, pad=pad)
+        bad = torch.as_tensor(np.asarray(status) != 0, device=dev) | torch.isnan(s)
+        s = torch.where(bad, torch.full_like(s, -math.inf), s)
+        i = torch.argmax(s)                       # the first of equal maxima
+        got = torch.stack((s[i], i.to(torch.float64))).cpu()
+        return float(got[0]), int(got[1])
+
+    cur = {nm: float(kw.get(nm, SOUNDGEN_DEFAULTS[nm])) for nm in pars}
+    best = best_of([cur])[0]
+    history = [dict(score=best, accepted=True, values=np.array([[cur[nm] for nm in pars]]), best=best)]
+    rng = np.random.default_rng(seed)
+    for _ in range(int(max_iter)):
+        cands = [wiggle_pars(cur, pars, prob_mutation, step_variance, rng) for _ in range(int(n_candidates))]
+        s, i = best_of(cands)
+        accepted = s > best + min_delta
+        if accepted:
+            cur, best = cands[i], s
+        history.append(dict(score=s, accepted=accepted, values=np.array([[c[nm] for nm in pars] for c in cands]),
+                            best=best))
+    return dict(kw, **cur), best, history
+
+
 class PipelinedBatches:
     """Several sub-batches, each with its own handle / CUDA stream, driven as a three-stage software
     pipeline: one thread uploads (H2D copy engine), `runners` threads run the kernels (two, so that the

@@ -53,6 +53,9 @@ size_t spectrogram_smem_bytes(int n, double h_in, int n_bands, int64_t n_w);
 cudaError_t launch_spectrogram(const FftSeg *, int, const SpecRow *, const FftPlan &, const float2 *, const float *,
                                const float *, int, const int32_t *, const float *, int, int, float, float *, size_t,
                                cudaStream_t);
+size_t spec_compare_smem_bytes(int method, int64_t max_short);
+cudaError_t launch_spec_compare(const float *, const float *, const void *, int, int, int, double, int64_t, double *,
+                                cudaStream_t);
 void launch_noise_final(const sgb_noise *, int, const NoiseLayout *, const double *, const double *, const int *, int,
                         const float *, float *, void *, double *, const int64_t *, int, cudaStream_t);
 size_t contour_tab_bytes();
@@ -1371,9 +1374,10 @@ int sgb_abi_sizes(int32_t *out, int32_t cap) {
   const int32_t v[] = {(int32_t)sizeof(sgb_syllable), (int32_t)sizeof(sgb_envelope), (int32_t)sizeof(sgb_noise),
                        (int32_t)sizeof(sgb_bout), (int32_t)sizeof(sgb_call), (int32_t)sizeof(sgb_formant_ref),
                        (int32_t)sizeof(sgb_batch_desc), (int32_t)sizeof(sgb_run_info), (int32_t)sizeof(sgb_soundgen_args),
-                       (int32_t)sizeof(sgb_device_out), (int32_t)sizeof(sgb_spec_params)};
+                       (int32_t)sizeof(sgb_device_out), (int32_t)sizeof(sgb_spec_params),
+                       (int32_t)sizeof(sgb_compare_params)};
   if (!out || cap < 9) return fail(SGB_ERR_INVALID, "need room for 9 sizes");
-  for (int i = 0; i < 11 && i < cap; i++) out[i] = v[i];
+  for (int i = 0; i < 12 && i < cap; i++) out[i] = v[i];
   return SGB_OK;
 }
 
@@ -1446,6 +1450,17 @@ int sgb_batch_fetch_pcm16(sgb_batch *b, int16_t *out, int64_t n) {
 }
 
 // ---- device output (sgb_batch_export / sgb_rows_export, sgb_batch_spectrogram / sgb_rows_spectrogram) ----
+// `p` must be device (or managed) memory of `device`.
+static int on_device(int device, const void *p, const char *what) {
+  cudaPointerAttributes a;
+  cudaError_t e = cudaPointerGetAttributes(&a, p);
+  if (e != cudaSuccess) { cudaGetLastError(); return fail(SGB_ERR_INVALID, "%s: not a CUDA allocation (%s)", what, cudaGetErrorString(e)); }
+  if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
+    return fail(SGB_ERR_INVALID, "%s is host memory (pinned or pageable), not device memory", what);
+  if (a.device != device) return fail(SGB_ERR_INVALID, "%s is memory of device %d, not of device %d", what, a.device, device);
+  return SGB_OK;
+}
+
 // Checks everything the host can check before anything is queued.  `src` (the rows entries) is checked like dst.
 // Row c occupies cap[c] * unit elements of dst (unit: floats per frame of a spectrogram, 1 for the exports).
 static int export_check(int device, const float *src, const int64_t *src_off, const int64_t *len, int32_t n,
@@ -1455,15 +1470,6 @@ static int export_check(int device, const float *src, const int64_t *src_off, co
     return fail(SGB_ERR_INVALID, "unsupported output format %d", o->format);
   if (n < 0 || o->dst_elems < 0) return fail(SGB_ERR_INVALID, "negative row count or dst_elems");
   if (n > 0 && (!o->dst_off || !o->cap || !len || (src && !src_off))) return fail(SGB_ERR_INVALID, "null row table");
-  auto on_device = [&](const void *p, const char *what) -> int {
-    cudaPointerAttributes a;
-    cudaError_t e = cudaPointerGetAttributes(&a, p);
-    if (e != cudaSuccess) { cudaGetLastError(); return fail(SGB_ERR_INVALID, "%s: not a CUDA allocation (%s)", what, cudaGetErrorString(e)); }
-    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
-      return fail(SGB_ERR_INVALID, "%s is host memory (pinned or pageable), not device memory", what);
-    if (a.device != device) return fail(SGB_ERR_INVALID, "%s is memory of device %d, not of device %d", what, a.device, device);
-    return SGB_OK;
-  };
   std::vector<std::pair<int64_t, int64_t>> rows;
   rows.reserve((size_t)n);
   for (int32_t c = 0; c < n; c++) {
@@ -1483,23 +1489,22 @@ static int export_check(int device, const float *src, const int64_t *src_off, co
     if (!o->dst) return fail(SGB_ERR_INVALID, "null dst");
     const size_t esz = o->format == SGB_OUT_F32 ? 4 : 2;
     if ((uintptr_t)o->dst % esz) return fail(SGB_ERR_INVALID, "dst is not aligned to its element type");
-    int rc = on_device(o->dst, "dst");
+    int rc = on_device(device, o->dst, "dst");
     if (rc != SGB_OK) return rc;
   }
   if (src) {
     if ((uintptr_t)src % 4) return fail(SGB_ERR_INVALID, "src is not aligned to float");
-    int rc = on_device(src, "src");
+    int rc = on_device(device, src, "src");
     if (rc != SGB_OK) return rc;
   }
   return SGB_OK;
 }
 
-// Queues work on `st` (the handle's stream, or the device's export stream) ordered against the caller's stream as
-// the header describes.  fill(h) writes `bytes` of host-built tables into a pinned staging slot; launch(d) queues
-// the kernels on their device copy.  Arguments were checked by export_check.
-static int export_queue(ExportCtx &X, cudaStream_t st, const sgb_device_out *o, size_t bytes,
+// Queues work on `st` (the handle's stream, or the device's export stream) ordered against the caller's stream
+// `user` as the header describes.  fill(h) writes `bytes` of host-built tables into a pinned staging slot; launch(d)
+// queues the kernels on their device copy.  Arguments were checked before.
+static int export_queue(ExportCtx &X, cudaStream_t st, cudaStream_t user, size_t bytes,
                         const std::function<void(char *)> &fill, const std::function<int(const char *)> &launch) {
-  cudaStream_t user = (cudaStream_t)o->stream;
   if (!X.ev_in) CK(cudaEventCreateWithFlags(&X.ev_in, cudaEventDisableTiming));
   ExportSlot *S = nullptr;
   for (auto s : X.slots) {
@@ -1558,7 +1563,7 @@ static int export_rows(ExportCtx &X, cudaStream_t st, const float *src, const in
     }
     return SGB_OK;
   };
-  int rc = export_queue(X, st, o, bytes, fill, launch);
+  int rc = export_queue(X, st, (cudaStream_t)o->stream, bytes, fill, launch);
   if (rc != SGB_OK) return rc;
   if (o->out_written)
     for (int32_t c = 0; c < n; c++) o->out_written[c] = std::min(len[c], o->cap[c]);
@@ -1772,7 +1777,7 @@ static int spec_queue(ExportCtx &X, cudaStream_t st, const float *src, const Spe
     }
     return SGB_OK;
   };
-  int rc = export_queue(X, st, o, bytes, fill, launch);
+  int rc = export_queue(X, st, (cudaStream_t)o->stream, bytes, fill, launch);
   if (rc != SGB_OK) return rc;
   if (o->out_written)
     for (size_t c = 0; c < J.rows.size(); c++) o->out_written[c] = std::min(J.rows[c].nc, J.rows[c].cap);
@@ -1808,6 +1813,67 @@ int sgb_rows_spectrogram(int32_t device, const float *src, const int64_t *src_of
   if ((rc = device_export(device, &D)) != SGB_OK) return rc;
   std::lock_guard<std::mutex> g(D->mu);
   return spec_queue(D->x, D->st, src, J, p, o);
+}
+
+// ---- similarity of spectrogram rows (K10) ----
+int sgb_rows_compare(int32_t device, const float *a, int64_t a_elems, const float *b, int64_t b_elems,
+                     const int64_t *a_off, const int64_t *a_frames, const int64_t *b_off, const int64_t *b_frames,
+                     int32_t n, const sgb_compare_params *p, double *dst, int64_t dst_elems, void *stream) {
+  // the parameters and the row tables alone (no device needed)
+  if (!p) return fail(SGB_ERR_INVALID, "null sgb_compare_params");
+  if (p->method != SGB_CMP_COR && p->method != SGB_CMP_COSINE && p->method != SGB_CMP_DTW)
+    return fail(SGB_ERR_INVALID, "unknown method %d", p->method);
+  if (p->n_feat < 1) return fail(SGB_ERR_INVALID, "n_feat %d < 1", p->n_feat);
+  if (!std::isfinite(p->pad)) return fail(SGB_ERR_INVALID, "pad %g is not finite", p->pad);
+  if (n < 0 || a_elems < 0 || b_elems < 0 || dst_elems < 0) return fail(SGB_ERR_INVALID, "negative count");
+  if (n > 0 && (!a_off || !a_frames || !b_off || !b_frames)) return fail(SGB_ERR_INVALID, "null row table");
+  std::vector<int64_t> tab(4 * (size_t)n);       // a_off, a_frames, b_off, b_frames per pair (the kernel's Pair)
+  int64_t max_short = 0;
+  bool any_cells = false;                         // a pair with frames on both sides reads a and b
+  for (int32_t c = 0; c < n; c++) {
+    const int64_t ao = a_off[c], af = a_frames[c], bo = b_off[c], bf = b_frames[c];
+    if (ao < 0 || af < 0 || bo < 0 || bf < 0) return fail(SGB_ERR_INVALID, "pair %d: negative offset or frames", c);
+    if (ao > a_elems || af > (a_elems - ao) / p->n_feat)
+      return fail(SGB_ERR_INVALID, "pair %d: row of a [%lld, %lld x %d more) outside a (%lld elements)", c,
+                  (long long)ao, (long long)af, p->n_feat, (long long)a_elems);
+    if (bo > b_elems || bf > (b_elems - bo) / p->n_feat)
+      return fail(SGB_ERR_INVALID, "pair %d: row of b [%lld, %lld x %d more) outside b (%lld elements)", c,
+                  (long long)bo, (long long)bf, p->n_feat, (long long)b_elems);
+    if (p->method == SGB_CMP_DTW && (af > SGB_CMP_DTW_MAX_FRAMES || bf > SGB_CMP_DTW_MAX_FRAMES))
+      return fail(SGB_ERR_UNSUPPORTED, "pair %d: DTW over %lld x %lld frames (at most %d per row)", c, (long long)af,
+                  (long long)bf, SGB_CMP_DTW_MAX_FRAMES);
+    if (af > 0 && bf > 0) {
+      any_cells = true;
+      max_short = std::max(max_short, std::min(af, bf));
+    }
+    tab[4 * (size_t)c] = ao; tab[4 * (size_t)c + 1] = af; tab[4 * (size_t)c + 2] = bo; tab[4 * (size_t)c + 3] = bf;
+  }
+  if (n > 0 && dst_elems < n) return fail(SGB_ERR_INVALID, "dst has %lld elements for %d scores", (long long)dst_elems, n);
+  int rc = rows_device_check(device, nullptr, 0);
+  if (rc != SGB_OK) return rc;
+  if (n == 0) return SGB_OK;
+  if (!dst) return fail(SGB_ERR_INVALID, "null dst");
+  if ((uintptr_t)dst % 8) return fail(SGB_ERR_INVALID, "dst is not aligned to double");
+  if ((rc = on_device(device, dst, "dst")) != SGB_OK) return rc;
+  if (any_cells) {
+    if (!a || (uintptr_t)a % 4 || !b || (uintptr_t)b % 4) return fail(SGB_ERR_INVALID, "null or misaligned a / b");
+    if ((rc = on_device(device, a, "a")) != SGB_OK || (rc = on_device(device, b, "b")) != SGB_OK) return rc;
+  }
+  DeviceExport *D;
+  if ((rc = device_export(device, &D)) != SGB_OK) return rc;
+  std::lock_guard<std::mutex> g(D->mu);
+  const size_t bytes = sizeof(int64_t) * tab.size();
+  auto fill = [&](char *h) { memcpy(h, tab.data(), bytes); };
+  auto launch = [&](const char *d) -> int {
+    cudaError_t e = launch_spec_compare(a, b, d, n, p->method, p->n_feat, p->pad, max_short, dst, D->st);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return fail(SGB_ERR_CUDA, "k_spec_compare launch failed (%d pairs, %zu bytes of shared memory): %s", n,
+                  spec_compare_smem_bytes(p->method, max_short), cudaGetErrorString(e));
+    }
+    return SGB_OK;
+  };
+  return export_queue(D->x, D->st, (cudaStream_t)stream, bytes, fill, launch);
 }
 
 // Diagnostic for a stuck run (callable from another thread): out[0] = which wait the handle's host thread

@@ -989,6 +989,14 @@ static void merge_shard(sgb_frontend *fe, Round &R, const Round &S) {
 
 extern "C" {
 
+int sgb_param_range(const char *name, double out3[3]) {
+  const Perm *q = name ? perm(name) : nullptr;
+  if (!q) return ffail(SGB_ERR_INVALID, "no permitted range for %s", name ? name : "(null)");
+  if (!out3) return ffail(SGB_ERR_INVALID, "null out3");
+  out3[0] = q->dflt; out3[1] = q->lo; out3[2] = q->hi;
+  return SGB_OK;
+}
+
 // test hook: worker threads of the host stage (0 = SGB_FRONTEND_THREADS / the default)
 int sgb_host_set_threads(int32_t n) { sgb_host_threads_override().store(n > 0 ? n : 0); return SGB_OK; }
 
