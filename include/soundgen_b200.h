@@ -316,6 +316,35 @@ typedef struct sgb_compare_params {
 int sgb_rows_compare(int32_t device, const float *a, int64_t a_elems, const float *b, int64_t b_elems,
                      const int64_t *a_off, const int64_t *a_frames, const int64_t *b_off, const int64_t *b_frames,
                      int32_t n, const sgb_compare_params *p, double *dst, int64_t dst_elems, void *stream);
+/* Cepstra and their deltas of spectrogram rows on the device (K11), into caller-owned device memory.  Row c has
+ * frames[c] = nc frames of n_in floats, frame after frame, from element src_off[c] of src (rows as
+ * sgb_rows_spectrogram writes them, typically log-mel).  With the caller's matrix M [n_ceps, n_in] (row-major,
+ * e.g. an orthonormal DCT-II for MFCCs), for frame t of a row:
+ *   cepstra  c_t[k] = sum_b M[k, b] x_t[b], FP32 in a fixed order of b;
+ *   deltas   order 1, N = delta_n in 1..8:
+ *            d_t = (sum_{j=1..N} j (c_{min(t+j, nc-1)} - c_{max(t-j, 0)})) / (2 sum_{j=1..N} j^2),
+ *            the row's first and last frames replicated at its edges (torchaudio's compute_deltas with
+ *            win_length 2N + 1 over the row's nc frames alone); order 2 adds the same formula over the d_t;
+ *   output   frame t = [c_t | d_t | dd_t], n_out = n_ceps (1 + delta_order) floats.
+ * Layout as sgb_device_out describes it, with cap counted in frames: row c gets exactly cap[c] frames of n_out
+ * floats from element dst_off[c] on; frames >= nc are zeros; out_written[c] = min(nc, cap[c]); a row with
+ * cap[c] = 0 is left alone.  format must be SGB_OUT_F32.  Frames at or past nc are never read, and the deltas near
+ * cap read the input past cap (up to nc): a row's values do not depend on cap or on the other rows, so a cropped
+ * row is a bit-exact prefix of the whole one.  Stream contract and pinned staging are those of the exports.
+ * Refused before anything is queued: n_in or n_ceps < 1, a null or non-finite matrix, delta_order not in {0, 1, 2},
+ * delta_n not in 1..8, negative offsets or frames, a row outside src_elems, frames[c] or cap[c] above 2^31 - 1,
+ * the export's checks on dst, a dst range [dst, dst + dst_elems) that intersects [src, src + src_elems), or src not
+ * device memory of `device` give SGB_ERR_INVALID.  A working set over 226 KB of shared memory gives
+ * SGB_ERR_UNSUPPORTED: with ld = n_in | 1, S = 64 + 2 delta_order delta_n, it is
+ *   4 (n_ceps ld + S ld + S n_ceps + (delta_order == 2 ? (64 + 2 delta_n) n_ceps : 0)) <= 226 * 1024 bytes,
+ * which holds for every delta_order and delta_n up to n_in 256 and n_ceps 64 (205 KB at the largest). */
+typedef struct sgb_ceps_params {
+  int32_t n_in, n_ceps;          /* floats per input frame; cepstra per frame                       */
+  const float *matrix;           /* host, n_ceps * n_in, row-major                                  */
+  int32_t delta_order, delta_n;  /* 0, 1 or 2; 1..8                                                 */
+} sgb_ceps_params;
+int sgb_rows_cepstra(int32_t device, const float *src, int64_t src_elems, const int64_t *src_off,
+                     const int64_t *frames, int32_t n, const sgb_ceps_params *p, const sgb_device_out *o);
 /* default, low and high of a scalar argument of soundgen() as the front-end checks it (permittedValues,
  * R/presets.R:22-79); SGB_ERR_INVALID for a name the front-end does not range-check. */
 int sgb_param_range(const char *name, double out3[3]);
@@ -358,7 +387,7 @@ int sgb_batch_set_tracks(sgb_batch *b, int32_t env, const double *rows, int32_t 
 int sgb_batch_z_used(sgb_batch *b, int32_t *out);
 /* sizeof() of the ABI structs, for bindings to verify their mirrors:
  * syllable, envelope, noise, bout, call, formant_ref, batch_desc, run_info, soundgen_args, device_out, spec_params,
- * compare_params (cap >= 9; the 10th to 12th are written when cap allows). */
+ * compare_params, ceps_params (cap >= 9; the 10th to 13th are written when cap allows). */
 int sgb_abi_sizes(int32_t *out, int32_t cap);
 /* The additive synthesis has two kernels: epochs with at least `rows` rows run on the tensor cores, the others on the
    FP32 pipe (default 224, or SGB_SYNTH / SGB_SYNTH_MIN_ROWS from the environment).  0 = tensor cores only, a huge value =

@@ -122,6 +122,10 @@ class CompareParams(C.Structure):
     _fields_ = [('method', i32), ('n_feat', i32), ('pad', f64)]
 
 
+class CepsParams(C.Structure):
+    _fields_ = [('n_in', i32), ('n_ceps', i32), ('matrix', C.c_void_p), ('delta_order', i32), ('delta_n', i32)]
+
+
 T_NAMES = ['h2d', 'control', 'ampl', 'synth', 'compose', 'noise', 'assemble', 'envelope',
            'filter', 'finalize', 'd2h', 'total']
 
@@ -143,7 +147,7 @@ EXPORTS = ['sgb_version', 'sgb_last_error', 'sgb_device_count', 'sgb_set_device'
            'sgb_batch_create', 'sgb_batch_destroy', 'sgb_batch_upload', 'sgb_batch_run',
            'sgb_batch_lengths', 'sgb_batch_fetch_f32', 'sgb_batch_fetch_f64', 'sgb_batch_fetch_pcm16', 'sgb_batch_status',
            'sgb_batch_export', 'sgb_rows_export', 'sgb_spec_frames', 'sgb_batch_spectrogram', 'sgb_rows_spectrogram',
-           'sgb_rows_compare', 'sgb_param_range',
+           'sgb_rows_compare', 'sgb_rows_cepstra', 'sgb_param_range',
            'sgb_batch_syllable_len', 'sgb_batch_syllable_fetch', 'sgb_batch_noise_fetch',
            'sgb_batch_artefacts', 'sgb_batch_artefact_ints', 'sgb_batch_pitch_per_gc', 'sgb_batch_checksums', 'sgb_batch_debug_state',
            'sgb_get_rolloff', 'sgb_get_spectral_envelope', 'sgb_filter_len', 'sgb_filter',
@@ -199,6 +203,7 @@ def load():
     L.sgb_batch_spectrogram.argtypes = [vp, C.POINTER(SpecParams), C.POINTER(DeviceOut)]
     L.sgb_rows_spectrogram.argtypes = [i32, vp, vp, vp, i32, C.POINTER(SpecParams), C.POINTER(DeviceOut)]
     L.sgb_rows_compare.argtypes = [i32, vp, i64, vp, i64, vp, vp, vp, vp, i32, C.POINTER(CompareParams), vp, i64, vp]
+    L.sgb_rows_cepstra.argtypes = [i32, vp, i64, vp, vp, i32, C.POINTER(CepsParams), C.POINTER(DeviceOut)]
     L.sgb_param_range.argtypes = [C.c_char_p, vp]
     L.sgb_batch_syllable_len.argtypes = [vp, i32, C.POINTER(i64)]
     L.sgb_batch_syllable_fetch.argtypes = [vp, i32, vp, i64]
@@ -241,10 +246,10 @@ def load():
     L.sgb_frontend_h2d_bytes.restype = i64
     L.sgb_rng_draw.argtypes = [C.c_uint32, i32, f64, f64, i32, vp, i32]
     L.sgb_smooth_contour.argtypes = [vp, vp, i32, i32, f64, i32, f64, i32, f64, i32, i32, vp]
-    sizes = (i32 * 12)()
-    L.sgb_abi_sizes(sizes, 12)
+    sizes = (i32 * 13)()
+    L.sgb_abi_sizes(sizes, 13)
     mine = [C.sizeof(t) for t in (Syllable, Envelope, Noise, Bout, Call, FormantRef, BatchDesc, RunInfo, SoundgenArgs,
-                                  DeviceOut, SpecParams, CompareParams)]
+                                  DeviceOut, SpecParams, CompareParams, CepsParams)]
     if list(sizes) != mine:
         raise RuntimeError('ctypes mirror out of date: library struct sizes %s, mirror %s' % (list(sizes), mine))
     _lib = L

@@ -919,6 +919,15 @@ def spectrogram_device(wave, lengths, samplingRate, windowLength=50, overlap=75,
     lengths may be host or CUDA; a CUDA tensor is read back once, which synchronises with its stream.
     The result is ordered on `stream` (default: the device's current torch stream), with no other host wait."""
     import torch
+    spec, frames = _spectrogram_device(wave, lengths, samplingRate, windowLength, overlap, window, n_mels, fmin, fmax,
+                                       mel_scale, norm, db, db_floor, max_frames, stream)
+    return spec, torch.as_tensor(frames, dtype=torch.int64).to(wave.device)
+
+
+def _spectrogram_device(wave, lengths, samplingRate, windowLength, overlap, window, n_mels, fmin, fmax, mel_scale, norm,
+                        db, db_floor, max_frames, stream):
+    """spectrogram_device with the frames per row as a host array."""
+    import torch
     if not (torch.is_tensor(wave) and wave.is_cuda and wave.dtype == torch.float32 and wave.dim() == 2):
         raise ValueError('wave must be a 2-D float32 CUDA tensor')
     if window not in _WINDOWS:
@@ -960,9 +969,91 @@ def spectrogram_device(wave, lengths, samplingRate, windowLength=50, overlap=75,
             cap[idx] = F
             rows_spectrogram(wave.device.index, src, rows * T, lens, spec, rows * F * n_feat, cap, w, overlap, window,
                              bands, db, db_floor, stream)
-    frames = torch.as_tensor(np.minimum(nc, F), dtype=torch.int64).to(wave.device)
-    return spec, frames
+    return spec, np.minimum(nc, F)
 
+
+
+def dct_matrix(n_mfcc, n_mels, include_c0=True):
+    """The orthonormal DCT-II that turns log-mel frames into MFCCs, as a float64 [n_mfcc, n_mels] array:
+    D[k, b] = sqrt((2 - delta_k0) / n_mels) cos(pi k (2 b + 1) / (2 n_mels)) for k = 0 .. n_mfcc - 1, or for
+    k = 1 .. n_mfcc with include_c0=False.  These are rows of scipy.fft.dct(eye(n_mels), type=2, norm='ortho',
+    axis=0), and with c0 the matrix is torchaudio.functional.create_dct(n_mfcc, n_mels, 'ortho').T.  The rows
+    k >= 1 sum to zero, so a constant frame (silence at the dB floor) has 0 in every coefficient but c0."""
+    n_mfcc, n_mels, k0 = int(n_mfcc), int(n_mels), 0 if include_c0 else 1
+    if n_mfcc < 1 or n_mels < 1 or k0 + n_mfcc > n_mels:
+        raise ValueError('need 1 <= n_mfcc <= n_mels%s (%d, %d)' % ('' if include_c0 else ' - 1 without c0', n_mfcc,
+                                                                    n_mels))
+    k = np.arange(k0, k0 + n_mfcc, dtype=np.int64)[:, None]
+    b = np.arange(n_mels, dtype=np.int64)[None, :]
+    # the angle reduced exactly, in integers, to [0, 2 pi): k (2b + 1) mod 4 n_mels quarter-turns of pi / (2 n_mels)
+    D = math.sqrt(2.0 / n_mels) * np.cos(math.pi * ((k * (2 * b + 1)) % (4 * n_mels)) / (2 * n_mels))
+    if include_c0:
+        D[0] = math.sqrt(1.0 / n_mels)
+    return D
+
+
+def rows_cepstra(device, src, src_off, frames, dst, dst_off, cap, matrix, deltas=0, delta_n=2, stream=None):
+    """sgb_rows_cepstra (K11): cepstra c = matrix @ x of the frames the caller holds in the float32 CUDA tensor `src`
+    (row c = frames[c] frames of n_in = matrix.shape[1] floats from element src_off[c], as rows_spectrogram writes
+    them), followed by `deltas` (0, 1 or 2) orders of deltas over 2 delta_n + 1 frames with the row's edge frames
+    replicated (torchaudio's compute_deltas over the row's own frames).  Row c of dst gets cap[c] frames of
+    n_ceps (1 + deltas) floats, [c | delta | delta-delta], from element dst_off[c] on, zeros past the row's frames.
+    Returns the frames written per row."""
+    import torch
+    so = np.ascontiguousarray(src_off, dtype=np.int64)
+    fr = np.ascontiguousarray(frames, dtype=np.int64)
+    if not (torch.is_tensor(src) and src.is_contiguous() and src.dtype == torch.float32) or so.shape != fr.shape \
+            or so.ndim != 1:
+        raise ValueError('src must be a contiguous float32 tensor, src_off and frames of one length')
+    M = np.ascontiguousarray(matrix, dtype=np.float32)
+    if M.ndim != 2 or M.size == 0:
+        raise ValueError('matrix must be a non-empty [n_ceps, n_in] array, not %r' % (M.shape,))
+    p = _abi.CepsParams()
+    p.n_ceps, p.n_in, p.matrix = M.shape[0], M.shape[1], _ptr(M)
+    p.delta_order, p.delta_n = int(deltas), int(delta_n)
+    L = _abi.load()
+    return _export(lambda o: L.sgb_rows_cepstra(int(device), src.data_ptr() or None, src.numel(), _ptr(so), _ptr(fr),
+                                                fr.size, C.byref(p), C.byref(o)), fr.size, dst, dst_off, cap, stream,
+                   'f32')
+
+
+def mfcc_device(wave, lengths, samplingRate, n_mfcc=13, include_c0=True, deltas=0, delta_n=2, windowLength=50,
+                overlap=75, window='hamming', n_mels=40, fmin=0, fmax=None, mel_scale='htk', norm=None, db_floor=1e-10,
+                max_frames=None, stream=None):
+    """MFCCs and their deltas of the [n, T] float32 CUDA tensor `wave` that soundgen_batch_device returns: the
+    log-mel spectrogram of spectrogram_device(..., n_mels, db=True) (mixed sampling rates as there), projected on
+    dct_matrix(n_mfcc, n_mels, include_c0) with `deltas` (0, 1 or 2) orders of deltas over 2 delta_n + 1 frames, in
+    one call of K11 (rows_cepstra) over all rows.  Returns (feat, frames): feat [n, F, n_mfcc (1 + deltas)] float32,
+    frame k of row c = [c | delta | delta-delta] at feat[c, k], zeros past the row's frames, F = max_frames or the
+    most frames of any row; frames: int64 CUDA tensor of the frames present per row.  A row cut at max_frames is a
+    bit-exact prefix of the whole row: its last deltas read the log-mel frames past the cut.  Ordered on `stream`
+    (default: the device's current torch stream), with no host wait besides reading back a CUDA `lengths`."""
+    import torch
+    if int(deltas) not in (0, 1, 2) or not 1 <= int(delta_n) <= 8:
+        raise ValueError('need deltas in 0, 1, 2 and delta_n in 1..8, not %r, %r' % (deltas, delta_n))
+    if max_frames is not None and int(max_frames) < 0:
+        raise ValueError('max_frames must be non-negative')
+    if n_mels is None:
+        raise ValueError('n_mels must be given')
+    M = dct_matrix(n_mfcc, n_mels, include_c0).astype(np.float32)
+    H = int(deltas) * int(delta_n)           # frames past the cut that the deltas before it read
+    spec, nc = _spectrogram_device(wave, lengths, samplingRate, windowLength, overlap, window, int(n_mels), fmin, fmax,
+                                   mel_scale, norm, True, db_floor, None if max_frames is None else int(max_frames) + H,
+                                   stream)
+    n, Fs, nm = spec.shape
+    F = int(max_frames) if max_frames is not None else Fs
+    n_out = M.shape[0] * (1 + int(deltas))
+    feat = torch.empty((n, F, n_out), dtype=torch.float32, device=wave.device)
+    if n and F:
+        rows = np.arange(n, dtype=np.int64)
+        rows_cepstra(wave.device.index, spec, rows * Fs * nm, nc, feat, rows * F * n_out, np.full(n, F, dtype=np.int64),
+                     M, deltas, delta_n, stream)
+        h = _stream_handle(stream, spec)
+        if h != torch.cuda.current_stream(spec.device).cuda_stream:
+            # spec goes back to the allocator here, on the current stream: keep it until K11 has read it on `stream`
+            spec.record_stream(stream if isinstance(stream, torch.cuda.Stream)
+                               else torch.cuda.ExternalStream(h, device=spec.device))
+    return feat, torch.as_tensor(np.minimum(nc, F), dtype=torch.int64).to(wave.device)
 
 def _torch_out_dtype(dtype):
     import torch
@@ -1157,7 +1248,8 @@ _DB_FLOOR = 1e-10
 
 
 def match_pars(target, samplingRate, pars, base=None, n_candidates=64, max_iter=50, prob_mutation=0.25,
-               step_variance=0.1, method='cor', min_delta=0.0, windowLength=40, overlap=50, n_mels=64, seed=0):
+               step_variance=0.1, method='cor', min_delta=0.0, windowLength=40, overlap=50, n_mels=64, seed=0,
+               features='mel', n_mfcc=13, deltas=0):
     """Searches soundgen() arguments for a call that sounds like `target` (a 1-D float32 waveform, numpy or CUDA, at
     samplingRate): a hill-climb in the manner of the reference's matchPars that tries n_candidates mutations of the
     current best per step on the GPU.  base: the fixed arguments (temperature defaults to 0); pars: the scalar
@@ -1170,14 +1262,23 @@ def match_pars(target, samplingRate, pars, base=None, n_candidates=64, max_iter=
     Returns (best_kwargs, best_score, history): history[0] is the starting point, history[k] step k, each a dict with
     'score' (the step's best), 'accepted', 'values' ([candidates, len(pars)] array of the values tried) and 'best'
     (the current score after the step).  The same seed, inputs and n_candidates give the same history, bit for bit.
+    features='mfcc' scores MFCCs instead: mfcc_device with the same windowLength, overlap and n_mels, n_mfcc
+    coefficients without c0 and `deltas` orders of deltas, missing frames read as 0 (silence: the DCT rows without
+    c0 sum to zero, so a frame at the dB floor has 0 in every coefficient and delta).
     This is not R's matchPars: the draws come from numpy's generator, not R's stream, and the features are this
-    library's log-mel spectrograms, not tuneR::melfcc."""
+    library's log-mel spectrograms or MFCCs, not tuneR::melfcc."""
     import torch
     pars = _searched(pars)
     if method not in _CMP_METHODS:
         raise ValueError("method must be 'cor', 'cosine' or 'dtw', not %r" % (method,))
     if int(n_candidates) < 1 or int(max_iter) < 0:
         raise ValueError('need n_candidates >= 1 and max_iter >= 0')
+    if features not in ('mel', 'mfcc'):
+        raise ValueError("features must be 'mel' or 'mfcc', not %r" % (features,))
+    if features == 'mfcc':
+        dct_matrix(n_mfcc, n_mels, include_c0=False)
+        if int(deltas) not in (0, 1, 2):
+            raise ValueError('deltas must be 0, 1 or 2, not %r' % (deltas,))
     sr = float(samplingRate)
     kw = dict(temperature=0)
     kw.update(base or {})
@@ -1196,13 +1297,18 @@ def match_pars(target, samplingRate, pars, base=None, n_candidates=64, max_iter=
         x = torch.as_tensor(np.asarray(target, dtype=np.float32), device=dev)
     if x.dim() != 1:
         raise ValueError('target must be a 1-D waveform')
-    spec_kw = dict(windowLength=windowLength, overlap=overlap, n_mels=int(n_mels), db=True, db_floor=_DB_FLOOR)
-    tgt, tgt_frames = spectrogram_device(x.reshape(1, -1).contiguous(), [x.numel()], sr, **spec_kw)
-    pad = 10.0 * math.log10(_DB_FLOOR)
+    if features == 'mel':
+        spec_kw = dict(windowLength=windowLength, overlap=overlap, n_mels=int(n_mels), db=True, db_floor=_DB_FLOOR)
+        feats, pad = spectrogram_device, 10.0 * math.log10(_DB_FLOOR)
+    else:
+        spec_kw = dict(windowLength=windowLength, overlap=overlap, n_mels=int(n_mels), n_mfcc=int(n_mfcc),
+                       include_c0=False, deltas=int(deltas), db_floor=_DB_FLOOR)
+        feats, pad = mfcc_device, 0.0
+    tgt, tgt_frames = feats(x.reshape(1, -1).contiguous(), [x.numel()], sr, **spec_kw)
 
     def best_of(cands):
         wave, lengths, status = soundgen_batch_device([dict(kw, **c) for c in cands], device=dev.index)
-        spec, frames = spectrogram_device(wave, lengths, sr, **spec_kw)
+        spec, frames = feats(wave, lengths, sr, **spec_kw)
         s = compare_spectrograms(spec, frames, tgt, tgt_frames, method, pad=pad)
         bad = torch.as_tensor(np.asarray(status) != 0, device=dev) | torch.isnan(s)
         s = torch.where(bad, torch.full_like(s, -math.inf), s)

@@ -56,6 +56,9 @@ cudaError_t launch_spectrogram(const FftSeg *, int, const SpecRow *, const FftPl
 size_t spec_compare_smem_bytes(int method, int64_t max_short);
 cudaError_t launch_spec_compare(const float *, const float *, const void *, int, int, int, double, int64_t, double *,
                                 cudaStream_t);
+size_t cepstra_smem_bytes(int n_in, int n_ceps, int order, int dn);
+cudaError_t launch_cepstra(const CepsTile *, int, const CepsRow *, const float *, const float *, float *, int, int, int,
+                           int, cudaStream_t);
 void launch_noise_final(const sgb_noise *, int, const NoiseLayout *, const double *, const double *, const int *, int,
                         const float *, float *, void *, double *, const int64_t *, int, cudaStream_t);
 size_t contour_tab_bytes();
@@ -1375,9 +1378,9 @@ int sgb_abi_sizes(int32_t *out, int32_t cap) {
                        (int32_t)sizeof(sgb_bout), (int32_t)sizeof(sgb_call), (int32_t)sizeof(sgb_formant_ref),
                        (int32_t)sizeof(sgb_batch_desc), (int32_t)sizeof(sgb_run_info), (int32_t)sizeof(sgb_soundgen_args),
                        (int32_t)sizeof(sgb_device_out), (int32_t)sizeof(sgb_spec_params),
-                       (int32_t)sizeof(sgb_compare_params)};
+                       (int32_t)sizeof(sgb_compare_params), (int32_t)sizeof(sgb_ceps_params)};
   if (!out || cap < 9) return fail(SGB_ERR_INVALID, "need room for 9 sizes");
-  for (int i = 0; i < 12 && i < cap; i++) out[i] = v[i];
+  for (int i = 0; i < 13 && i < cap; i++) out[i] = v[i];
   return SGB_OK;
 }
 
@@ -1874,6 +1877,82 @@ int sgb_rows_compare(int32_t device, const float *a, int64_t a_elems, const floa
     return SGB_OK;
   };
   return export_queue(D->x, D->st, (cudaStream_t)stream, bytes, fill, launch);
+}
+
+// ---- cepstra of spectrogram rows (K11) ----
+int sgb_rows_cepstra(int32_t device, const float *src, int64_t src_elems, const int64_t *src_off, const int64_t *frames,
+                     int32_t n, const sgb_ceps_params *p, const sgb_device_out *o) {
+  // the parameters and the source rows alone (no device needed)
+  if (!p) return fail(SGB_ERR_INVALID, "null sgb_ceps_params");
+  if (p->n_in < 1 || p->n_ceps < 1) return fail(SGB_ERR_INVALID, "n_in %d, n_ceps %d: at least 1 each", p->n_in, p->n_ceps);
+  if (p->delta_order < 0 || p->delta_order > 2) return fail(SGB_ERR_INVALID, "delta_order %d not 0, 1 or 2", p->delta_order);
+  if (p->delta_n < 1 || p->delta_n > 8) return fail(SGB_ERR_INVALID, "delta_n %d outside 1..8", p->delta_n);
+  if (!p->matrix) return fail(SGB_ERR_INVALID, "null matrix");
+  const size_t smem = cepstra_smem_bytes(p->n_in, p->n_ceps, p->delta_order, p->delta_n);
+  if (smem > 226 * 1024)
+    return fail(SGB_ERR_UNSUPPORTED, "%d inputs, %d cepstra, delta order %d over %d frames: %zu bytes of shared memory",
+                p->n_in, p->n_ceps, p->delta_order, p->delta_n, smem);
+  const int64_t n_m = (int64_t)p->n_ceps * p->n_in;
+  for (int64_t i = 0; i < n_m; i++)
+    if (!std::isfinite(p->matrix[i])) return fail(SGB_ERR_INVALID, "matrix element %lld is not finite", (long long)i);
+  if (n < 0 || src_elems < 0) return fail(SGB_ERR_INVALID, "negative row count or src_elems");
+  if (n > 0 && (!src_off || !frames)) return fail(SGB_ERR_INVALID, "null row table");
+  for (int32_t c = 0; c < n; c++) {
+    const int64_t so = src_off[c], nc = frames[c];
+    if (so < 0 || nc < 0) return fail(SGB_ERR_INVALID, "row %d: negative source offset or frames", c);
+    if (nc > INT32_MAX) return fail(SGB_ERR_INVALID, "row %d: %lld frames (at most 2^31 - 1)", c, (long long)nc);
+    if (so > src_elems || nc > (src_elems - so) / p->n_in)
+      return fail(SGB_ERR_INVALID, "row %d: elements [%lld, %lld x %d more) outside src (%lld elements)", c,
+                  (long long)so, (long long)nc, p->n_in, (long long)src_elems);
+  }
+  int rc = rows_device_check(device, src, n);
+  if (rc != SGB_OK) return rc;
+  const int n_out = p->n_ceps * (1 + p->delta_order);
+  if ((rc = export_check(device, n > 0 ? src : nullptr, src_off, frames, n, o, n_out, false)) != SGB_OK) return rc;
+  std::vector<CepsRow> rows((size_t)n);
+  std::vector<CepsTile> tiles;
+  const int64_t zf = std::max(1, 8192 / n_out);       // zero tails: about 8192 floats per tile
+  for (int32_t c = 0; c < n; c++) {
+    if (o->cap[c] > INT32_MAX) return fail(SGB_ERR_INVALID, "row %d: %lld frames of capacity (at most 2^31 - 1)", c,
+                                           (long long)o->cap[c]);
+    const int32_t nc = (int32_t)frames[c], cap = (int32_t)o->cap[c], m = std::min(nc, cap);
+    rows[c] = CepsRow{src_off[c], o->dst_off[c], nc, cap};
+    for (int64_t t = 0; t < m; t += CEPS_TILE)
+      tiles.push_back(CepsTile{c, (int32_t)t, (int32_t)std::min<int64_t>(m, t + CEPS_TILE), 0});
+    for (int64_t t = m; t < cap; t += zf) tiles.push_back(CepsTile{c, (int32_t)t, (int32_t)std::min<int64_t>(cap, t + zf), 1});
+  }
+  if (tiles.size() > (size_t)INT32_MAX) return fail(SGB_ERR_UNSUPPORTED, "too many tiles");
+  if (!tiles.empty() && src_elems > 0) {             // the kernel reads src while it writes dst
+    const char *s0 = reinterpret_cast<const char *>(src), *s1 = s0 + 4 * src_elems;
+    const char *d0 = reinterpret_cast<const char *>(o->dst), *d1 = d0 + 4 * o->dst_elems;
+    if (d0 < s1 && s0 < d1) return fail(SGB_ERR_INVALID, "dst overlaps src");
+  }
+  DeviceExport *D;
+  if ((rc = device_export(device, &D)) != SGB_OK) return rc;
+  std::lock_guard<std::mutex> g(D->mu);
+  auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
+  const size_t o_tiles = up16(sizeof(CepsRow) * rows.size()), o_m = up16(o_tiles + sizeof(CepsTile) * tiles.size());
+  const size_t bytes = o_m + sizeof(float) * (size_t)n_m;
+  auto fill = [&](char *h) {
+    if (n) memcpy(h, rows.data(), sizeof(CepsRow) * rows.size());
+    if (!tiles.empty()) memcpy(h + o_tiles, tiles.data(), sizeof(CepsTile) * tiles.size());
+    memcpy(h + o_m, p->matrix, sizeof(float) * (size_t)n_m);
+  };
+  auto launch = [&](const char *d) -> int {
+    cudaError_t e = launch_cepstra(reinterpret_cast<const CepsTile *>(d + o_tiles), (int)tiles.size(),
+                                   reinterpret_cast<const CepsRow *>(d), reinterpret_cast<const float *>(d + o_m), src,
+                                   (float *)o->dst, p->n_in, p->n_ceps, p->delta_order, p->delta_n, D->st);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return fail(SGB_ERR_CUDA, "k_cepstra launch failed (%zu tiles, %zu bytes of shared memory): %s", tiles.size(),
+                  smem, cudaGetErrorString(e));
+    }
+    return SGB_OK;
+  };
+  if ((rc = export_queue(D->x, D->st, (cudaStream_t)o->stream, bytes, fill, launch)) != SGB_OK) return rc;
+  if (o->out_written)
+    for (int32_t c = 0; c < n; c++) o->out_written[c] = std::min(frames[c], o->cap[c]);
+  return SGB_OK;
 }
 
 // Diagnostic for a stuck run (callable from another thread): out[0] = which wait the handle's host thread

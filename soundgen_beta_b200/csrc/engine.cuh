@@ -154,6 +154,14 @@ struct SpecRow {             // one row of a spectrogram (K9); nc and cap count 
   int64_t cap;               // frames written (the first min(nc, cap) computed, the rest zeros)
 };
 
+struct CepsRow {             // one row of cepstra (K11); nc counts input frames, cap output frames
+  int64_t src_off;           // floats into the source
+  int64_t dst_off;           // floats into the destination
+  int32_t nc, cap;
+};
+struct CepsTile { int32_t row, t0, t1, zero; };   // output frames [t0, t1) of a row; zero: the tail past nc
+constexpr int CEPS_TILE = 64;                     // most frames of a compute tile (the choice: kernels_ceps.cu)
+
 
 // Ordered-int encoding so that atomicMax on int implements a signed float max.
 __device__ __forceinline__ int float_to_ordered(float f) {
