@@ -537,6 +537,8 @@ class HarmonicsArtefacts:
     mats: list = None                  # per-epoch (matrix, rownames)
     integr: np.ndarray = None          # cumsum(pitch_upsampled) / samplingRate
     epoch_waves: list = field(default_factory=list)
+    ampl_gain: np.ndarray = None       # 2^(amplEnvelope / 10) per sample of the joined waveform, or None
+    drift_upsampled: np.ndarray = None # drift gain per sample of the output (temperature > 0), or None
 
 
 def generateHarmonics(pitch, attackLen=50, nonlinBalance=0, nonlinDep=0, jitterDep=0,
@@ -670,13 +672,15 @@ def generateHarmonics(pitch, attackLen=50, nonlinBalance=0, nonlinDep=0, jitterD
     if use_ampl:  # :436-448
         amplEnvelope = getSmoothContour(amplAnchors, length=waveform.size, valueFloor=0,
                                         samplingRate=samplingRate, method=contour_method)
-        waveform = waveform * 2 ** (amplEnvelope / 10)
+        art.ampl_gain = 2 ** (amplEnvelope / 10)
+        waveform = waveform * art.ampl_gain
     art.raw_max = float(np.max(waveform))
     waveform = waveform / np.max(waveform)  # :449 signed max
     if attackLen > 0:  # :452-456
         waveform = fadeInOut(waveform, length_fade=math.floor(attackLen * samplingRate / 1000))
     if temperature > 0:  # :459-467
         drift_upsampled = r_approx(drift, waveform.size, x=gc_upsampled[:-1].astype(np.float64))
+        art.drift_upsampled = drift_upsampled
         waveform = waveform * drift_upsampled
     art.z_used = getattr(rng, "zi", None)
     return (waveform, art) if want_artefacts else waveform

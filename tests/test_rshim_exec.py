@@ -3,24 +3,32 @@ runtime (tests/rstub/fake_r.c: heap SEXPs, attributes, PROTECT counter, Rf_error
 the real libsoundgen_b200.so.  CPU part: the error paths (Rf_error before and after native resources exist,
 PROTECT balance, "no device" -- there is no CPU fallback).  GPU part: all six entry points, outputs compared
 with the ctypes path on the same inputs, R's .Random.seed handed in and back."""
+import atexit
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 STUB = os.path.join(ROOT, 'tests', 'rstub')
-EXE = os.path.join(STUB, 'run_shim')
+_exe = []
 
 
 def build():
-    lib = os.path.join(ROOT, 'soundgen_beta_b200')
-    srcs = [os.path.join(STUB, 'fake_r.c'), os.path.join(STUB, 'run_shim.c'), os.path.join(ROOT, 'r', 'src', 'rshim.c')]
-    if os.path.exists(EXE) and all(os.path.getmtime(EXE) > os.path.getmtime(s) for s in srcs):
-        return
-    subprocess.check_call(['gcc', '-O1', '-Wall', '-Werror', '-I', STUB, '-I', os.path.join(ROOT, 'include'), '-o', EXE] + srcs +
-                          ['-L', lib, '-lsoundgen_b200', '-Wl,-rpath,' + lib, '-lm'])
+    """Compile the shim driver once per process into a temporary directory (the checkout may be read-only)."""
+    if not _exe:
+        d = tempfile.mkdtemp(prefix='sgb_rshim_')
+        atexit.register(shutil.rmtree, d, True)
+        exe = os.path.join(d, 'run_shim')
+        lib = os.path.join(ROOT, 'soundgen_beta_b200')
+        srcs = [os.path.join(STUB, 'fake_r.c'), os.path.join(STUB, 'run_shim.c'), os.path.join(ROOT, 'r', 'src', 'rshim.c')]
+        subprocess.check_call(['gcc', '-O1', '-Wall', '-Werror', '-I', STUB, '-I', os.path.join(ROOT, 'include'), '-o', exe] +
+                              srcs + ['-L', lib, '-lsoundgen_b200', '-Wl,-rpath,' + lib, '-lm'])
+        _exe.append(exe)
+    return _exe[0]
 
 
 def inputs():
@@ -52,10 +60,10 @@ def read(path):
 
 
 def run(mode, tmp_path, env=None):
-    build()
+    exe = build()
     inp, outp = str(tmp_path / 'in.txt'), str(tmp_path / 'out.txt')
     write(inp, inputs())
-    r = subprocess.run([EXE, mode, inp, outp], capture_output=True, text=True, timeout=600, env=env)
+    r = subprocess.run([exe, mode, inp, outp], capture_output=True, text=True, timeout=600, env=env)
     return r, read(outp)
 
 
