@@ -365,6 +365,13 @@ int sgb_batch_artefacts(sgb_batch *b, int32_t syl, sgb_syl_artefacts *out);
  *        (2*nEpochs: zc1, zc2; 0 = NA) */
 int sgb_batch_artefact_ints(sgb_batch *b, int32_t syl, int which, int32_t *out, int32_t cap);
 int sgb_batch_pitch_per_gc(sgb_batch *b, int32_t syl, double *out, int32_t cap);
+/* Diagnostic: the amplitude tables of epoch `epoch` of syllable `syl` of the last run.  shape[3] receives
+ * {rows, columns, pairs}.  f64 (cap >= rows * columns doubles) receives the FP64 matrix, column by column;
+ * f32 (4 * cap floats) the epoch's FP32 table region, 16 bytes per element: with pairs, {Y_g, Y_{g+1} - Y_g}
+ * float pairs for columns 0..columns-2 at its start and zeros after; otherwise {Y, Y, dY, dY} per element.
+ * Null f64 and f32 report the shape only. */
+int sgb_batch_amp_tables(sgb_batch *b, int32_t syl, int32_t epoch, double *f64, float *f32, int64_t cap,
+                         int32_t *shape);
 /* Diagnostic: nine position-weighted checksums of the last run's intermediates (see engine.cu);
  * identical inputs must give identical checksums on every run. */
 int sgb_batch_checksums(sgb_batch *b, uint64_t *out, int32_t cap);

@@ -242,6 +242,7 @@ struct sgb_batch {
   std::vector<int32_t> call_status;
   int64_t total_out = 0;
   int64_t last_amp = 0, last_wave = 0, last_raw = 0, last_tiles = 0, last_sound = 0;
+  int last_tc_min_rows = 0;          // K1 dispatch threshold of the last run (the FP32 table's layout per epoch)
   volatile int where = 0;   // progress marker for sgb_batch_debug_state: which wait the host thread is in
   volatile int reached[16] = {0};   // SGB_TRACE=1: stage events the stream has passed (set by host callbacks)
   struct Mark { volatile int *dst; } marks[16];
@@ -870,6 +871,7 @@ int sgb_batch_run_begin(sgb_batch *b) {
   }();
   const int tc_min_rows = g_synth_min_rows_override >= 0 ? g_synth_min_rows_override : tc_min_rows_env;
   synth_min_rows_set(tc_min_rows);
+  b->last_tc_min_rows = tc_min_rows;
   launch_control(d_syl, S, b->ctrl_dense, b->d_order.as<int32_t>(), b->d_pitch.as<double>(), b->d_anchors.as<double>(), b->d_z.as<double>(), P, d_ctrl, d_lay,
                  d_tot, st);
   CKL("launch_control");
@@ -2085,6 +2087,29 @@ int sgb_batch_artefact_ints(sgb_batch *b, int32_t syl, int which, int32_t *out, 
   if (cap < n) return fail(SGB_ERR_INVALID, "buffer too small");
   if (n > 0) CK(cudaMemcpy(out, src, 4 * (size_t)n, cudaMemcpyDeviceToHost));
   return n;
+}
+
+// Diagnostic: K3's tables of one epoch of the last run.  shape = {rows, columns, pairs}; f64 gets the rows x columns
+// FP64 matrix (column-major), f32 the epoch's 16-byte-per-element FP32 region as K3 left it (pairs: {Y, dY} packed
+// at its start, zeros after; otherwise {Y, Y, dY, dY}).  Null f64 and f32 only report the shape.
+int sgb_batch_amp_tables(sgb_batch *b, int32_t syl, int32_t epoch, double *f64, float *f32, int64_t cap,
+                         int32_t *shape) {
+  if (!shape) return fail(SGB_ERR_INVALID, "null argument");
+  SylCtrl C;
+  int rc = get_ctrl(b, syl, &C);
+  if (rc) return rc;
+  if (C.status != SGB_OK || C.nGC == 0) return fail(SGB_ERR_STATE, "syllable %d has no amplitude matrices", syl);
+  if (epoch < 0 || epoch >= C.nEpochs) return fail(SGB_ERR_INVALID, "epoch index");
+  const int64_t rows = C.ep_rows[epoch], cols = C.ep_end[epoch] - C.ep_start[epoch] + 1, n = rows * cols;
+  shape[0] = (int32_t)rows; shape[1] = (int32_t)cols; shape[2] = rows >= b->last_tc_min_rows;
+  if (!f64 && !f32) return SGB_OK;
+  if (!f64 || !f32 || cap < n) return fail(SGB_ERR_INVALID, "buffer too small");
+  SylLayout lay;
+  CK(cudaMemcpy(&lay, b->d_lay.as<SylLayout>() + syl, sizeof(SylLayout), cudaMemcpyDeviceToHost));
+  const int64_t off = lay.amp_off + C.ep_amp_off[epoch];
+  CK(cudaMemcpy(f64, b->d_amp.as<double>() + off, 8 * (size_t)n, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(f32, b->d_amp32.as<float4>() + off, 16 * (size_t)n, cudaMemcpyDeviceToHost));
+  return SGB_OK;
 }
 
 int sgb_batch_pitch_per_gc(sgb_batch *b, int32_t syl, double *out, int32_t cap) {

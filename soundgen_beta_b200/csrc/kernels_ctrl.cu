@@ -230,20 +230,26 @@ __global__ void k_build_tiles(const SylCtrl *ctrl, int S, const SylLayout *lay, 
 
 // K3: dense per-epoch amplitude matrices A[e][g][j] (column per glottal cycle, rows =
 // multiples of f0/(nSubharm+1)), exact doubles: getRolloff + shimmer + getVocalFry
-// (R/sourceSpectrum.R:71-186, R/source.R:348-375, R/subharmonics.R:25-163).
-// grid (S, chunks of glottal cycles).  Per epoch the CTA tabulates what the reference's
-// quirk makes column-independent -- the f-harmonic amplitudes of the epoch's FIRST cycle
-// (subharmonics.R:76-77) -- and the per-(s, cycle) sideband multipliers, so that an f row
-// costs one exp2 and a g row two FMAs.
-#define AMP_MAXH 1024
-#define AMP_MAXS 16
-#define AMP_CG 32
+// (R/sourceSpectrum.R:71-186, R/source.R:348-375, R/subharmonics.R:25-163), and the FP32 table
+// {Y_g, Y_{g+1} - Y_g} K1 reads.  grid (S, column ranges of the syllable).
+// K3 reads almost nothing and writes 16-24 B per element, so it is organised to spend few instructions per element.
+// Epochs whose rows fit the shared tables (Hk <= AMP_MAXH, n <= AMP_MAXS) are done in chunks of up to AMP_CC columns,
+// two barriers per chunk:
+//   phase 1  the Hk x chunk f-harmonic amplitudes (rolloff + exp2, the only costly values) over all threads, into a
+//            shared ring of chunk + 1 columns, and the chunk's sideband multipliers ML, MU;
+//   phase 2  every thread writes the rows it owns over the chunk's columns.  A sideband row (k, s) is
+//            A0[k] ML + A0[k+1] MU, where A0 are the f-harmonics of the epoch's FIRST cycle (the reference's quirk,
+//            subharmonics.R:76-77): (k, s), A0[k] and A0[k+1] are fetched once per row and chunk.  The ring's extra
+//            column is the previous chunk's last one, for the dY differences.
+// Every value keeps its expression; the unit is compiled with -fmad=false, so the order of work changes no bits.
+#define AMP_MAXH 1024    // kept rows of the shared tables
+#define AMP_MAXS 16      // sub-harmonics of the sideband multipliers
+#define AMP_CC 8         // most columns per chunk
+#define AMP_VF 3072      // doubles of the f-harmonic ring, (columns per chunk + 1) x Hk
 #ifndef AMP_MIN_CTAS
-#define AMP_MIN_CTAS 4      // resident CTAs per SM (64 registers): measured 2 / 3 / 4 / 5 / 6 -> cfg3 6.0 / 5.8 / 5.9 / 6.7 / 7.0 ms, preset sweep 17.7 / 15.3 / 14.3 / 14.7 / 16.9 ms
+#define AMP_MIN_CTAS 4   // resident CTAs per SM: 64 registers and 47 KB of shared memory each.  Measured on cfg3:
+                         // 3.28 ms; 3 CTAs (more registers) 3.60 ms; the column loop of phase 2 unrolled 4x: no change
 #endif
-#define AMP_RPT 4
-#define AMP_VF 1024      // f-harmonics per column the dense variant keeps in shared memory
-#define AMP_DR 10        // rows per thread of the dense variant (rows <= 2560)
 __global__ void __launch_bounds__(256, AMP_MIN_CTAS)
 k_amp(const sgb_syllable *syl, int S, const SylCtrl *ctrl, const SylLayout *lay, Pools P, double *amp,
       float4 *amp32, int tc_min_rows) {
@@ -251,158 +257,169 @@ k_amp(const sgb_syllable *syl, int S, const SylCtrl *ctrl, const SylLayout *lay,
   if (s >= S) return;
   const SylCtrl &C = ctrl[s];
   if (C.status != SGB_OK || C.nGC == 0) return;
+  const int G = C.nGC, Hk = C.rows_kept;
+  // this CTA's columns [c0, c1)
+  const int c0 = (int)((int64_t)G * blockIdx.y / gridDim.y), c1 = (int)((int64_t)G * (blockIdx.y + 1) / gridDim.y);
+  if (c0 >= c1) return;
   const sgb_syllable sp = syl[s];
-  SylArrays A = make_arrays(P, sp, s);
+  // the per-cycle arrays are addressed from the pool bases (kernel parameters): SylArrays would hold 8 pointers in
+  // registers through the whole kernel
+  const int64_t o = P.gc_off[s];
+  const int32_t *rowmap = P.rowmap + P.h_off[s];
   double *out = amp + lay[s].amp_off;
   float4 *out32 = amp32 + lay[s].amp_off;
-  __shared__ double A0[AMP_MAXH + 2];
-  __shared__ double ML[AMP_MAXS * (AMP_CG + 1)], MU[AMP_MAXS * (AMP_CG + 1)];
-  __shared__ double VF[2][AMP_VF + 2];
-  const int G = C.nGC, Hk = C.rows_kept;
+  __shared__ double A0[AMP_MAXH + 2];                        // f-harmonics of the epoch's first cycle, ends 0
+  __shared__ double LG[AMP_MAXH];                            // log2(h) of kept row k
+  __shared__ int HK[AMP_MAXH];                               // harmonic number h of kept row k
+  __shared__ double VF[AMP_VF];                              // ring of f-harmonic columns
+  __shared__ double ML[(AMP_CC + 1) * AMP_MAXS], MU[(AMP_CC + 1) * AMP_MAXS];
+  __shared__ double CP[2][AMP_CC][5];                        // column terms of this chunk and the next
+  const int tid = threadIdx.x;
+  const bool ao = C.any_oct != 0;
   const double thr01 = exp2(sp.throwaway / 10.0);
-  for (int c0 = blockIdx.y * AMP_CG; c0 < G; c0 += gridDim.y * AMP_CG) {
-    const int c1 = min(G, c0 + AMP_CG);
-    for (int e = 0; e < C.nEpochs; e++) {
-      const int ga = max(c0, C.ep_start[e] - 1), gb = min(c1, C.ep_end[e]);   // [ga, gb) 0-based
-      if (ga >= gb) continue;
-      const int gx = min(gb + 1, C.ep_end[e]);     // one extra column for the differences
-      const int n = C.vf_active ? C.ep_nsub[e] : 0;
-      const int rows = C.ep_rows[e];
-      const int g0 = C.ep_start[e] - 1;
-      double *oe = out + C.ep_amp_off[e];
-      float4 *oe32 = out32 + C.ep_amp_off[e];
-      // the tensor-core kernel reads {Y, dY} pairs (8 B per element, packed at the start of the epoch's region); the
-      // FP32-pipe kernel wants {Y, Y, dY, dY} (one broadcast LDS.128 feeds both packed lanes)
-      const bool tc_ep = rows >= tc_min_rows;
-      const bool tabled = (n == 0) || (Hk <= AMP_MAXH && n <= AMP_MAXS);
-      __syncthreads();
-      if (tabled && n > 0) {
-        for (int k = threadIdx.x; k <= Hk + 1; k += blockDim.x) {   // A0[k], k = 0..Hk+1 (ends are 0)
+  const bool fits = Hk <= AMP_MAXH;
+  if (fits)
+    for (int k = tid; k < Hk; k += 256) { const int h = rowmap[k]; HK[k] = h; LG[k] = log2((double)h); }
+  const int cc = fits ? min(AMP_CC, AMP_VF / Hk - 1) : 0;    // columns per chunk (>= 2)
+  const int ring = cc + 1;
+  auto col_terms = [&](double *t, int g) {
+    const double pg = P.ppg[o + g];
+    t[0] = pg;
+    t[1] = P.ro[o + g] + P.rk[o + g] * (pg - 200.0) / 1000.0;       // column term of rolloff_db_l
+    t[2] = P.roct[o + g];
+    t[3] = P.colmax[o + g];
+    t[4] = P.shimmer[o + g];
+  };
+  for (int e = 0; e < C.nEpochs; e++) {
+    const int ga = max(c0, C.ep_start[e] - 1), gb = min(c1, C.ep_end[e]);   // [ga, gb) 0-based
+    if (ga >= gb) continue;
+    const int gx = min(gb + 1, C.ep_end[e]);     // one extra column for the differences
+    const int n = C.vf_active ? C.ep_nsub[e] : 0;
+    const int rows = C.ep_rows[e];
+    const int g0 = C.ep_start[e] - 1;
+    double *oe = out + C.ep_amp_off[e];
+    float4 *oe32 = out32 + C.ep_amp_off[e];
+    // the tensor-core kernel reads {Y, dY} pairs (8 B per element, packed at the start of the epoch's region); the
+    // FP32-pipe kernel wants {Y, Y, dY, dY} (one broadcast LDS.128 feeds both packed lanes)
+    float2 *oe2 = reinterpret_cast<float2 *>(oe32);
+    const bool tc_ep = rows >= tc_min_rows;
+    if (fits && n <= AMP_MAXS) {
+      if (n > 0) {
+        for (int k = tid; k <= Hk + 1; k += 256) {   // A0[k], k = 0..Hk+1 (ends are 0)
           double v = 0.0;
           if (k >= 1 && k <= Hk) {
-            int h = A.rowmap[k - 1];
-            double r = rolloff_db(h, A.ppg[g0], A.ro[g0], A.roct[g0], A.rk[g0], C.any_oct != 0, sp.rolloffParab,
+            int h = rowmap[k - 1];
+            double r = rolloff_db(h, P.ppg[o + g0], P.ro[o + g0], P.roct[o + g0], P.rk[o + g0], ao, sp.rolloffParab,
                                   C.parab_harm, C.parab_a, C.parab_b, C.parab_c, 200.0, sp.throwaway, sp.samplingRate);
-            v = exp2((r - A.colmax[g0]) / 10.0) * A.shimmer[g0];
+            v = exp2((r - P.colmax[o + g0]) / 10.0) * P.shimmer[o + g0];
           }
           A0[k] = v;
         }
-        const int ncol = gx - ga;
-        for (int idx = threadIdx.x; idx < n * ncol; idx += blockDim.x) {
-          int si = idx / ncol, gi = idx - si * ncol;
-          int g = ga + gi, sidx = si + 1;
-          double sw = A.subdep[g];
-          double dl = A.ppg[g] * (double)sidx / (double)(n + 1);
-          double du = A.ppg[g] * (double)(n + 1 - sidx) / (double)(n + 1);
-          double ml = 0.0, mu = 0.0;
-          if (sw != 0.0) { ml = exp(-0.5 * (dl / sw) * (dl / sw)); mu = exp(-0.5 * (du / sw) * (du / sw)); }
-          ML[si * (AMP_CG + 1) + gi] = ml; MU[si * (AMP_CG + 1) + gi] = mu;
-        }
       }
+      if (tid < min(cc, gx - ga)) col_terms(CP[0][tid], ga + tid);
       __syncthreads();
-      if (tabled && n > 0 && rows >= 512 && Hk <= AMP_VF && rows <= 256 * AMP_DR) {
-        // Dense variant (epochs with sub-harmonics).  Only every (n+1)-th row is an f-harmonic (rolloff + exp2, the
-        // expensive rows); evaluated row by row they would keep 1/(n+1) of a warp's lanes busy.  So per
-        // column the f-harmonics are first computed densely over the threads into shared memory
-        // (double-buffered: one barrier per column), then every thread writes the rows it owns.
-        double prev[AMP_DR], lgk[AMP_VF / 256];
-        int hk[AMP_VF / 256];
-#pragma unroll
-        for (int i = 0; i < AMP_VF / 256; i++) {
-          const int k = (int)threadIdx.x + 1 + 256 * i;
-          hk[i] = 1; lgk[i] = 0.0;
-          if (k <= Hk) { hk[i] = A.rowmap[k - 1]; lgk[i] = log2((double)hk[i]); }
+      const int d = n + 1;
+      const unsigned magic = n > 0 ? 0xFFFFFFFFu / (unsigned)d + 1u : 0u;   // j / d = umulhi(j, magic) for j < 2^28
+      int pos0 = 0;                                // ring slot of the chunk's first column; one less every chunk
+      int buf = 0;
+      for (int cs = ga; cs < gx; cs += cc) {
+        const int ncc = min(cc, gx - cs);
+        // phase 1: f-harmonics (cut at thr01 when there are sub-harmonics), sideband multipliers, next column terms
+        // items (column c, row k) strided by 256 over the threads, stepped without a division (Hk > 128 in most epochs)
+        int c = 0, k = tid;
+        while (k >= Hk && c < ncc) { k -= Hk; c++; }
+        while (c < ncc) {
+          const double *t = CP[buf][c];
+          const double r = rolloff_db_s(HK[k], LG[k], t[0], t[1], t[2], ao, sp.rolloffParab, C.parab_harm, C.parab_a,
+                                        C.parab_b, C.parab_c, 200.0, sp.throwaway, sp.samplingRate);
+          double v = exp2((r - t[3]) / 10.0) * t[4];
+          if (n > 0 && v < thr01) v = 0.0;
+          int p = pos0 + c;
+          if (p >= ring) p -= ring;
+          VF[p * Hk + k] = v;
+          k += 256;
+          while (k >= Hk && c < ncc) { k -= Hk; c++; }
         }
-#pragma unroll
-        for (int i = 0; i < AMP_DR; i++) prev[i] = 0.0;
-        for (int g = ga; g < gx; g++) {
-          const int gi = g - ga;
-          const double pg = A.ppg[g], roctg = A.roct[g], cmg = A.colmax[g], shg = A.shimmer[g];
-          const double slope = A.ro[g] + A.rk[g] * (pg - 200.0) / 1000.0;   // column term of rolloff_db_l
-          double *vf = VF[gi & 1];
-#pragma unroll
-          for (int i = 0; i < AMP_VF / 256; i++) {
-            const int k = (int)threadIdx.x + 1 + 256 * i;
-            if (k > Hk) continue;
-            double r = rolloff_db_s(hk[i], lgk[i], pg, slope, roctg, C.any_oct != 0, sp.rolloffParab, C.parab_harm,
-                                    C.parab_a, C.parab_b, C.parab_c, 200.0, sp.throwaway, sp.samplingRate);
-            vf[k] = exp2((r - cmg) / 10.0) * shg;
+        {
+          const int idx = 255 - tid, c = idx / AMP_MAXS, si = idx % AMP_MAXS;   // the last threads: fewest f items
+          if (c < ncc && si < n) {
+            const int g = cs + c, sidx = si + 1;
+            double sw = P.subdep[o + g];
+            double dl = P.ppg[o + g] * (double)sidx / (double)(n + 1);
+            double du = P.ppg[o + g] * (double)(n + 1 - sidx) / (double)(n + 1);
+            double ml = 0.0, mu = 0.0;
+            if (sw != 0.0) { ml = exp(-0.5 * (dl / sw) * (dl / sw)); mu = exp(-0.5 * (du / sw) * (du / sw)); }
+            int p = pos0 + c;
+            if (p >= ring) p -= ring;
+            ML[p * AMP_MAXS + si] = ml; MU[p * AMP_MAXS + si] = mu;
           }
-          __syncthreads();
-          double *oc = oe + (int64_t)(g - g0) * rows;
-          float4 *oc32 = oe32 + (int64_t)(g - 1 - g0) * rows;
-#pragma unroll
-          for (int i = 0; i < AMP_DR; i++) {
-            const int j = i * 256 + (int)threadIdx.x + 1;
-            if (j > rows) continue;
-            double v;
-            if (n == 0) {
-              v = vf[j];
-            } else {
-              const int k = j / (n + 1), si = j - k * (n + 1);
-              if (si == 0) v = vf[k];
-              else v = A0[k] * ML[(si - 1) * (AMP_CG + 1) + gi] + A0[k + 1] * MU[(si - 1) * (AMP_CG + 1) + gi];
-              if (v < thr01) v = 0.0;
-            }
-            if (g < gb) oc[j - 1] = v;
+          const int cn = cs + cc;
+          if (tid < min(cc, gx - cn)) col_terms(CP[buf ^ 1][tid], cn + tid);
+        }
+        __syncthreads();
+        // phase 2: the rows x ncc block
+        for (int j = tid + 1; j <= rows; j += 256) {
+          const int k = n > 0 ? (int)__umulhi((unsigned)j, magic) : j;
+          const int si = j - k * d;
+          const double a0 = si ? A0[k] : 0.0, a1 = si ? A0[k + 1] : 0.0;
+          const double *vf = VF + (k - 1);
+          const double *ml = ML + (si - 1), *mu = MU + (si - 1);
+          auto val = [&](int p) -> double {
+            if (si == 0) return vf[p * Hk];
+            double v = a0 * ml[p * AMP_MAXS] + a1 * mu[p * AMP_MAXS];
+            if (v < thr01) v = 0.0;
+            return v;
+          };
+          double prev = 0.0;
+          if (cs > ga) prev = val(pos0 == 0 ? ring - 1 : pos0 - 1);
+          int64_t i = (int64_t)(cs - g0) * rows + (j - 1);
+          int p = pos0;
+          for (int c = 0; c < ncc; c++, i += rows) {
+            const int g = cs + c;
+            const double v = val(p);
+            if (++p == ring) p = 0;
+            if (g < gb) oe[i] = v;
             if (g > ga) {   // {Y, Y, dY, dY}: one 16-byte load gives K1 both packed FFMA2 operands
-              const float y = (float)prev[i], dy = (float)(v - prev[i]);
-              if (tc_ep) reinterpret_cast<float2 *>(oe32)[(int64_t)(g - 1 - g0) * rows + (j - 1)] = make_float2(y, dy);
-              else oc32[j - 1] = make_float4(y, y, dy, dy);
+              const float y = (float)prev, dy = (float)(v - prev);
+              if (tc_ep) oe2[i - rows] = make_float2(y, dy);
+              else oe32[i - rows] = make_float4(y, y, dy, dy);
             }
-            prev[i] = v;
+            prev = v;
           }
         }
-        continue;
+        __syncthreads();
+        pos0 = pos0 == 0 ? ring - 1 : pos0 - 1;
+        buf ^= 1;
       }
-      // General variant: each thread owns rows j = rb + tid + i*256 and walks the columns, so that the
-      // FP32 {Y_g, Y_{g+1} - Y_g} table K1 consumes falls out of the same pass
-      for (int rb = 0; rb < rows; rb += 256 * AMP_RPT) {
-        double prev[AMP_RPT], lg[AMP_RPT];
-        int rk_[AMP_RPT], rs_[AMP_RPT], rh_[AMP_RPT];     // per owned row: f index k, sub index s, harmonic h
-#pragma unroll
-        for (int i = 0; i < AMP_RPT; i++) {
-          const int j = rb + i * 256 + (int)threadIdx.x + 1;
-          rk_[i] = 0; rs_[i] = 0; rh_[i] = 1; lg[i] = 0.0; prev[i] = 0.0;
-          if (j <= rows) {
-            rk_[i] = (n == 0) ? j : j / (n + 1);
-            rs_[i] = (n == 0) ? 0 : j % (n + 1);
-            if (rs_[i] == 0) { rh_[i] = A.rowmap[rk_[i] - 1]; lg[i] = log2((double)rh_[i]); }
-          }
+      continue;
+    }
+    // Per-element path (Hk > AMP_MAXH, or n > AMP_MAXS: ampl_exact): each thread owns rows j = tid + 1 + 256 i and
+    // walks the columns
+    const bool exact = n > 0;
+    const SylArrays A = make_arrays(P, sp, s);
+    for (int j = tid + 1; j <= rows; j += 256) {
+      const int h = exact ? 1 : rowmap[j - 1];
+      const double lg = exact ? 0.0 : log2((double)h);
+      double prev = 0.0;
+      for (int g = ga; g < gx; g++) {
+        double v;
+        if (exact) {
+          v = ampl_exact(sp, A, C, e, j, g);
+        } else {
+          const double pg = P.ppg[o + g];
+          const double slope = P.ro[o + g] + P.rk[o + g] * (pg - 200.0) / 1000.0;   // column term of rolloff_db_l
+          double r = rolloff_db_s(h, lg, pg, slope, P.roct[o + g], ao, sp.rolloffParab, C.parab_harm, C.parab_a,
+                                  C.parab_b, C.parab_c, 200.0, sp.throwaway, sp.samplingRate);
+          v = exp2((r - P.colmax[o + g]) / 10.0) * P.shimmer[o + g];
         }
-        for (int g = ga; g < gx; g++) {
-          const int gi = g - ga;
-          const double pg = A.ppg[g], roctg = A.roct[g], cmg = A.colmax[g], shg = A.shimmer[g];
-          const double slope = A.ro[g] + A.rk[g] * (pg - 200.0) / 1000.0;   // column term of rolloff_db_l
-          double *oc = oe + (int64_t)(g - g0) * rows;
-          float4 *oc32 = oe32 + (int64_t)(g - 1 - g0) * rows;
-#pragma unroll
-          for (int i = 0; i < AMP_RPT; i++) {
-            const int j = rb + i * 256 + (int)threadIdx.x + 1;
-            if (j > rows) continue;
-            double v;
-            if (!tabled) {
-              v = ampl_exact(sp, A, C, e, j, g);
-            } else {
-              if (rs_[i] == 0) {
-                double r = rolloff_db_s(rh_[i], lg[i], pg, slope, roctg, C.any_oct != 0, sp.rolloffParab,
-                                        C.parab_harm, C.parab_a, C.parab_b, C.parab_c, 200.0, sp.throwaway,
-                                        sp.samplingRate);
-                v = exp2((r - cmg) / 10.0) * shg;
-              } else {
-                v = A0[rk_[i]] * ML[(rs_[i] - 1) * (AMP_CG + 1) + gi] + A0[rk_[i] + 1] * MU[(rs_[i] - 1) * (AMP_CG + 1) + gi];
-              }
-              if (n > 0 && v < thr01) v = 0.0;
-            }
-            if (g < gb) oc[j - 1] = v;
-            if (g > ga) {   // {Y, Y, dY, dY}: one 16-byte load gives K1 both packed FFMA2 operands
-              const float y = (float)prev[i], dy = (float)(v - prev[i]);
-              if (tc_ep) reinterpret_cast<float2 *>(oe32)[(int64_t)(g - 1 - g0) * rows + (j - 1)] = make_float2(y, dy);
-              else oc32[j - 1] = make_float4(y, y, dy, dy);
-            }
-            prev[i] = v;
-          }
+        const int64_t i = (int64_t)(g - g0) * rows + (j - 1);
+        if (g < gb) oe[i] = v;
+        if (g > ga) {
+          const float y = (float)prev, dy = (float)(v - prev);
+          if (tc_ep) oe2[i - rows] = make_float2(y, dy);
+          else oe32[i - rows] = make_float4(y, y, dy, dy);
         }
+        prev = v;
       }
     }
   }

@@ -175,6 +175,33 @@ def thinned(calls, points=60):
     return out
 
 
+def amp_paths(seed=20260010):
+    """One call per code path of the amplitude kernel K3, 400 ms each at 48 kHz: epochs without sub-harmonics on both
+    sides of the tensor-core row threshold (224) and with more than 1024 kept rows, dense sub-harmonic epochs up to
+    more than 2560 rows, sub-harmonic epochs of fewer than 512 rows, and untabled epochs (more than 16 sub-harmonics,
+    or more than 1024 kept rows with sub-harmonics)."""
+    r = np.random.default_rng(seed)
+    cases = [(60, 90, 35, 60),      # dense: 600-1900 rows, several epochs
+             (50, 55, 9, 100),      # n = 5 on up to 479 kept rows: more than 2560 rows
+             (100, 110, 40, 0),     # no sub-harmonics, > 224 rows
+             (400, 420, 40, 0),     # no sub-harmonics, < 224 rows
+             (300, 320, 150, 80),   # n = 1, < 512 rows (and < 224)
+             (180, 200, 90, 80),    # n = 1, 224-512 rows
+             (80, 160, 60, 80),     # epochs without and with sub-harmonics in one syllable
+             (400, 410, 20, 100),   # n > 16: untabled
+             (21, 22, 40, 0),       # > 1024 kept rows, no sub-harmonics
+             (21, 22, 10, 100)]     # > 1024 kept rows with sub-harmonics: untabled
+    out = []
+    for lo, hi, sub_freq, sub_dep in cases:
+        out.append(dict(
+            sylLen=400, samplingRate=48000, invalidArgAction='ignore', temperature=0, pitchFloor=1,
+            pitchAnchors=(host.seq_len(0, 1, 2), [lo, hi]), contour_method='spline',
+            rolloff=r.uniform(-6, -1), rolloffOct=0, rolloffKHz=0, nonlinBalance=100,
+            jitterDep=r.uniform(0.5, 2), jitterLen=r.uniform(1, 20), shimmerDep=r.uniform(5, 30),
+            subFreq=sub_freq, subDep=sub_dep, shortestEpoch=100, z=[r.standard_normal(1024)]))
+    return out
+
+
 CONFIGS = {0: config0, 1: config1, 2: config2, 3: config3, 4: config4}
 NAMES = {0: 'cfg0 soundgen() defaults, 1 x 1000 ms @ 16 kHz',
          1: 'cfg1 voiced batch, 1024 x 500 ms @ 44.1 kHz',
