@@ -11,7 +11,8 @@
 // glottal cycle of one epoch, a "unit") at a time:
 //   * it stages the amplitude operand of the interval ONCE: Y | dY of up to 1152 rows from K3's FP32 table, scaled by
 //     a power of two and split hi + lo in FP16 (22 significant bits), in shared memory in the canonical K-major
-//     core-matrix layout, one image per pass of 384 rows;
+//     core-matrix layout, one image per pass of 384 rows; the rows arrive by cp.async while the unit before runs,
+//     and rows above the highest nonzero one (they add exactly 0) are skipped in whole block pairs;
 //   * per tile of 128 samples (thread = sample = TMEM lane) every thread writes its trig row cos / sin(m theta'),
 //     m < KR, hi + lo in FP16, into TMEM with tcgen05.st: the A operand of the MMAs never touches shared memory;
 //   * per pass two threads issue three tcgen05.mma kind::f16 each (M 128, N = 2 x blocks <= 48, K 16: hi hi + lo hi +
@@ -119,7 +120,8 @@ __global__ void k_build_units_tc(const sgb_syllable *syl, const SylCtrl *ctrl, i
 #define TC_B_PASSES 3                             // passes whose amplitude operand is resident (1152 rows)
 #define TC_MAX_ROWS (TC_B_PASSES * TC_PASS_ROWS)
 #define TC_IMG_BYTES (2 * TC_PASS_BLOCKS * TC_KR * 2)  // one FP16 amplitude image of a pass: 48 columns (Y, dY of 24 blocks) x KR
-#define TC_SMEM (TC_B_PASSES * 2 * TC_IMG_BYTES)
+#define TC_IMGS_BYTES (TC_B_PASSES * 2 * TC_IMG_BYTES)
+#define TC_SMEM (TC_IMGS_BYTES + 2 * TC_MAX_ROWS * 8)   // the images, then two staging buffers of {Y, dY} rows
 #define TC_NPC 4                                  // spline pieces staged per unit (an interval spans two or three)
 // instruction descriptor of kind::f16: FP16 x FP16 -> FP32, both operands K-major, M 128
 #define TC_IDESC(N) ((1u << 4) | ((uint32_t)((N) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24))
@@ -171,16 +173,58 @@ __device__ __forceinline__ void tc_issue_chain(uint32_t tmem_d, uint32_t tmem_a_
   tc_mma_ts(tmem_d, tmem_a_hi, descB + (uint64_t)(TC_IMG_BYTES >> 4), idesc, 1u);
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar_addr) : "memory");
 }
+// global -> shared without a register round trip (L1-allocating): 8 B for a {Y, dY} row (a column starts on any
+// pair, so wider copies would be misaligned), 16 B for the unit record
+__device__ __forceinline__ void tc_cp8(void *s, const void *g) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" :: "r"(tc_smem_u32(s)), "l"(g) : "memory");
+}
+__device__ __forceinline__ void tc_cp16(void *s, const void *g) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" :: "r"(tc_smem_u32(s)), "l"(g) : "memory");
+}
 
 __global__ void __launch_bounds__(128, 4)
 k_synth_tc(const TcUnit *__restrict__ units, int nunits, const double *__restrict__ pc, const float4 *__restrict__ amp,
            float *__restrict__ wave, int *__restrict__ epmax) {
-  extern __shared__ __align__(1024) uint8_t sB[];        // per resident pass: hi, lo images of the amplitude operand
+  // per resident pass: hi, lo images of the amplitude operand; then two staging buffers of TC_MAX_ROWS {Y, dY} rows
+  extern __shared__ __align__(1024) uint8_t sB[];
+  float2 *const stage = reinterpret_cast<float2 *>(sB + TC_IMGS_BYTES);
   __shared__ uint64_t bar;
-  __shared__ double spc[TC_NPC * SYNTH_PC];   // the unit's first spline pieces {knot, c0..c4}
+  __shared__ __align__(16) TcUnit su[2];               // the current and the next unit
+  __shared__ double spc[2][TC_NPC * SYNTH_PC];        // their first spline pieces {knot, c0..c4}
   __shared__ float smax[4];
+  __shared__ int stop[4];
   __shared__ uint32_t tmem_base_s;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const float2 *__restrict__ amp2 = reinterpret_cast<const float2 *>(amp);
+
+  // ---- operand prefetch, one item (super-pass of a unit) ahead, with cp.async: the item's {Y, dY} rows into a staging
+  // buffer (row0 + r at r), and for a new unit its record and spline pieces.  Waited for, and made visible by a
+  // barrier, at the end of the item before.  The next unit's column and pieces are loaded when the current unit
+  // starts and used after its staging, so that the loads are in flight meanwhile.
+  int64_t ncol = 0, npco = 0;
+  int nJ = 0, nG = 0, nalo = 0;
+  auto locate_unit = [&](int u) {
+    const TcUnit *N = units + u;
+    ncol = __ldg(&N->col_off); nJ = __ldg(&N->J);
+    npco = __ldg(&N->pc_off); nG = __ldg(&N->G); nalo = __ldg(&N->a_lo);
+  };
+  auto fetch_rows = [&](float2 *dst, const float2 *col, int J, int row0) {    // rows j = 0 (zero) .. J: col[j - 1]
+#pragma unroll
+    for (int i = 0; i < TC_MAX_ROWS / 128; i++) {
+      const int j = row0 + tid + 128 * i;
+      if (j >= 1 && j <= J) tc_cp8(dst + tid + 128 * i, col + (j - 1));
+    }
+  };
+  auto fetch_unit = [&](int u, int ub, int buf) {
+    if (tid < (int)(sizeof(TcUnit) / 16)) tc_cp16(reinterpret_cast<uint4 *>(&su[ub]) + tid, reinterpret_cast<const uint4 *>(units + u) + tid);
+    if (tid < TC_NPC * SYNTH_PC && nG > 0)     // pieces a_lo .. a_lo + 3 (the syllable has G of them)
+      tc_cp8(&spc[ub][tid], pc + SYNTH_PC * (npco + min(nalo + tid / SYNTH_PC, nG - 1)) + tid % SYNTH_PC);
+    fetch_rows(stage + buf * TC_MAX_ROWS, amp2 + ncol, nJ, 0);
+  };
+  int ui = blockIdx.x, ub = 0, buf = 0;       // unit, its buffer (su, spc), the current item's staging buffer
+  if (ui < nunits) { locate_unit(ui); fetch_unit(ui, 0, 0); }
+  asm volatile("cp.async.commit_group;" ::: "memory");
+
   if (warp == 0) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(tc_smem_u32(&tmem_base_s)), "n"(128));
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
@@ -189,6 +233,7 @@ k_synth_tc(const TcUnit *__restrict__ units, int nunits, const double *__restric
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 2;" :: "r"(tc_smem_u32(&bar)));
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
+  asm volatile("cp.async.wait_all;" ::: "memory");
   asm volatile("tcgen05.fence::before_thread_sync;");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;");
@@ -203,200 +248,229 @@ k_synth_tc(const TcUnit *__restrict__ units, int nunits, const double *__restric
   bool dead = false;
   TP_DECL
 
-  for (int ui = blockIdx.x; ui < nunits && !dead; ui += gridDim.x) {
-    const TcUnit U = units[ui];
-    if (U.kend <= U.kbeg) continue;
-    TP(0)
+  for (; ui < nunits && !dead; ui += gridDim.x, ub ^= 1) {
+    const TcUnit U = su[ub];
+    const int un = ui + gridDim.x;
+    if (un < nunits) locate_unit(un);
+    const bool work = U.kend > U.kbeg;
     const int J = U.J;
-    const float2 *__restrict__ col = reinterpret_cast<const float2 *>(amp) + U.col_off;   // {Y, dY} of the interval, row j - 1
+    const float2 *__restrict__ col = amp2 + U.col_off;                // {Y, dY} of the interval, row j - 1
     const double *__restrict__ pcs = pc + SYNTH_PC * U.pc_off;
+    const double *spcu = spc[ub];
     const int x_first_i = (int)U.x_first;
     const float inv_dx = __frcp_rn((float)(U.xn - U.xg));
-    const int nrows = J + 1;                                        // rows j = 0 (zero) .. J
-    const int nsuper = (nrows + TC_MAX_ROWS - 1) / TC_MAX_ROWS;
+    const int nsuper = work ? (J + TC_MAX_ROWS) / TC_MAX_ROWS : 1;    // rows j = 0 (zero) .. J, 1152 per super-pass
+    float unit_max = 0.f;
 
-    for (int sp = 0; sp < nsuper; sp++) {
-      const int row0 = sp * TC_MAX_ROWS;
-      const int rows_here = min(nrows - row0, TC_MAX_ROWS);
-      const int blocks_here = ((rows_here + TC_KR - 1) / TC_KR + 7) & ~7;    // N = 2 x blocks is a multiple of 16
-      if (sp == 0 && tid < TC_NPC * SYNTH_PC) {        // pieces a_lo .. a_lo + 3 (the syllable has G of them)
-        const int pi = min(U.a_lo + tid / SYNTH_PC, U.G - 1);
-        spc[tid] = __ldg(&pcs[SYNTH_PC * pi + tid % SYNTH_PC]);
-      }
-      // ---- amplitude operand: rows row0 .. row0 + 16 blocks_here - 1, scaled by a power of two so that the largest
-      // |Y|, |dY| sits in [2^14, 2^15): hi + lo in FP16 then carry 22 bits of every value down to 2^-39 of the largest ----
-      float yv[TC_MAX_ROWS / 128], dv[TC_MAX_ROWS / 128];
-      float mx = 0.f;
-#pragma unroll
-      for (int i = 0; i < TC_MAX_ROWS / 128; i++) {
-        const int j = row0 + tid + 128 * i;
-        yv[i] = 0.f; dv[i] = 0.f;
-        if (tid + 128 * i < blocks_here * TC_KR && j >= 1 && j <= J) { const float2 q = __ldg(&col[j - 1]); yv[i] = q.x; dv[i] = q.y; }
-        mx = fmaxf(mx, fmaxf(fabsf(yv[i]), fabsf(dv[i])));
-      }
-#pragma unroll
-      for (int of = 16; of > 0; of >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, of));
-      if (lane == 0) smax[warp] = mx;
-      __syncthreads();
-      mx = fmaxf(fmaxf(smax[0], smax[1]), fmaxf(smax[2], smax[3]));
-      const int ex = (mx > 0.f && mx < 3.0e38f) ? ilogbf(mx) : 14;
-      const float scale = scalbnf(1.0f, 14 - ex), unscale = scalbnf(1.0f, ex - 14);
-#pragma unroll
-      for (int i = 0; i < TC_MAX_ROWS / 128; i++) {
-        const int r = tid + 128 * i;
-        if (r < blocks_here * TC_KR) {
-          const int p = r / TC_PASS_ROWS, rr = r % TC_PASS_ROWS, b = rr / TC_KR, m = rr % TC_KR;
-          const float ys = yv[i] * scale, ds = dv[i] * scale;
-          const __half yh = __float2half_rn(ys), dh = __float2half_rn(ds);
-          const __half yl = __float2half_rn(ys - __half2float(yh)), dl = __float2half_rn(ds - __half2float(dh));
-          // accumulator columns of a block pair: {Y_2q, Y_2q+1, dY_2q, dY_2q+1} (register pairs for the packed epilogue)
-          uint8_t *hi = sB + p * (2 * TC_IMG_BYTES) + tc_off16(4 * (b >> 1) + (b & 1), m), *lo = hi + TC_IMG_BYTES;
-          *reinterpret_cast<__half *>(hi) = yh; *reinterpret_cast<__half *>(hi + 32) = dh;
-          *reinterpret_cast<__half *>(lo) = yl; *reinterpret_cast<__half *>(lo + 32) = dl;
-        }
-      }
-      const int npass = (blocks_here + TC_PASS_BLOCKS - 1) / TC_PASS_BLOCKS;
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      __syncthreads();                               // spc, sB
-      TP(1)
-
-      // phase of sample k of the unit: FP64 closed form of the spline piece; returns integr / (nSubharm + 1) in cycles
-      auto sample_phase = [&](int k, float &ww_out) -> double {
-        const double v = (k >= U.Ne - 1) ? U.x_last : (U.x_first + (double)k * U.by);
-        ww_out = (float)(v - (double)U.xg) * inv_dx;
-        const double u = (double)(x_first_i + k);
-        int a = 0;                               // piece: largest a with knot <= u; staged ones first
-        const int na = min(TC_NPC, U.G - U.a_lo);
-        while (a < na - 1 && u >= spc[SYNTH_PC * (a + 1)]) a++;
-        double p0 = spc[SYNTH_PC * a], p1 = spc[SYNTH_PC * a + 1], p2 = spc[SYNTH_PC * a + 2], p3 = spc[SYNTH_PC * a + 3],
-               p4 = spc[SYNTH_PC * a + 4], p5 = spc[SYNTH_PC * a + 5];
-        if (a == TC_NPC - 1) {                   // rare: the interval reaches past the staged pieces
-          int ag = U.a_lo + a;
-          while (ag < U.G - 1 && u >= pcs[SYNTH_PC * (ag + 1)]) ag++;
-          const double *pp = pcs + SYNTH_PC * ag;
-          p0 = pp[0]; p1 = pp[1]; p2 = pp[2]; p3 = pp[3]; p4 = pp[4]; p5 = pp[5];
-        }
-        const double M = u - p0;
-        const double ph = fma(fma(fma(fma(p5, M, p4), M, p3), M, p2), M, p1);
-        const double x = ph * U.inv_sr_np1;
-        return x - floor(x);
+    for (int sp = 0; sp < nsuper && !dead; sp++, buf ^= 1) {
+      bool fetched = false;
+      auto prefetch = [&]() {
+        if (sp + 1 < nsuper) fetch_rows(stage + (buf ^ 1) * TC_MAX_ROWS, col, J, (sp + 1) * TC_MAX_ROWS);
+        else if (un < nunits) fetch_unit(un, ub ^ 1, buf ^ 1);
+        asm volatile("cp.async.commit_group;" ::: "memory");
+        fetched = true;
       };
-      float ww_n;
-      double x_n = sample_phase(min(U.kbeg + tid, U.kend - 1), ww_n);
-      float unit_max = 0.f;
-
-      for (int k0 = U.kbeg; k0 < U.kend && !dead; k0 += TC_TILE) {
-        // ---- this thread's sample: interval weight and phase (computed one tile ahead, in the shadow of the MMAs) ----
-        const bool live = k0 + tid < U.kend;
-        const int k = live ? k0 + tid : k0;
-        const float ww = ww_n;
-        const double x = x_n;
-        TP(2)
-        // ---- trig operand rows: cos / sin (m theta'), m < KR, hi + lo in FP16, into this thread's TMEM lane; even and
-        // odd m are two packed FP32 chains and share a column ----
-        {
-          float s1, c1;
-          sincospif(2.0f * (float)x, &s1, &c1);
-          const float c2 = fmaf(c1, c1, -(s1 * s1)), s2 = 2.0f * s1 * c1;        // e^{2 i theta'}
-          const float2 C2 = make_float2(c2, c2), S2 = make_float2(s2, s2), nS2 = make_float2(-s2, -s2);
-          float2 cm = make_float2(1.f, c1), sm = make_float2(0.f, s1);            // rows m, m + 1
-          uint32_t ch[8], cl[8], sh[8], sl[8];
+      if (work) {
+        TP(0)
+        const int row0 = sp * TC_MAX_ROWS;
+        const float2 *stg = stage + buf * TC_MAX_ROWS;
+        // ---- amplitude operand: rows row0 .. row0 + 16 blocks - 1, scaled by a power of two so that the largest
+        // |Y|, |dY| sits in [2^14, 2^15): hi + lo in FP16 then carry 22 bits of every value down to 2^-39 of the
+        // largest.  Rows above the highest one with Y != 0 or dY != 0 (the live top) contribute exactly 0 and are
+        // left out in whole block pairs: blocks, passes and the Horner start follow the live top ----
+        float mx = 0.f;
+        int top = -1;
 #pragma unroll
-          for (int h = 0; h < TC_KR / 2; h++) {
-            tc_split16(cm, ch[h], cl[h]); tc_split16(sm, sh[h], sl[h]);
-            const float2 nc = __ffma2_rn(cm, C2, __fmul2_rn(sm, nS2)), ns = __ffma2_rn(cm, S2, __fmul2_rn(sm, C2));
-            cm = nc; sm = ns;
+        for (int i = 0; i < TC_MAX_ROWS / 128; i++) {
+          const int r = tid + 128 * i, j = row0 + r;
+          if (j >= 1 && j <= J) {
+            const float2 q = stg[r];
+            mx = fmaxf(mx, fmaxf(fabsf(q.x), fabsf(q.y)));
+            if (q.x != 0.f || q.y != 0.f) top = r;
           }
-          tc_st8(lane_addr + TC_COL_CH, ch); tc_st8(lane_addr + TC_COL_CL, cl);
-          tc_st8(lane_addr + TC_COL_SH, sh); tc_st8(lane_addr + TC_COL_SL, sl);
-          asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
         }
-        TP(3)
-        asm volatile("tcgen05.fence::before_thread_sync;");
+#pragma unroll
+        for (int of = 16; of > 0; of >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, of));
+        top = __reduce_max_sync(0xffffffffu, top);
+        if (lane == 0) { smax[warp] = mx; stop[warp] = top; }
         __syncthreads();
-        if (issuer) {
-          asm volatile("tcgen05.fence::after_thread_sync;");
-          tc_issue_chain(my_d, my_ahi, my_alo, descB, min(blocks_here, TC_PASS_BLOCKS), barA);
+        mx = fmaxf(fmaxf(smax[0], smax[1]), fmaxf(smax[2], smax[3]));
+        top = max(max(stop[0], stop[1]), max(stop[2], stop[3]));
+        const int ex = (mx > 0.f && mx < 3.0e38f) ? ilogbf(mx) : 14;
+        const float scale = scalbnf(1.0f, 14 - ex), unscale = scalbnf(1.0f, ex - 14);
+        const int lblocks = (top + TC_KR) / TC_KR;                      // blocks up to the live top (0: none)
+        const int blocks = (lblocks + 7) & ~7;                          // N = 2 x blocks is a multiple of 16
+        const int npass = (blocks + TC_PASS_BLOCKS - 1) / TC_PASS_BLOCKS;
+        const int qtop = (((lblocks - 1) % TC_PASS_BLOCKS) >> 1) & 3;  // top block pair of the last pass, in its group
+#pragma unroll
+        for (int i = 0; i < TC_MAX_ROWS / 128; i++) {
+          const int r = tid + 128 * i, j = row0 + r;
+          if (r < blocks * TC_KR) {
+            const float2 q = (j >= 1 && j <= J) ? stg[r] : make_float2(0.f, 0.f);
+            const int p = r / TC_PASS_ROWS, rr = r % TC_PASS_ROWS, b = rr / TC_KR, m = rr % TC_KR;
+            const float ys = q.x * scale, ds = q.y * scale;
+            const __half yh = __float2half_rn(ys), dh = __float2half_rn(ds);
+            const __half yl = __float2half_rn(ys - __half2float(yh)), dl = __float2half_rn(ds - __half2float(dh));
+            // accumulator columns of a block pair: {Y_2q, Y_2q+1, dY_2q, dY_2q+1} (register pairs for the packed epilogue)
+            uint8_t *hi = sB + p * (2 * TC_IMG_BYTES) + tc_off16(4 * (b >> 1) + (b & 1), m), *lo = hi + TC_IMG_BYTES;
+            *reinterpret_cast<__half *>(hi) = yh; *reinterpret_cast<__half *>(hi + 32) = dh;
+            *reinterpret_cast<__half *>(lo) = yl; *reinterpret_cast<__half *>(lo + 32) = dl;
+          }
         }
-        TP(4)
-        // in the shadow of the first MMAs: z = e^{i KR theta'}, z^2, the pass rotation P = e^{i 384 theta'}, E = e^{i row0 theta'}
-        float zc, zs;
-        { double q = x * (double)TC_KR; q -= floor(q); sincospif(2.0f * (float)q, &zs, &zc); }
-        const float zc2 = fmaf(zc, zc, -(zs * zs)), zs2 = 2.0f * zs * zc;
-        const float2 z2c = make_float2(zc2, zc2), z2s = make_float2(zs2, zs2), nz2s = make_float2(-zs2, -zs2);
-        const float2 ww2 = make_float2(ww, ww);
-        float ec = 1.f, es = 0.f, pc_ = 1.f, ps_ = 0.f;
-        if (npass > 1) { double q = x * (double)TC_PASS_ROWS; q -= floor(q); sincospif(2.0f * (float)q, &ps_, &pc_); }
-        float acc = 0.f, prev = 0.f;
-        if (sp > 0) {
-          double q = x * (double)row0; q -= floor(q); sincospif(2.0f * (float)q, &es, &ec);
-          if (live) prev = wave[U.wave_off + k];
-        }
-        if (k0 + TC_TILE < U.kend) x_n = sample_phase(min(k0 + TC_TILE + tid, U.kend - 1), ww_n);
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        __syncthreads();                               // sB
+        TP(1)
+        auto pass_blocks = [&](int p) { return min(blocks - p * TC_PASS_BLOCKS, TC_PASS_BLOCKS); };   // 8, 16 or 24
 
-        for (int p = 0; p < npass; p++) {
-          const int nb = min(blocks_here - p * TC_PASS_BLOCKS, TC_PASS_BLOCKS);   // 8, 16 or 24 blocks
-          uint32_t ok = 0, polls = 0;
-          while (!ok) {
-            asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.b32 %0, 1, 0, p;\n}\n"
-                         : "=r"(ok) : "r"(barA), "r"(phase) : "memory");
-            if (!ok && ++polls > (1u << 24)) { g_tc_timeout = 1; dead = true; break; }
+        // phase of sample k of the unit: FP64 closed form of the spline piece; returns integr / (nSubharm + 1) in cycles
+        auto sample_phase = [&](int k, float &ww_out) -> double {
+          const double v = (k >= U.Ne - 1) ? U.x_last : (U.x_first + (double)k * U.by);
+          ww_out = (float)(v - (double)U.xg) * inv_dx;
+          const double u = (double)(x_first_i + k);
+          int a = 0;                               // piece: largest a with knot <= u; staged ones first
+          const int na = min(TC_NPC, U.G - U.a_lo);
+          while (a < na - 1 && u >= spcu[SYNTH_PC * (a + 1)]) a++;
+          double p0 = spcu[SYNTH_PC * a], p1 = spcu[SYNTH_PC * a + 1], p2 = spcu[SYNTH_PC * a + 2], p3 = spcu[SYNTH_PC * a + 3],
+                 p4 = spcu[SYNTH_PC * a + 4], p5 = spcu[SYNTH_PC * a + 5];
+          if (a == TC_NPC - 1) {                   // rare: the interval reaches past the staged pieces
+            int ag = U.a_lo + a;
+            while (ag < U.G - 1 && u >= pcs[SYNTH_PC * (ag + 1)]) ag++;
+            const double *pp = pcs + SYNTH_PC * ag;
+            p0 = pp[0]; p1 = pp[1]; p2 = pp[2]; p3 = pp[3]; p4 = pp[4]; p5 = pp[5];
           }
-          phase ^= 1u;
-          TP(5)
-          asm volatile("tcgen05.fence::after_thread_sync;");
-          // ---- R = sum_b z^b (S_b - i C_b): Horner in z^2 from the top, even and odd blocks as the two halves of
-          // packed FP32 pairs; Q = -Im R ----
-          float2 Rr = make_float2(0.f, 0.f), Q = make_float2(0.f, 0.f);
-          float Cv[2][16], Sv[2][16];                      // 8 blocks = 16 accumulator columns of C and of S, two in flight
-          int g = nb / 8 - 1;
-          tc_ld16(lane_addr + TC_COL_C + 16 * g, Cv[0]); tc_ld16(lane_addr + TC_COL_S + 16 * g, Sv[0]);
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+          const double M = u - p0;
+          const double ph = fma(fma(fma(fma(p5, M, p4), M, p3), M, p2), M, p1);
+          const double x = ph * U.inv_sr_np1;
+          return x - floor(x);
+        };
+        // a super-pass after the first with no live row adds exactly 0: its samples keep what the one before wrote.  A
+        // first super-pass without one still writes its zeros, and issues no MMA
+        if (sp == 0 || npass > 0) {
+          float ww_n;
+          double x_n = sample_phase(min(U.kbeg + tid, U.kend - 1), ww_n);
+          unit_max = 0.f;
+
+          for (int k0 = U.kbeg; k0 < U.kend && !dead; k0 += TC_TILE) {
+            // ---- this thread's sample: interval weight and phase (computed one tile ahead, in the shadow of the MMAs) ----
+            const bool live = k0 + tid < U.kend;
+            const int k = live ? k0 + tid : k0;
+            const float ww = ww_n;
+            const double x = x_n;
+            TP(2)
+            // ---- trig operand rows: cos / sin (m theta'), m < KR, hi + lo in FP16, into this thread's TMEM lane; even and
+            // odd m are two packed FP32 chains and share a column ----
+            if (npass > 0) {
+              {
+                float s1, c1;
+                sincospif(2.0f * (float)x, &s1, &c1);
+                const float c2 = fmaf(c1, c1, -(s1 * s1)), s2 = 2.0f * s1 * c1;        // e^{2 i theta'}
+                const float2 C2 = make_float2(c2, c2), S2 = make_float2(s2, s2), nS2 = make_float2(-s2, -s2);
+                float2 cm = make_float2(1.f, c1), sm = make_float2(0.f, s1);            // rows m, m + 1
+                uint32_t ch[8], cl[8], sh[8], sl[8];
 #pragma unroll
-          for (int it = 0; it < TC_PASS_BLOCKS / 8; it++) {
-            const int cur = it & 1;
-            if (g - it < 0) break;
-            if (g - it - 1 >= 0) {
-              tc_ld16(lane_addr + TC_COL_C + 16 * (g - it - 1), Cv[cur ^ 1]); tc_ld16(lane_addr + TC_COL_S + 16 * (g - it - 1), Sv[cur ^ 1]);
+                for (int h = 0; h < TC_KR / 2; h++) {
+                  tc_split16(cm, ch[h], cl[h]); tc_split16(sm, sh[h], sl[h]);
+                  const float2 nc = __ffma2_rn(cm, C2, __fmul2_rn(sm, nS2)), ns = __ffma2_rn(cm, S2, __fmul2_rn(sm, C2));
+                  cm = nc; sm = ns;
+                }
+                tc_st8(lane_addr + TC_COL_CH, ch); tc_st8(lane_addr + TC_COL_CL, cl);
+                tc_st8(lane_addr + TC_COL_SH, sh); tc_st8(lane_addr + TC_COL_SL, sl);
+                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+              }
+              TP(3)
+              asm volatile("tcgen05.fence::before_thread_sync;");
+              __syncthreads();
+              if (issuer) {
+                asm volatile("tcgen05.fence::after_thread_sync;");
+                tc_issue_chain(my_d, my_ahi, my_alo, descB, pass_blocks(0), barA);
+              }
             }
+            TP(4)
+            // in the shadow of the first MMAs: z = e^{i KR theta'}, z^2, the pass rotation P = e^{i 384 theta'}, E = e^{i row0 theta'}
+            float zc, zs;
+            { double q = x * (double)TC_KR; q -= floor(q); sincospif(2.0f * (float)q, &zs, &zc); }
+            const float zc2 = fmaf(zc, zc, -(zs * zs)), zs2 = 2.0f * zs * zc;
+            const float2 z2c = make_float2(zc2, zc2), z2s = make_float2(zs2, zs2), nz2s = make_float2(-zs2, -zs2);
+            const float2 ww2 = make_float2(ww, ww);
+            float ec = 1.f, es = 0.f, pc_ = 1.f, ps_ = 0.f;
+            if (npass > 1) { double q = x * (double)TC_PASS_ROWS; q -= floor(q); sincospif(2.0f * (float)q, &ps_, &pc_); }
+            float acc = 0.f, prev = 0.f;
+            if (sp > 0) {
+              double q = x * (double)row0; q -= floor(q); sincospif(2.0f * (float)q, &es, &ec);
+              if (live) prev = wave[U.wave_off + k];
+            }
+            if (k0 + TC_TILE < U.kend) x_n = sample_phase(min(k0 + TC_TILE + tid, U.kend - 1), ww_n);
+            if (k0 == U.kbeg) prefetch();
+
+            for (int p = 0; p < npass; p++) {
+              const int nb = pass_blocks(p);
+              uint32_t ok = 0, polls = 0;
+              while (!ok) {
+                asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.b32 %0, 1, 0, p;\n}\n"
+                             : "=r"(ok) : "r"(barA), "r"(phase) : "memory");
+                if (!ok && ++polls > (1u << 24)) { g_tc_timeout = 1; dead = true; break; }
+              }
+              phase ^= 1u;
+              TP(5)
+              asm volatile("tcgen05.fence::after_thread_sync;");
+              // ---- R = sum_b z^b (S_b - i C_b): Horner in z^2 from the top live block pair, even and odd blocks as the
+              // two halves of packed FP32 pairs; Q = -Im R ----
+              float2 Rr = make_float2(0.f, 0.f), Q = make_float2(0.f, 0.f);
+              float Cv[2][16], Sv[2][16];                      // 8 blocks = 16 accumulator columns of C and of S, two in flight
+              const int g = nb / 8 - 1, qt = p == npass - 1 ? qtop : 3;
+              tc_ld16(lane_addr + TC_COL_C + 16 * g, Cv[0]); tc_ld16(lane_addr + TC_COL_S + 16 * g, Sv[0]);
+              asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
-            for (int q = 3; q >= 0; q--) {
-              const float2 Cc = __ffma2_rn(ww2, make_float2(Cv[cur][4 * q + 2], Cv[cur][4 * q + 3]), make_float2(Cv[cur][4 * q], Cv[cur][4 * q + 1]));
-              const float2 Ss = __ffma2_rn(ww2, make_float2(Sv[cur][4 * q + 2], Sv[cur][4 * q + 3]), make_float2(Sv[cur][4 * q], Sv[cur][4 * q + 1]));
-              const float2 nr = __ffma2_rn(Rr, z2c, __ffma2_rn(Q, z2s, Ss)), nq = __ffma2_rn(Rr, nz2s, __ffma2_rn(Q, z2c, Cc));
-              Rr = nr; Q = nq;
+              for (int it = 0; it < TC_PASS_BLOCKS / 8; it++) {
+                const int cur = it & 1;
+                if (g - it < 0) break;
+                if (g - it - 1 >= 0) {
+                  tc_ld16(lane_addr + TC_COL_C + 16 * (g - it - 1), Cv[cur ^ 1]); tc_ld16(lane_addr + TC_COL_S + 16 * (g - it - 1), Sv[cur ^ 1]);
+                }
+#pragma unroll
+                for (int q = 3; q >= 0; q--) {
+                  if (it == 0 && q > qt) continue;
+                  const float2 Cc = __ffma2_rn(ww2, make_float2(Cv[cur][4 * q + 2], Cv[cur][4 * q + 3]), make_float2(Cv[cur][4 * q], Cv[cur][4 * q + 1]));
+                  const float2 Ss = __ffma2_rn(ww2, make_float2(Sv[cur][4 * q + 2], Sv[cur][4 * q + 3]), make_float2(Sv[cur][4 * q], Sv[cur][4 * q + 1]));
+                  const float2 nr = __ffma2_rn(Rr, z2c, __ffma2_rn(Q, z2s, Ss)), nq = __ffma2_rn(Rr, nz2s, __ffma2_rn(Q, z2c, Cc));
+                  Rr = nr; Q = nq;
+                }
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+              }
+              asm volatile("tcgen05.fence::before_thread_sync;");
+              __syncthreads();                       // the accumulators are free
+              if (issuer && p + 1 < npass) {
+                asm volatile("tcgen05.fence::after_thread_sync;");
+                tc_issue_chain(my_d, my_ahi, my_alo, descB + (uint64_t)(((p + 1) * 2 * TC_IMG_BYTES) >> 4), pass_blocks(p + 1), barA);
+              }
+              TP(6)
+              // R = R_even + z R_odd;  acc += Re (E R)
+              const float Rre = fmaf(zc, Rr.y, fmaf(zs, Q.y, Rr.x));            // zc Rr_o - zs Ri_o, Ri_o = -Q_o
+              const float Rim = fmaf(zs, Rr.y, fmaf(-zc, Q.y, -Q.x));           // zs Rr_o + zc Ri_o + Ri_e
+              acc = fmaf(ec, Rre, fmaf(-es, Rim, acc));
+              const float ne = fmaf(ec, pc_, -(es * ps_)), nsn = fmaf(ec, ps_, es * pc_); ec = ne; es = nsn;
+              TP(7)
             }
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            acc = fmaf(acc, unscale, prev);
+            if (live) wave[U.wave_off + k] = acc;
+            if (live) unit_max = fmaxf(unit_max, fabsf(acc));
+            TP(8)
           }
-          asm volatile("tcgen05.fence::before_thread_sync;");
-          __syncthreads();                       // the accumulators are free
-          if (issuer && p + 1 < npass) {
-            asm volatile("tcgen05.fence::after_thread_sync;");
-            tc_issue_chain(my_d, my_ahi, my_alo, descB + (uint64_t)(((p + 1) * 2 * TC_IMG_BYTES) >> 4),
-                           min(blocks_here - (p + 1) * TC_PASS_BLOCKS, TC_PASS_BLOCKS), barA);
-          }
-          TP(6)
-          // R = R_even + z R_odd;  acc += Re (E R)
-          const float Rre = fmaf(zc, Rr.y, fmaf(zs, Q.y, Rr.x));            // zc Rr_o - zs Ri_o, Ri_o = -Q_o
-          const float Rim = fmaf(zs, Rr.y, fmaf(-zc, Q.y, -Q.x));           // zs Rr_o + zc Ri_o + Ri_e
-          acc = fmaf(ec, Rre, fmaf(-es, Rim, acc));
-          const float ne = fmaf(ec, pc_, -(es * ps_)), nsn = fmaf(ec, ps_, es * pc_); ec = ne; es = nsn;
-          TP(7)
         }
-        acc = fmaf(acc, unscale, prev);
-        if (live) wave[U.wave_off + k] = acc;
-        if (live) unit_max = fmaxf(unit_max, fabsf(acc));
-        TP(8)
       }
-      if (sp == nsuper - 1) {        // max |w| of the epoch (tolerance of the zero-crossing searches in K6)
-#pragma unroll
+      if (work && sp == nsuper - 1) {   // max |w| of the epoch over what the last super-pass that ran wrote (tolerance of
+#pragma unroll                          // the zero-crossing searches in K6)
         for (int of = 16; of > 0; of >>= 1) unit_max = fmaxf(unit_max, __shfl_xor_sync(0xffffffffu, unit_max, of));
         if (lane == 0 && unit_max > 0.0f) atomicMax(&epmax[U.epmax_idx], float_to_ordered(unit_max));
       }
-      __syncthreads();               // sB, spc, smax are rewritten next: all MMAs completed above, every thread is past its reads
+      if (!fetched) prefetch();
+      asm volatile("cp.async.wait_all;" ::: "memory");
+      __syncthreads();               // sB, smax, stop and the staging buffer are rewritten next, su / spc one unit later:
+                                     // all MMAs completed above, every thread is past its reads; the prefetch landed
     }
   }
   TP_END
+  asm volatile("cp.async.wait_all;" ::: "memory");
   __syncthreads();
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem_base), "n"(128));
 }
