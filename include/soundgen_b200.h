@@ -345,6 +345,30 @@ typedef struct sgb_ceps_params {
 } sgb_ceps_params;
 int sgb_rows_cepstra(int32_t device, const float *src, int64_t src_elems, const int64_t *src_off,
                      const int64_t *frames, int32_t n, const sgb_ceps_params *p, const sgb_device_out *o);
+/* The f0 track of every call of the last run (K12a), aligned sample for sample with the rows sgb_batch_export
+ * writes: the fundamental frequency in Hz of the contour the harmonics of that sample were built on, 0 where the
+ * sample is unvoiced.  A sample is voiced when it lies in the span of a voiced syllable (not a pause, a silence, a
+ * noise-only stretch, a filter tail past the last syllable, or any sample of a failed call).  Its value is
+ * pitch_upsampled of the reference (source.R:382, after vibrato, jitter, drift and pitchAnchorsGlobal) at the
+ * sample's position in the epoch that produced it -- the incoming epoch inside a cross-fade, the first epoch's
+ * first sample for the two leading zeros of a syllable -- evaluated in FP64 from the spline piece K1's phase
+ * integrates, rounded to float once.  With sub-harmonics (nSubharm > 0) the partials are multiples of
+ * f0 / (nSubharm + 1); the track still reports f0.
+ * Layout, capacity, zero tail, crop, argument checks and stream contract are those of sgb_batch_export (row c gets
+ * exactly cap[c] floats, out_written[c] = min(len_c, cap_c)); format must be SGB_OUT_F32. */
+int sgb_batch_f0(sgb_batch *b, const sgb_device_out *o);
+/* Frame labels of n float32 rows on `device` (K12b), typically f0 tracks of sgb_batch_f0: row c = len[c] samples
+ * at src + src_off[c], inside [src, src + src_elems).  Frames k = 0 .. nc-1 are K9's for the same wl and overlap
+ * (start s_k = floor(1 + k h), nc = sgb_spec_frames(len, wl, overlap)); label k is two floats:
+ *   [x[s_k - 1 + wl/2] (0 at or past len),  (nonzero samples in [s_k - 1, s_k - 1 + wl) ∩ [0, len)) / wl],
+ * the count exact in integers and divided once.  Row c gets exactly cap[c] labels (2 cap[c] floats) from element
+ * dst_off[c] on, zeros past nc; out_written[c] = min(nc, cap[c]); a label does not depend on cap or on other rows.
+ * Refused before anything is queued with SGB_ERR_INVALID: wl odd or < 4, overlap outside [0, 100) or a hop below
+ * one sample, a format other than SGB_OUT_F32, a row outside src_elems, the export's checks on dst, a dst range
+ * that intersects [src, src + src_elems), src or dst not device memory of `device`.  No device: SGB_ERR_CUDA.
+ * Stream contract and pinned staging are those of the exports. */
+int sgb_rows_f0_frames(int32_t device, const float *src, int64_t src_elems, const int64_t *src_off,
+                       const int64_t *len, int32_t n, int32_t wl, double overlap, const sgb_device_out *o);
 /* default, low and high of a scalar argument of soundgen() as the front-end checks it (permittedValues,
  * R/presets.R:22-79); SGB_ERR_INVALID for a name the front-end does not range-check. */
 int sgb_param_range(const char *name, double out3[3]);

@@ -147,7 +147,7 @@ EXPORTS = ['sgb_version', 'sgb_last_error', 'sgb_device_count', 'sgb_set_device'
            'sgb_batch_create', 'sgb_batch_destroy', 'sgb_batch_upload', 'sgb_batch_run',
            'sgb_batch_lengths', 'sgb_batch_fetch_f32', 'sgb_batch_fetch_f64', 'sgb_batch_fetch_pcm16', 'sgb_batch_status',
            'sgb_batch_export', 'sgb_rows_export', 'sgb_spec_frames', 'sgb_batch_spectrogram', 'sgb_rows_spectrogram',
-           'sgb_rows_compare', 'sgb_rows_cepstra', 'sgb_param_range',
+           'sgb_rows_compare', 'sgb_rows_cepstra', 'sgb_batch_f0', 'sgb_rows_f0_frames', 'sgb_param_range',
            'sgb_batch_syllable_len', 'sgb_batch_syllable_fetch', 'sgb_batch_noise_fetch',
            'sgb_batch_artefacts', 'sgb_batch_artefact_ints', 'sgb_batch_pitch_per_gc', 'sgb_batch_amp_tables', 'sgb_batch_checksums', 'sgb_batch_debug_state',
            'sgb_get_rolloff', 'sgb_get_spectral_envelope', 'sgb_filter_len', 'sgb_filter',
@@ -204,6 +204,8 @@ def load():
     L.sgb_rows_spectrogram.argtypes = [i32, vp, vp, vp, i32, C.POINTER(SpecParams), C.POINTER(DeviceOut)]
     L.sgb_rows_compare.argtypes = [i32, vp, i64, vp, i64, vp, vp, vp, vp, i32, C.POINTER(CompareParams), vp, i64, vp]
     L.sgb_rows_cepstra.argtypes = [i32, vp, i64, vp, vp, i32, C.POINTER(CepsParams), C.POINTER(DeviceOut)]
+    L.sgb_batch_f0.argtypes = [vp, C.POINTER(DeviceOut)]
+    L.sgb_rows_f0_frames.argtypes = [i32, vp, i64, vp, vp, i32, i32, f64, C.POINTER(DeviceOut)]
     L.sgb_param_range.argtypes = [C.c_char_p, vp]
     L.sgb_batch_syllable_len.argtypes = [vp, i32, C.POINTER(i64)]
     L.sgb_batch_syllable_fetch.argtypes = [vp, i32, vp, i64]

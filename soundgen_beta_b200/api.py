@@ -679,6 +679,15 @@ class Batch:
         return _spectrogram(lambda p, o: self.L.sgb_batch_spectrogram(self.h, C.byref(p), C.byref(o)), n, dst, dst_off,
                             cap, wl, overlap, window, bands, db, db_floor, stream)
 
+    def f0(self, dst, dst_off, cap, stream=None):
+        """The f0 track of every call of the last run (K12a, sgb_batch_f0) into the float32 CUDA tensor `dst`, laid out
+        as export() lays out the samples: call c fills exactly cap[c] elements from element dst_off[c], the f0 in Hz of
+        each of its first min(len, cap) samples (0 where unvoiced) and then zeros.  With sub-harmonics the partials
+        are multiples of f0 / (nSubharm + 1); the track still reports f0.  Ordered on `stream` like export().
+        Returns the samples written per call."""
+        n = self.desc.n_calls if self.desc is not None else 0
+        return _export(lambda o: self.L.sgb_batch_f0(self.h, C.byref(o)), n, dst, dst_off, cap, stream, 'f32')
+
     def syllable(self, s):
         n = C.c_int64()
         _check(self.L.sgb_batch_syllable_len(self.h, s, C.byref(n)))
@@ -859,6 +868,59 @@ def rows_spectrogram(device, src, src_off, lens, dst, dst_off, cap, wl, overlap=
     return _spectrogram(lambda p, o: L.sgb_rows_spectrogram(int(device), src.data_ptr() or None, _ptr(so), _ptr(ln),
                                                             ln.size, C.byref(p), C.byref(o)),
                         ln.size, dst, dst_off, cap, wl, overlap, window, bands, db, db_floor, stream)
+
+
+def rows_f0_frames(device, src, src_off, lens, dst, dst_off, cap, wl, overlap=75, stream=None):
+    """sgb_rows_f0_frames (K12b): frame labels of float32 rows the caller holds in the CUDA tensor `src` (row c =
+    lens[c] samples from element src_off[c]), typically f0 tracks.  Frame k of a row is K9's frame k at the same wl
+    and overlap; its label is [f0 at the frame's centre sample, fraction of the frame's wl samples that are nonzero
+    (voiced)].  Row c fills exactly cap[c] labels (2 cap[c] floats) of the float32 CUDA tensor `dst` from element
+    dst_off[c], zeros past the row's frames.  Ordered on `stream` like export().  Returns the frames written per row."""
+    import torch
+    so = np.ascontiguousarray(src_off, dtype=np.int64)
+    ln = np.ascontiguousarray(lens, dtype=np.int64)
+    if not (torch.is_tensor(src) and src.is_contiguous() and src.dtype == torch.float32) or so.shape != ln.shape \
+            or so.ndim != 1:
+        raise ValueError('src must be a contiguous float32 tensor, src_off and lens of one length')
+    L = _abi.load()
+    return _export(lambda o: L.sgb_rows_f0_frames(int(device), src.data_ptr() or None, src.numel(), _ptr(so), _ptr(ln),
+                                                  ln.size, int(wl), float(overlap), C.byref(o)), ln.size, dst, dst_off,
+                   cap, stream, 'f32')
+
+
+def f0_frames_device(f0, lengths, samplingRate, windowLength=50, overlap=75):
+    """Frame labels of the [n, T] float32 f0 tracks that soundgen_batch_device(..., f0=True) returns, aligned frame
+    for frame with spectrogram_device(wave, lengths, samplingRate, windowLength, overlap): the same per-row window
+    wl = floor(windowLength / 1000 * sr / 2) * 2 at the row's rate (samplingRate: one value or one per row; one
+    library call per window length) and the same frames.  Returns (labels, frames): labels [n, F, 2] float32 on the
+    same device, labels[c, k] = [f0 at frame k's centre sample, voiced fraction of its wl samples], zeros past the
+    row's frames, F = the most frames of any row; frames: int64 CUDA tensor, equal to spectrogram_device's.  Ordered
+    on the device's current torch stream; a CUDA `lengths` is read back once."""
+    import torch
+    if not (torch.is_tensor(f0) and f0.is_cuda and f0.dtype == torch.float32 and f0.dim() == 2):
+        raise ValueError('f0 must be a 2-D float32 CUDA tensor')
+    n, T = f0.shape
+    lens = (lengths.cpu().numpy() if torch.is_tensor(lengths) else np.asarray(lengths)).astype(np.int64).reshape(-1)
+    if lens.shape != (n,) or np.any(lens < 0) or np.any(lens > T):
+        raise ValueError('lengths needs one value in [0, %d] per row (%d)' % (T, n))
+    sr = np.broadcast_to(np.asarray(samplingRate, dtype=np.float64).reshape(-1), (n,)) if n else np.zeros(0)
+    if not np.all(np.isfinite(sr) & (sr > 0)):
+        raise ValueError('samplingRate must be positive')
+    wl = (np.floor(windowLength / 1000 * sr / 2) * 2).astype(np.int64)
+    L = _abi.load()
+    nc = np.array([L.sgb_spec_frames(int(l), int(w), float(overlap)) for l, w in zip(lens, wl)], dtype=np.int64)
+    if np.any(nc < 0):
+        raise SoundgenError(_abi.SGB_ERR_UNSUPPORTED, 'window of %s points / overlap %r cannot be analysed'
+                            % (np.unique(wl[nc < 0]), overlap))
+    F = int(nc.max(initial=0))
+    labels = torch.empty((n, F, 2), dtype=torch.float32, device=f0.device)
+    if n and F:
+        src = f0.contiguous()
+        rows = np.arange(n, dtype=np.int64)
+        for w in np.unique(wl):
+            cap = np.where(wl == w, F, 0).astype(np.int64)
+            rows_f0_frames(f0.device.index, src, rows * T, lens, labels, rows * F * 2, cap, int(w), overlap)
+    return labels, torch.as_tensor(nc, dtype=torch.int64).to(f0.device)
 
 
 def _hz_to_mel(f, mel_scale):
@@ -1064,13 +1126,15 @@ def _torch_out_dtype(dtype):
     raise ValueError('dtype must be torch.float32 or torch.int16 (PCM16), not %r' % (dtype,))
 
 
-def soundgen_batch_device(calls, dtype=None, device=None, max_len=None, u_dtype=np.float64):
+def soundgen_batch_device(calls, dtype=None, device=None, max_len=None, u_dtype=np.float64, f0=False):
     """soundgen_batch with the waveforms delivered on the GPU: returns (wave, lengths, status).
     wave: [n_calls, T] tensor on the device, rows padded with zeros, T = max_len (longer calls are cropped) or else
     the longest call; lengths: int64 CUDA tensor of the samples present per row; status: as soundgen_batch returns it.
     dtype: torch.float32 (the samples soundgen() returns) or torch.int16 (16-bit PCM as seewave::savewav writes it,
     normalised over the whole call, before any cropping).  device: CUDA device index (default: torch's current one).
-    The result is ordered on the device's current torch stream."""
+    f0=True also returns the exact f0 track of every call (Batch.f0, K12a) as a fourth element: a [n_calls, T]
+    float32 tensor aligned sample for sample with wave (same rounds, offsets and crop), f0 in Hz, 0 where unvoiced and
+    in every row whose status is not 0.  The result is ordered on the device's current torch stream."""
     import torch
     fmt = _torch_out_dtype(torch.float32 if dtype is None else dtype)
     if max_len is not None and int(max_len) < 0:
@@ -1132,11 +1196,26 @@ def soundgen_batch_device(calls, dtype=None, device=None, max_len=None, u_dtype=
             done[ci] += bt.seg_len
         if fmt == 'pcm16':
             rows_export(device, tgt, base, total, wave, rows * T, np.full(n, T, dtype=np.int64), stream, 'pcm16')
+        if f0:                             # the f32 layout of wave: the same segments at the same places
+            track = torch.empty((n, T), dtype=torch.float32, device=dev)
+            if np.any(last < 0):
+                track.zero_()
+            done = np.zeros(n, dtype=np.int64)
+            for r, bt in enumerate(rounds):
+                ci = bt.round_calls
+                room = np.maximum(T - done[ci], 0)
+                cap = np.where(last[ci] == r, room, np.minimum(bt.seg_len, room))
+                bt.f0(track, rows[ci] * T + np.minimum(done[ci], T), cap, stream)
+                done[ci] += bt.seg_len
+            failed = np.flatnonzero(np.asarray(status) != 0)    # also the calls the front-end failed: no voiced sample
+            if failed.size:
+                with torch.cuda.stream(stream):
+                    track.index_fill_(0, torch.as_tensor(failed, device=dev), 0.0)
         lengths = torch.as_tensor(np.minimum(total, T), dtype=torch.int64).to(dev)
     finally:
         for bt in rounds:      # destroying a handle waits for its stream, i.e. for the export queued on it
             bt.close()
-    return wave, lengths, status
+    return (wave, lengths, status, track) if f0 else (wave, lengths, status)
 
 
 _CMP_METHODS = {'cor': _abi.SGB_CMP_COR, 'cosine': _abi.SGB_CMP_COSINE, 'dtw': _abi.SGB_CMP_DTW}

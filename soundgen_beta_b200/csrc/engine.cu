@@ -59,6 +59,9 @@ cudaError_t launch_spec_compare(const float *, const float *, const void *, int,
 size_t cepstra_smem_bytes(int n_in, int n_ceps, int order, int dn);
 cudaError_t launch_cepstra(const CepsTile *, int, const CepsRow *, const float *, const float *, float *, int, int, int,
                            int, cudaStream_t);
+cudaError_t launch_f0_track(const sgb_syllable *, int, const SylCtrl *, const Pools &, F0Epochs *, const F0Chunk *, int,
+                            const int64_t *, const int64_t *, const F0Span *, float *, cudaStream_t);
+cudaError_t launch_f0_frames(const F0Seg *, int, const F0Row *, const float *, int, double, float *, cudaStream_t);
 void launch_noise_final(const sgb_noise *, int, const NoiseLayout *, const double *, const double *, const int *, int,
                         const float *, float *, void *, double *, const int64_t *, int, cudaStream_t);
 size_t contour_tab_bytes();
@@ -220,6 +223,7 @@ struct sgb_batch {
   DBuf d_amp, d_amp32, d_wave, d_raw, d_sound, d_voiced, d_filt, d_noise_raw, d_noise_fin, d_env, d_out, d_out64;
   DBuf d_trk, d_mouth, d_formants_late, d_tiles_tc, d_ntabs, d_order, d_mtabs;
   DBuf d_knots, d_koff, d_ctab, d_btabs, d_envk;   // contour knot pool, per-contour offsets, headers (contour.cuh)
+  DBuf d_f0ep;                                     // K6's epoch spans replayed for the f0 track (sgb_batch_f0)
   int64_t knot_total = 0;
   bool any_aglobal = false;
   struct RunState *rs = nullptr;     // state carried from run_begin to run_finish
@@ -449,7 +453,7 @@ void sgb_batch_destroy(sgb_batch *b) {
                  &b->d_sound, &b->d_voiced, &b->d_filt, &b->d_noise_raw, &b->d_noise_fin, &b->d_env, &b->d_out,
                  &b->d_out64, &b->d_bl, &b->d_place, &b->d_nl, &b->d_envinst, &b->d_plans, &b->d_tw, &b->d_win,
                  &b->d_fjobs, &b->d_njobs, &b->d_fsegs, &b->d_nsegs, &b->d_max, &b->d_trk, &b->d_mouth, &b->d_formants_late, &b->d_tiles_tc, &b->d_ntabs, &b->d_order, &b->d_mtabs,
-                 &b->d_knots, &b->d_koff, &b->d_ctab, &b->d_btabs, &b->d_envk};
+                 &b->d_knots, &b->d_koff, &b->d_ctab, &b->d_btabs, &b->d_envk, &b->d_f0ep};
   for (auto d : all) d->release();
   for (auto &d : b->p_i32) d.release();
   for (auto &d : b->p_f64) d.release();
@@ -1954,6 +1958,137 @@ int sgb_rows_cepstra(int32_t device, const float *src, int64_t src_elems, const 
   if ((rc = export_queue(D->x, D->st, (cudaStream_t)o->stream, bytes, fill, launch)) != SGB_OK) return rc;
   if (o->out_written)
     for (int32_t c = 0; c < n; c++) o->out_written[c] = std::min(frames[c], o->cap[c]);
+  return SGB_OK;
+}
+
+// ---- f0 track of the last run (K12a) ----
+int sgb_batch_f0(sgb_batch *b, const sgb_device_out *o) {
+  if (!b) return fail(SGB_ERR_INVALID, "null batch");
+  if (!b->have_run) return fail(SGB_ERR_STATE, "no completed run");
+  CK(cudaSetDevice(b->device));
+  const int32_t n = (int32_t)b->call_len.size();
+  const int S = (int)b->syls.size();
+  int rc = export_check(b->device, nullptr, nullptr, b->call_len.data(), n, o, 1, false);
+  if (rc != SGB_OK) return rc;
+  // voiced spans: syllables of kind 1 that synthesised, in calls that did, where they land in the call's output
+  // (bout start + final_shift + the syllable's place in `sound`, cut at filt_len: istft overlap-adds at the stft
+  // frame starts, so positions in the filtered bout are positions in `sound`)
+  std::vector<F0Span> spans;
+  std::vector<F0Chunk> chunks;
+  for (int32_t c = 0; c < n; c++) {
+    const int32_t s_lo = (int32_t)spans.size();
+    if (b->call_status[c] == SGB_OK) {
+      const sgb_call &CL = b->calls[c];
+      for (int bi = CL.bout_begin; bi < CL.bout_end; bi++) {
+        const BoutLayout &L = b->bl[bi];
+        const int64_t t_bout = L.out_off - b->call_off[c] + L.final_shift;
+        for (int s = b->bouts[bi].syl_begin; s < b->bouts[bi].syl_end; s++) {
+          if (b->syls[s].kind != 1 || b->summary[s].status != SGB_OK) continue;
+          const int64_t r0 = b->place[s].dst_off - L.sound_off;
+          const int64_t m = std::min<int64_t>(b->place[s].len, L.filt_len - r0);
+          if (m > 0) spans.push_back(F0Span{t_bout + r0, (int32_t)m, s});
+        }
+      }
+    }
+    const int32_t s_hi = (int32_t)spans.size();
+    int32_t sp = s_lo;
+    for (int64_t k = 0; k * F0_CHUNK < o->cap[c]; k++) {
+      while (sp < s_hi && spans[sp].t0 + spans[sp].n <= k * F0_CHUNK) sp++;
+      chunks.push_back(F0Chunk{c, (int32_t)k, sp, s_hi});
+    }
+  }
+  if (chunks.size() > (size_t)INT32_MAX) return fail(SGB_ERR_UNSUPPORTED, "too many chunks");
+  CK(b->d_f0ep.ensure(sizeof(F0Epochs) * (size_t)std::max(S, 1)));
+  if (!b->xo) b->xo = new ExportCtx();
+  auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
+  const size_t o_spans = up16(16 * (size_t)n), o_chunks = up16(o_spans + sizeof(F0Span) * spans.size());
+  const size_t bytes = o_chunks + sizeof(F0Chunk) * chunks.size();
+  auto fill = [&](char *h) {
+    int64_t *t = reinterpret_cast<int64_t *>(h);
+    for (int32_t c = 0; c < n; c++) { t[c] = o->dst_off[c]; t[n + c] = o->cap[c]; }
+    if (!spans.empty()) memcpy(h + o_spans, spans.data(), sizeof(F0Span) * spans.size());
+    if (!chunks.empty()) memcpy(h + o_chunks, chunks.data(), sizeof(F0Chunk) * chunks.size());
+  };
+  auto launch = [&](const char *d) -> int {
+    const int64_t *t = reinterpret_cast<const int64_t *>(d);
+    cudaError_t e = launch_f0_track(b->d_syls.as<sgb_syllable>(), S, b->d_ctrl.as<SylCtrl>(), b->pools,
+                                    b->d_f0ep.as<F0Epochs>(), reinterpret_cast<const F0Chunk *>(d + o_chunks),
+                                    (int)chunks.size(), t, t + n, reinterpret_cast<const F0Span *>(d + o_spans),
+                                    (float *)o->dst, b->st);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return fail(SGB_ERR_CUDA, "k_f0_track launch failed (%zu chunks): %s", chunks.size(), cudaGetErrorString(e));
+    }
+    return SGB_OK;
+  };
+  // on the handle's stream, like the export: the handle's next run cannot overwrite the spline or SylCtrl first
+  if ((rc = export_queue(*b->xo, b->st, (cudaStream_t)o->stream, bytes, fill, launch)) != SGB_OK) return rc;
+  if (o->out_written)
+    for (int32_t c = 0; c < n; c++) o->out_written[c] = std::min(b->call_len[c], o->cap[c]);
+  return SGB_OK;
+}
+
+// ---- frame labels of f0 tracks (K12b) ----
+int sgb_rows_f0_frames(int32_t device, const float *src, int64_t src_elems, const int64_t *src_off, const int64_t *len,
+                       int32_t n, int32_t wl, double overlap, const sgb_device_out *o) {
+  // the parameters and the source rows alone (no device needed)
+  if (wl < 4 || (wl & 1)) return fail(SGB_ERR_INVALID, "window of %d points: an even wl >= 4 is needed", wl);
+  if (!(overlap >= 0.0 && overlap < 100.0)) return fail(SGB_ERR_INVALID, "overlap %g out of [0, 100)", overlap);
+  const double h = wl - (overlap * wl / 100.0);
+  if (!(h >= 1.0)) return fail(SGB_ERR_INVALID, "hop %g of a %d-point window is below one sample", h, wl);
+  if (!o) return fail(SGB_ERR_INVALID, "null sgb_device_out");
+  if (o->format != SGB_OUT_F32) return fail(SGB_ERR_INVALID, "unsupported output format %d", o->format);
+  if (n < 0 || src_elems < 0) return fail(SGB_ERR_INVALID, "negative row count or src_elems");
+  if (n > 0 && (!src_off || !len)) return fail(SGB_ERR_INVALID, "null row table");
+  for (int32_t c = 0; c < n; c++) {
+    const int64_t so = src_off[c], ln = len[c];
+    if (so < 0 || ln < 0) return fail(SGB_ERR_INVALID, "row %d: negative source offset or length", c);
+    if (so > src_elems || ln > src_elems - so)
+      return fail(SGB_ERR_INVALID, "row %d: samples [%lld, %lld more) outside src (%lld elements)", c, (long long)so,
+                  (long long)ln, (long long)src_elems);
+  }
+  int rc = rows_device_check(device, src, n);
+  if (rc != SGB_OK) return rc;
+  if ((rc = export_check(device, n > 0 ? src : nullptr, src_off, len, n, o, 2, false)) != SGB_OK) return rc;
+  std::vector<F0Row> rows((size_t)n);
+  std::vector<F0Seg> segs;
+  for (int32_t c = 0; c < n; c++) {
+    if (o->cap[c] > INT32_MAX) return fail(SGB_ERR_INVALID, "row %d: %lld frames of capacity (at most 2^31 - 1)", c,
+                                           (long long)o->cap[c]);
+    const int64_t nc = spec_nc(len[c], wl, h), m = std::min(nc, o->cap[c]);
+    rows[c] = F0Row{src_off[c], o->dst_off[c], len[c], nc, o->cap[c]};
+    for (int64_t k = 0; k < m; k += F0F_FRAMES)
+      segs.push_back(F0Seg{c, (int32_t)k, (int32_t)std::min<int64_t>(m, k + F0F_FRAMES), 0});
+    for (int64_t k = m; k < o->cap[c]; k += 4096)    // zero tails: 8192 floats per segment
+      segs.push_back(F0Seg{c, (int32_t)k, (int32_t)std::min<int64_t>(o->cap[c], k + 4096), 1});
+  }
+  if (segs.size() > (size_t)INT32_MAX) return fail(SGB_ERR_UNSUPPORTED, "too many segments");
+  if (!segs.empty() && src_elems > 0) {               // the kernel reads src while it writes dst
+    const char *s0 = reinterpret_cast<const char *>(src), *s1 = s0 + 4 * src_elems;
+    const char *d0 = reinterpret_cast<const char *>(o->dst), *d1 = d0 + 4 * o->dst_elems;
+    if (d0 < s1 && s0 < d1) return fail(SGB_ERR_INVALID, "dst overlaps src");
+  }
+  DeviceExport *D;
+  if ((rc = device_export(device, &D)) != SGB_OK) return rc;
+  std::lock_guard<std::mutex> g(D->mu);
+  const size_t o_segs = (sizeof(F0Row) * rows.size() + 15) & ~(size_t)15;
+  const size_t bytes = o_segs + sizeof(F0Seg) * segs.size();
+  auto fill = [&](char *hp) {
+    if (n) memcpy(hp, rows.data(), sizeof(F0Row) * rows.size());
+    if (!segs.empty()) memcpy(hp + o_segs, segs.data(), sizeof(F0Seg) * segs.size());
+  };
+  auto launch = [&](const char *d) -> int {
+    cudaError_t e = launch_f0_frames(reinterpret_cast<const F0Seg *>(d + o_segs), (int)segs.size(),
+                                     reinterpret_cast<const F0Row *>(d), src, wl, h, (float *)o->dst, D->st);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return fail(SGB_ERR_CUDA, "k_f0_frames launch failed (%zu segments): %s", segs.size(), cudaGetErrorString(e));
+    }
+    return SGB_OK;
+  };
+  if ((rc = export_queue(D->x, D->st, (cudaStream_t)o->stream, bytes, fill, launch)) != SGB_OK) return rc;
+  if (o->out_written)
+    for (int32_t c = 0; c < n; c++) o->out_written[c] = std::min(rows[c].nc, rows[c].cap);
   return SGB_OK;
 }
 

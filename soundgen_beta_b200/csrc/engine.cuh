@@ -162,6 +162,20 @@ struct CepsRow {             // one row of cepstra (K11); nc counts input frames
 struct CepsTile { int32_t row, t0, t1, zero; };   // output frames [t0, t1) of a row; zero: the tail past nc
 constexpr int CEPS_TILE = 64;                     // most frames of a compute tile (the choice: kernels_ceps.cu)
 
+// f0 track (K12a).  A voiced span: n output samples of a row from sample t0 on, the composed samples [0, n) of
+// syllable syl.  A row's spans are sorted and disjoint; everything outside them is unvoiced.
+struct F0Span { int64_t t0; int32_t n, syl; };
+// one CTA of K12a: samples [chunk * F0_CHUNK, (chunk + 1) * F0_CHUNK) of a row, whose spans are [s_lo, s_hi)
+struct F0Chunk { int32_t row, chunk, s_lo, s_hi; };
+// K6's epoch spans of one syllable, replayed by k_f0_epochs: epoch e covers the composed positions q >= ep[e].x
+// (up to the next epoch's), where pitch_upsampled is read at the 1-based index u = ep[e].y + q
+struct F0Epochs { int32_t nE, G; int2 ep[SGB_MAX_EPOCHS]; };
+constexpr int F0_THREADS = 256, F0_PER_THREAD = 32, F0_CHUNK = F0_THREADS * F0_PER_THREAD;
+// K12b: frames [ka, kb) of a row (zero: frames at or past nc, written as zeros)
+struct F0Row { int64_t src_off, dst_off, len, nc, cap; };
+struct F0Seg { int32_t row, ka, kb, zero; };
+constexpr int F0F_THREADS = 256, F0F_FRAMES = 256;  // frames per segment: at most one per thread
+
 
 // Ordered-int encoding so that atomicMax on int implements a signed float max.
 __device__ __forceinline__ int float_to_ordered(float f) {
