@@ -396,6 +396,11 @@ int sgb_batch_pitch_per_gc(sgb_batch *b, int32_t syl, double *out, int32_t cap);
  * Null f64 and f32 report the shape only. */
 int sgb_batch_amp_tables(sgb_batch *b, int32_t syl, int32_t epoch, double *f64, float *f32, int64_t cap,
                          int32_t *shape);
+/* Diagnostic: the FP32 spectral envelope the last run filtered with.  kind 0: the main filter of bout `index`;
+ * kind 1: the filter of noise `index`.  shape[2] receives {nr, nint}; out (cap >= nr * nint floats) the table
+ * column by column, copied on the handle's stream (the call returns once it has arrived).  A bypassed bout or an
+ * unfiltered noise has shape {0, 0}; a null out reports the shape only.  SGB_ERR_STATE before the first run. */
+int sgb_batch_envelope(sgb_batch *b, int32_t kind, int32_t index, float *out, int64_t cap, int32_t *shape);
 /* Diagnostic: nine position-weighted checksums of the last run's intermediates (see engine.cu);
  * identical inputs must give identical checksums on every run. */
 int sgb_batch_checksums(sgb_batch *b, uint64_t *out, int32_t cap);

@@ -712,10 +712,13 @@ def getSpectralEnvelope(nr, nc, formants=None, formantDep=1, rolloffLip=6, mouth
                         mouthOpenThres=0, openMouthBoost=0, vocalTract=None, temperature=0,
                         smoothLinearFactor=1, samplingRate=16000, speedSound=35400,
                         formants_upsampled=None, contour_method='loess', formDrift=.3, formDisp=.2,
-                        formantDepStoch=30, rng=None):
+                        formantDepStoch=30, rng=None, terms=None):
     """sourceSpectrum.R:261-566 with temperature == 0 (the stochastic block
     :346-415 draws rgamma/rnorm on the host; pass its result via
-    `formants_upsampled`).  `formants`: list of (k,4) arrays or None."""
+    `formants_upsampled`).  `formants`: list of (k,4) arrays or None.
+    `terms` (a dict) receives the intermediates an error bound needs: 'tracks' (the formant tracks in Hz after
+    the stochastic block), 'smoothed' (the tracks or the mouth opening come from a contour), 'bins' (the (nc, 4) rows of every gamma bump in bins, nasal pole and zero included),
+    'mouth_open', 'mouth_bin', 'formantDep', 'rolloffLip', 'openMouthBoost'."""
     nr = int(nr)
     nc = int(nc)
     if formants is not None and not (isinstance(vocalTract, (int, float))) and formants[0].shape[1] > 2:
@@ -766,6 +769,11 @@ def getSpectralEnvelope(nr, nc, formants=None, formantDep=1, rolloffLip=6, mouth
                     if rw.size > 1:
                         rw = rw - r_mean(rw) + 1
                     f[:, c] = f[:, c] * rw
+        if terms is not None:
+            terms['tracks'] = [f.copy() for f in fu]
+            # tracks that a device evaluates (splines) or draws (temperature > 0) on its own, or a mouth contour
+            terms['smoothed'] = (mouthAnchors is not None or temperature > 0 or
+                                 (formants_upsampled is None and max(np.asarray(f).shape[0] for f in formants) > 1))
         bin_width = samplingRate / 2 / nr  # :419
         for f in fu:
             f[:, 1] = (f[:, 1] - bin_width / 2) / bin_width + 1
@@ -814,10 +822,17 @@ def getSpectralEnvelope(nr, nc, formants=None, formantDep=1, rolloffLip=6, mouth
                 logd = (shape[c] - 1) * lx - rate[c] * x  # dgamma up to a constant
                 env[:, c] += np.exp(logd - np.max(logd)) * f[c, 2]
         env = env * formantDep
+        if terms is not None:
+            terms['bins'] = fu
     lip_dB = rolloffLip * np.log2(np.arange(1, nr + 1, dtype=np.float64))  # :532-537
     for c in range(nc):
         env[:, c] = (env[:, c] + lip_dB * mouthOpen_binary[c]) * \
             2 ** (mouthOpening_upsampled[c] * openMouthBoost / 10)
+    if terms is not None:
+        terms.setdefault('bins', [])
+        terms.setdefault('smoothed', mouthAnchors is not None)
+        terms.update(mouth_open=mouthOpening_upsampled, mouth_bin=mouthOpen_binary, formantDep=formantDep,
+                     rolloffLip=rolloffLip, openMouthBoost=openMouthBoost)
     return 2 ** (env / 10)  # :540
 
 

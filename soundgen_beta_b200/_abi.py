@@ -149,7 +149,7 @@ EXPORTS = ['sgb_version', 'sgb_last_error', 'sgb_device_count', 'sgb_set_device'
            'sgb_batch_export', 'sgb_rows_export', 'sgb_spec_frames', 'sgb_batch_spectrogram', 'sgb_rows_spectrogram',
            'sgb_rows_compare', 'sgb_rows_cepstra', 'sgb_batch_f0', 'sgb_rows_f0_frames', 'sgb_param_range',
            'sgb_batch_syllable_len', 'sgb_batch_syllable_fetch', 'sgb_batch_noise_fetch',
-           'sgb_batch_artefacts', 'sgb_batch_artefact_ints', 'sgb_batch_pitch_per_gc', 'sgb_batch_amp_tables', 'sgb_batch_checksums', 'sgb_batch_debug_state',
+           'sgb_batch_artefacts', 'sgb_batch_artefact_ints', 'sgb_batch_pitch_per_gc', 'sgb_batch_amp_tables', 'sgb_batch_envelope', 'sgb_batch_checksums', 'sgb_batch_debug_state',
            'sgb_get_rolloff', 'sgb_get_spectral_envelope', 'sgb_filter_len', 'sgb_filter',
            'sgb_batch_run_begin', 'sgb_batch_run_finish', 'sgb_batch_bout_geometry', 'sgb_batch_set_tracks',
            'sgb_batch_z_used', 'sgb_abi_sizes', 'sgb_synth_min_rows_set', 'sgb_host_set_threads', 'sgb_frontend_create', 'sgb_frontend_destroy', 'sgb_frontend_add', 'sgb_frontend_add_seeded', 'sgb_frontend_add_many', 'sgb_frontend_clear',
@@ -214,6 +214,7 @@ def load():
     L.sgb_batch_artefact_ints.argtypes = [vp, i32, C.c_int, vp, i32]
     L.sgb_batch_pitch_per_gc.argtypes = [vp, i32, vp, i32]
     L.sgb_batch_amp_tables.argtypes = [vp, i32, i32, vp, vp, i64, vp]
+    L.sgb_batch_envelope.argtypes = [vp, i32, i32, vp, i64, vp]
     L.sgb_batch_checksums.argtypes = [vp, vp, i32]
     L.sgb_batch_debug_state.argtypes = [vp, vp, i32]
     L.sgb_get_rolloff.argtypes = [vp, i32, i32, vp, i32, vp, i32, vp, i32, f64, f64, f64, f64,

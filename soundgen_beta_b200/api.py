@@ -700,6 +700,18 @@ class Batch:
         _check(self.L.sgb_batch_noise_fetch(self.h, n, _ptr(out), out.size))
         return out[:int(length)]
 
+    def envelope(self, kind, index):
+        """The FP32 spectral envelope (nr x nint) the last run filtered with: kind 0 the main filter of bout `index`,
+        kind 1 the filter of noise `index`; None for a bypassed bout or an unfiltered noise."""
+        shape = np.zeros(2, dtype=np.int32)
+        _check(self.L.sgb_batch_envelope(self.h, kind, index, None, 0, _ptr(shape)))
+        nr, nint = (int(v) for v in shape)
+        if nr * nint == 0:
+            return None
+        out = np.zeros(nr * nint, dtype=np.float32)
+        _check(self.L.sgb_batch_envelope(self.h, kind, index, _ptr(out), out.size, _ptr(shape)))
+        return out.reshape(nint, nr).T.copy()
+
     def artefacts(self, s):
         a = SylArtefacts()
         _check(self.L.sgb_batch_artefacts(self.h, s, C.byref(a)))

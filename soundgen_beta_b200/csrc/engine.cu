@@ -39,10 +39,12 @@ void launch_place_voiced(const sgb_syllable *, int, const SylCtrl *, const SylLa
                          const Pools &, const float *, float *, int, cudaStream_t);
 void launch_env_tracks(const EnvInst *, int, const sgb_envelope *, const sgb_formant_ref *, const double *,
                        const double *, double *, double *, void *, double *, cudaStream_t);
-void launch_envelope_f32(const EnvInst *, int, int, const sgb_envelope *, const sgb_formant_ref *, const double *,
-                         const double *, const double *, const double *, const double *, float *, cudaStream_t);
-void launch_envelope_f64(const EnvInst *, int, int, const sgb_envelope *, const sgb_formant_ref *, const double *,
-                         const double *, const double *, const double *, const double *, double *, cudaStream_t);
+cudaError_t launch_envelope_f32(const EnvInst *, int, int, int, const sgb_envelope *, const sgb_formant_ref *,
+                                const double *, const double *, const double *, const double *, const double *, float *,
+                                cudaStream_t);
+cudaError_t launch_envelope_f64(const EnvInst *, int, int, int, const sgb_envelope *, const sgb_formant_ref *,
+                                const double *, const double *, const double *, const double *, const double *, double *,
+                                cudaStream_t);
 size_t stft_smem_bytes(int n, double h_in, double h_out, int mode);
 size_t stft_smem_bytes_spec(int n, double h_in, double h_out, int mode, int spec);
 cudaError_t launch_stft(int mode, int u_is_float, int spec, const FftSeg *, int, const FftJob *, const FftPlan *,
@@ -535,7 +537,8 @@ int sgb_batch_upload(sgb_batch *b, const sgb_batch_desc *D) {
   }
   for (int e = 0; e < D->n_envelopes; e++) {
     const sgb_envelope &E = D->envelopes[e];
-    if (E.n_formants < 0 || E.n_formants > 62) return fail(SGB_ERR_UNSUPPORTED, "envelope %d: more than 62 formants", e);
+    if (E.n_formants < 0 || E.n_formants > SGB_MAX_FORMANTS)
+      return fail(SGB_ERR_UNSUPPORTED, "envelope %d: %d formants (at most %d)", e, E.n_formants, SGB_MAX_FORMANTS);
     if (E.n_formants > 0 && (E.formant_off < 0 || E.formant_off + E.n_formants > D->n_formant_refs))
       return fail(SGB_ERR_INVALID, "envelope %d: formant refs", e);
     if (E.mouth_n < 0 || (E.mouth_n > 0 && (E.mouth_off < 0 || E.mouth_off + E.mouth_n > D->n_anchors)))
@@ -1191,11 +1194,13 @@ int sgb_batch_run_finish(sgb_batch *b, sgb_run_info *info_out) {
   std::vector<float> &win_host = PT.win;
   const int64_t tw_total = (int64_t)tw_host.size(), win_total = (int64_t)win_host.size();
   // ---- upload layout ----
-  int max_nc = 0;   // total (instance, column) work items of K4: the kernel runs one CTA per item
+  int max_nc = 0;   // total (instance, column) work items of K4: the kernel runs one warp per item
+  int max_f = 0;    // most formants of one of K4's envelopes: sizes its shared memory
   int64_t trk_total = 0, envk_total = 0;
   for (auto &I : envinst) {
     I.col0 = max_nc; max_nc += I.nc;
     const sgb_envelope &E = b->envs[I.env_id];
+    max_f = std::max(max_f, E.n_formants);
     bool moving = false;
     if (E.tracks_given == 0)
       for (int f = 0; f < E.n_formants; f++) if (b->frefs[E.formant_off + f].n > 1) moving = true;
@@ -1262,10 +1267,9 @@ int sgb_batch_run_finish(sgb_batch *b, sgb_run_info *info_out) {
                     b->d_frefs.as<sgb_formant_ref>(), b->d_formants.as<double>(), b->d_anchors.as<double>(),
                     b->d_trk.as<double>(), b->d_mouth.as<double>(), b->d_mtabs.p, b->d_envk.as<double>(), st);
   CKL("launch_env_tracks");
-  launch_envelope_f32(b->d_envinst.as<EnvInst>(), (int)envinst.size(), max_nc, b->d_envs.as<sgb_envelope>(),
-                      b->d_frefs.as<sgb_formant_ref>(), b->d_formants.as<double>(), b->d_formants_late.as<double>(), b->d_trk.as<double>(),
-                      b->d_mouth.as<double>(), b->d_pre.as<double>(), b->d_env.as<float>(), st);
-  CKL("launch_envelope_f32");
+  CK(launch_envelope_f32(b->d_envinst.as<EnvInst>(), (int)envinst.size(), max_nc, max_f, b->d_envs.as<sgb_envelope>(),
+                         b->d_frefs.as<sgb_formant_ref>(), b->d_formants.as<double>(), b->d_formants_late.as<double>(),
+                         b->d_trk.as<double>(), b->d_mouth.as<double>(), b->d_pre.as<double>(), b->d_env.as<float>(), st));
   if (!envinst.empty()) launches += 2;
   CK(cudaEventRecord(ev[6], st)); trace_mark(b, 6);
   // ---- K5 noise ----
@@ -1352,7 +1356,8 @@ int sgb_batch_bout_geometry(sgb_batch *b, int32_t bout, int32_t *nc, int32_t *ni
 int sgb_batch_set_tracks(sgb_batch *b, int32_t env, const double *rows, int32_t n_formants, int32_t nc) {
   if (!b || !b->rs || !b->rs->begun) return fail(SGB_ERR_STATE, "sgb_batch_set_tracks outside run_begin / run_finish");
   if (env < 0 || env >= (int)b->envs.size() || !rows || nc < 1) return fail(SGB_ERR_INVALID, "bad argument");
-  if (n_formants < 1 || n_formants > 62) return fail(SGB_ERR_UNSUPPORTED, "%d formant tracks (at most 62)", n_formants);
+  if (n_formants < 1 || n_formants > SGB_MAX_FORMANTS)
+    return fail(SGB_ERR_UNSUPPORTED, "%d formant tracks (at most %d)", n_formants, SGB_MAX_FORMANTS);
   sgb_envelope &E = b->envs[env];
   E.tracks_given = 1;
   E.n_formants = n_formants;
@@ -2247,6 +2252,35 @@ int sgb_batch_amp_tables(sgb_batch *b, int32_t syl, int32_t epoch, double *f64, 
   return SGB_OK;
 }
 
+// Diagnostic: the FP32 envelope table K4 wrote for the main filter of bout `index` (kind 0) or for the filter of noise
+// `index` (kind 1) in the last run, nr x nint column-major as K2 / K5 read it.  shape = {nr, nint}, {0, 0} for a
+// bypassed bout or an unfiltered noise.  A null out only reports the shape.
+int sgb_batch_envelope(sgb_batch *b, int32_t kind, int32_t index, float *out, int64_t cap, int32_t *shape) {
+  if (!b || !shape) return fail(SGB_ERR_INVALID, "null argument");
+  if (!b->have_run) return fail(SGB_ERR_STATE, "no run");
+  int64_t off = -1;
+  int32_t nr = 0, nint = 0;
+  if (kind == 0) {
+    if (index < 0 || index >= (int)b->bl.size()) return fail(SGB_ERR_INVALID, "bout index");
+    const BoutLayout &L = b->bl[index];
+    if (!L.bypass) { off = L.env_off; nr = L.wl / 2; nint = L.nint; }
+  } else if (kind == 1) {
+    if (index < 0 || index >= (int)b->nl.size()) return fail(SGB_ERR_INVALID, "noise index");
+    const NoiseLayout &Q = b->nl[index];
+    if (Q.env_off >= 0) { off = Q.env_off; nr = b->noises[index].wl / 2; nint = Q.nc_env; }
+  } else {
+    return fail(SGB_ERR_INVALID, "kind must be 0 (bout) or 1 (noise)");
+  }
+  shape[0] = nr; shape[1] = nint;
+  const int64_t n = (int64_t)nr * nint;
+  if (!out || n == 0) return SGB_OK;
+  if (cap < n) return fail(SGB_ERR_INVALID, "buffer too small");
+  CK(cudaSetDevice(b->device));
+  CK(cudaMemcpyAsync(out, b->d_env.as<float>() + off, 4 * (size_t)n, cudaMemcpyDeviceToHost, b->st));
+  CK(cudaStreamSynchronize(b->st));
+  return SGB_OK;
+}
+
 int sgb_batch_pitch_per_gc(sgb_batch *b, int32_t syl, double *out, int32_t cap) {
   if (!out) return fail(SGB_ERR_INVALID, "null argument");
   SylCtrl C;
@@ -2299,7 +2333,8 @@ int sgb_get_spectral_envelope(int32_t nr, int32_t nc, const sgb_envelope *env, c
                               const int32_t *formant_n, const double *mouth_anchors, double *out) {
   if (!env || !out) return fail(SGB_ERR_INVALID, "null argument");
   if (nr < 1 || nc < 1) return fail(SGB_ERR_INVALID, "nr and nc must be positive");
-  if (env->n_formants < 0 || env->n_formants > 62) return fail(SGB_ERR_UNSUPPORTED, "more than 62 formants");
+  if (env->n_formants < 0 || env->n_formants > SGB_MAX_FORMANTS)
+    return fail(SGB_ERR_UNSUPPORTED, "%d formants (at most %d)", env->n_formants, SGB_MAX_FORMANTS);
   if (env->n_formants > 0 && (!formants || !formant_n)) return fail(SGB_ERR_INVALID, "formants missing");
   if (env->mouth_n > 0 && !mouth_anchors) return fail(SGB_ERR_INVALID, "mouth anchors missing");
   int nd = 0;
@@ -2337,9 +2372,8 @@ int sgb_get_spectral_envelope(int32_t nr, int32_t nc, const sgb_envelope *env, c
     launch_env_tracks(dI.as<EnvInst>(), 1, dE.as<sgb_envelope>(), dR.as<sgb_formant_ref>(), dF.as<double>(),
                       dA.as<double>(), dT.as<double>(), dM.as<double>(), dTab.p, dK.as<double>(), 0);
     CKL("launch_env_tracks");
-    launch_envelope_f64(dI.as<EnvInst>(), 1, nc, dE.as<sgb_envelope>(), dR.as<sgb_formant_ref>(), dF.as<double>(),
-                        nullptr, dT.as<double>(), dM.as<double>(), nullptr, dO.as<double>(), 0);
-    CK(cudaGetLastError());
+    CK(launch_envelope_f64(dI.as<EnvInst>(), 1, nc, E.n_formants, dE.as<sgb_envelope>(), dR.as<sgb_formant_ref>(),
+                           dF.as<double>(), nullptr, dT.as<double>(), dM.as<double>(), nullptr, dO.as<double>(), 0));
     CK(cudaMemcpy(out, dO.p, 8 * (size_t)nr * nc, cudaMemcpyDeviceToHost));
     return SGB_OK;
   };

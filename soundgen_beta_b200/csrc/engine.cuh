@@ -10,6 +10,11 @@
 #define SYNTH_STAGE 128                     // float4 entries per warp stage: columns x rows per block
 #define SYNTH_PC 6                          // doubles per spline piece {kt, c0..c4}
 
+// Formants per filter: the given ones, the stochastic pseudo-formants and host-drawn tracks together (K4 adds the
+// nasal pole and zero on top).  K4 keeps 7 FP64 values per formant for each of its 4 warps in dynamic shared memory,
+// sized by the launch's largest count: 224 B x (1024 + 2) = 229,824 B, inside the 232,448 B a block may opt in to.
+#define SGB_MAX_FORMANTS 1024
+
 // Pooled per-glottal-cycle scratch: syllable s owns [gc_off[s], gc_off[s+1]) of every array.
 struct Pools {
   double *pitch_w;      // vibrato'd pitch, same layout as the pitch pool

@@ -18,7 +18,7 @@
 #include <vector>
 #include <chrono>
 
-#include "ctrl.cuh"
+#include "engine.cuh"
 #include "rrng.h"
 #include "hostpar.h"
 
@@ -320,8 +320,9 @@ void upsample_formants(const std::vector<Formant> &fl, int nc, double smoothLine
 }
 
 // Stochastic block of getSpectralEnvelope (sourceSpectrum.R:346-415): extra pseudo-formants up to
-// Nyquist - 1000 Hz, then a random-walk wiggle of every formant's freq / amp / width.
-void stochastic_formants(RRng &g, std::vector<std::vector<double>> &up, int nc, double temperature, double formDrift,
+// Nyquist - 1000 Hz, then a random-walk wiggle of every formant's freq / amp / width.  R's loop has no cap; a filter
+// that would need more than SGB_MAX_FORMANTS formants is not drawn further: false, and the caller refuses the call.
+bool stochastic_formants(RRng &g, std::vector<std::vector<double>> &up, int nc, double temperature, double formDrift,
                          double formDisp, double formantDep, double formantDepStoch, double vocalTract,
                          double samplingRate, double speedSound) {
   const double formantDispersion = 2 * speedSound / (4 * vocalTract);    // vocalTract is numeric in soundgen()
@@ -332,7 +333,7 @@ void stochastic_formants(RRng &g, std::vector<std::vector<double>> &up, int nc, 
   const double rr = temperature * formDrift;
   if (!std::isnan(sdG) && formantDepStoch > 0) {
     while (freq_max < (samplingRate / 2 - 1000)) {
-      if (nF >= 62) break;
+      if (nF >= SGB_MAX_FORMANTS) return false;
       std::vector<double> rw;
       random_walk_host(g, nc, rr, 0.0, [] { return 0.0; }, rw);
       if (rw.size() > 1) { double m = r_mean(rw.data(), (int)rw.size()); for (auto &e : rw) e = e - m + 1; }
@@ -361,6 +362,12 @@ void stochastic_formants(RRng &g, std::vector<std::vector<double>> &up, int nc, 
       if (rw.size() > 1) { double m = r_mean(rw.data(), (int)rw.size()); for (auto &e : rw) e = e - m + 1; }
       for (int k = 0; k < nc; k++) up[f][4 * k + j] = up[f][4 * k + j] * rw[rw.size() > 1 ? k : 0];
     }
+  return true;
+}
+
+void refuse_formants(CallState &C) {
+  C.status = SGB_ERR_UNSUPPORTED;
+  warn(C, "the stochastic formants reach past %d formants per filter", SGB_MAX_FORMANTS);
 }
 
 // number of normals generateHarmonics will consume for this syllable (source.R:239-353), from the
@@ -833,8 +840,9 @@ bool emit_bout(sgb_frontend *fe, int ci, int b) {
         if (T > 0) {
           std::vector<std::vector<double>> up;
           upsample_formants(C.formantsNoise, nInt, 1.0, up);
-          stochastic_formants(g, up, nInt, T, a.tempEffects[1], a.tempEffects[2], a.formantDep, a.formantDepStoch,
-                              C.vocalTract, sr, 35400.0);
+          if (!stochastic_formants(g, up, nInt, T, a.tempEffects[1], a.tempEffects[2], a.formantDep, a.formantDepStoch,
+                                   C.vocalTract, sr, 35400.0))
+            refuse_formants(C);
           N.env_id = add_envelope(fe, C, &C.formantsNoise, true, nInt, &up, nInt, false);
         } else {
           N.env_id = add_envelope(fe, C, &C.formantsNoise, true, nInt, nullptr, 0, false);
@@ -898,7 +906,9 @@ bool emit_bout(sgb_frontend *fe, int ci, int b) {
         schwa.push_back(f); fl = &schwa;
       }
       upsample_formants(*fl, 1, 1.0, up);
-      stochastic_formants(g, up, 1, T, a.tempEffects[1], a.tempEffects[2], a.formantDep, a.formantDepStoch, C.vocalTract, sr, 35400.0);
+      if (!stochastic_formants(g, up, 1, T, a.tempEffects[1], a.tempEffects[2], a.formantDep, a.formantDepStoch,
+                               C.vocalTract, sr, 35400.0))
+        refuse_formants(C);
       env_main = add_envelope(fe, C, fl, true, 0, &up, 1, false);
     }
   } else {
@@ -1074,9 +1084,10 @@ int sgb_frontend_resolve(sgb_frontend *fe, sgb_batch *b) {
     }
     std::vector<std::vector<double>> up;
     upsample_formants(*fl, J.ncol, 1.0, up);
-    if (J.nint >= 1)    // sum(sound) == 0 skips the filter block, and with it the draws (soundgen.R:736-739)
-      stochastic_formants(C.rng, up, J.ncol, a.temperature, a.tempEffects[1], a.tempEffects[2], a.formantDep,
-                          a.formantDepStoch, C.vocalTract, a.samplingRate, 35400.0);
+    // sum(sound) == 0 skips the filter block, and with it the draws (soundgen.R:736-739)
+    if (J.nint >= 1 && !stochastic_formants(C.rng, up, J.ncol, a.temperature, a.tempEffects[1], a.tempEffects[2],
+                                            a.formantDep, a.formantDepStoch, C.vocalTract, a.samplingRate, 35400.0))
+      refuse_formants(C);
     for (auto &t : up) J.rows.insert(J.rows.end(), t.begin(), t.end());
     J.nf = (int)up.size();
   });

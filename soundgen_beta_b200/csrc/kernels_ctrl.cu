@@ -42,8 +42,9 @@ k_control(const sgb_syllable *syl, int S, const int32_t *__restrict__ order, con
   __shared__ int sh_status;
   if (sp.kind != 1) {
     if (threadIdx.x == 0) {
-      C.status = SGB_OK; C.nGC = 0; C.nEpochs = 0; C.tiles = 0; C.amp_elems = 0; C.wave_elems = 0;
-      C.n_up = 0; C.rows_kept = 0; C.nHarmonics = 0; C.n_jidx = 0; C.z_used = 0; C.use_ampl = 0;
+      // every count k_scan_sizes sums: the handle's SylCtrl slots keep whatever an earlier run left there
+      C.status = SGB_OK; C.nGC = 0; C.nEpochs = 0; C.tiles = 0; C.tiles_tc = 0; C.pad_tc = 0; C.amp_elems = 0;
+      C.wave_elems = 0; C.n_up = 0; C.rows_kept = 0; C.nHarmonics = 0; C.n_jidx = 0; C.z_used = 0; C.use_ampl = 0;
       C.out_len = (sp.kind == 0) ? sp.silent_len : sp.pitch_len;
       C.raw_max = 1.0;
     }

@@ -7,7 +7,10 @@
 
 #define ENV_THREADS 128
 #define ENV_WARPS (ENV_THREADS / 32)
-#define ENV_MAXF 64        // formants per filter (incl. stochastic extras and the nasal pole / zero)
+#define ENV_TABS 7         // per-warp formant tables (freq, amp, width; shape, rate, ref, amp of the bumps)
+
+// dynamic shared memory of k_envelope for filters of at most max_f formants (+ the nasal pole and zero)
+static size_t env_smem(int max_f) { return sizeof(double) * ENV_TABS * ENV_WARPS * (size_t)(max_f + 2); }
 
 template <typename OutT>
 __global__ void __launch_bounds__(ENV_THREADS, 6)
@@ -15,7 +18,7 @@ k_envelope(const EnvInst *__restrict__ inst, const sgb_envelope *__restrict__ en
            const sgb_formant_ref *__restrict__ fidx, const double *__restrict__ formants,
            const double *__restrict__ formants_late, const double *__restrict__ trk,
            const double *__restrict__ mouth, const double *__restrict__ pre,
-           OutT *__restrict__ out, int n_flat, int n_items) {
+           OutT *__restrict__ out, int n_flat, int n_items, int max_f) {
   // work item -> (instance, column): flat list (one item per warp; the instance is found by bisection
   // over col0) or the plain 2-D grid of the stand-alone API call (blockIdx.y = instance)
   const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -41,14 +44,14 @@ k_envelope(const EnvInst *__restrict__ inst, const sgb_envelope *__restrict__ en
     for (int r = lane; r < nr; r += 32) colL[r] = (OutT)m[r];
     return;
   }
-  __shared__ double sf_freq[ENV_WARPS][ENV_MAXF], sf_amp[ENV_WARPS][ENV_MAXF], sf_width[ENV_WARPS][ENV_MAXF];
-  __shared__ double sg_shape[ENV_WARPS][ENV_MAXF], sg_rate[ENV_WARPS][ENV_MAXF], sg_ref[ENV_WARPS][ENV_MAXF],
-      sg_amp[ENV_WARPS][ENV_MAXF];
+  // the warp's ENV_TABS tables of max_f + 2 entries (env_smem)
+  extern __shared__ double s_tabs[];
   __shared__ int s_nF[ENV_WARPS];
   __shared__ double s_mouth_open[ENV_WARPS], s_mouth_bin[ENV_WARPS];
-  double *f_freq = sf_freq[wid], *f_amp = sf_amp[wid], *f_width = sf_width[wid];
-  double *g_shape = sg_shape[wid], *g_rate = sg_rate[wid], *g_ref = sg_ref[wid], *g_amp = sg_amp[wid];
-  const int F = E.n_formants;     // <= ENV_MAXF - 2, checked at upload
+  const int nt = max_f + 2;
+  double *f_freq = s_tabs + (size_t)wid * ENV_TABS * nt, *f_amp = f_freq + nt, *f_width = f_amp + nt;
+  double *g_shape = f_width + nt, *g_rate = g_shape + nt, *g_ref = g_rate + nt, *g_amp = g_ref + nt;
+  const int F = E.n_formants;     // <= max_f <= SGB_MAX_FORMANTS, checked at upload
 
   // ---- formant values at column c (sourceSpectrum.R:321-344) ----
   for (int fl = lane; fl < F; fl += 32) {
@@ -232,18 +235,36 @@ void launch_env_tracks(const EnvInst *inst, int n_inst, const sgb_envelope *envs
   k_env_tracks<<<n_inst, ENV_THREADS, 0, st>>>(inst, envs, fidx, formants, (const ContourTab *)tabs, knots, trk, mouth);
 }
 
-void launch_envelope_f32(const EnvInst *inst, int n_inst, int max_nc, const sgb_envelope *envs,
-                         const sgb_formant_ref *fidx, const double *formants, const double *formants_late,
-                         const double *trk, const double *mouth, const double *pre, float *out, cudaStream_t st) {
-  if (n_inst <= 0 || max_nc <= 0) return;
-  // max_nc carries the TOTAL number of (instance, column) work items here: one warp each
-  k_envelope<float><<<(max_nc + ENV_WARPS - 1) / ENV_WARPS, ENV_THREADS, 0, st>>>(inst, envs, fidx, formants, formants_late, trk, mouth, pre,
-                                                                           out, n_inst, max_nc);
+// The opt-in is a property of the function on the device, shared by every handle and thread that launches it: always
+// the same value (room for SGB_MAX_FORMANTS), so that a concurrent launch never lowers it below what another needs.
+template <typename OutT>
+static cudaError_t env_smem_optin(size_t smem) {
+  if (smem <= 48 * 1024) return cudaSuccess;
+  return cudaFuncSetAttribute(k_envelope<OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              (int)env_smem(SGB_MAX_FORMANTS));
 }
-void launch_envelope_f64(const EnvInst *inst, int n_inst, int max_nc, const sgb_envelope *envs,
-                         const sgb_formant_ref *fidx, const double *formants, const double *formants_late,
-                         const double *trk, const double *mouth, const double *pre, double *out, cudaStream_t st) {
-  if (n_inst <= 0 || max_nc <= 0) return;
+
+// max_f: the largest n_formants of the launch's envelopes (<= SGB_MAX_FORMANTS)
+cudaError_t launch_envelope_f32(const EnvInst *inst, int n_inst, int max_nc, int max_f, const sgb_envelope *envs,
+                                const sgb_formant_ref *fidx, const double *formants, const double *formants_late,
+                                const double *trk, const double *mouth, const double *pre, float *out, cudaStream_t st) {
+  if (n_inst <= 0 || max_nc <= 0) return cudaSuccess;
+  const size_t smem = env_smem(max_f);
+  cudaError_t e = env_smem_optin<float>(smem);
+  if (e != cudaSuccess) return e;
+  // max_nc carries the TOTAL number of (instance, column) work items here: one warp each
+  k_envelope<float><<<(max_nc + ENV_WARPS - 1) / ENV_WARPS, ENV_THREADS, smem, st>>>(inst, envs, fidx, formants, formants_late,
+                                                                              trk, mouth, pre, out, n_inst, max_nc, max_f);
+  return cudaGetLastError();
+}
+cudaError_t launch_envelope_f64(const EnvInst *inst, int n_inst, int max_nc, int max_f, const sgb_envelope *envs,
+                                const sgb_formant_ref *fidx, const double *formants, const double *formants_late,
+                                const double *trk, const double *mouth, const double *pre, double *out, cudaStream_t st) {
+  if (n_inst <= 0 || max_nc <= 0) return cudaSuccess;
+  const size_t smem = env_smem(max_f);
+  cudaError_t e = env_smem_optin<double>(smem);
+  if (e != cudaSuccess) return e;
   dim3 g((max_nc + ENV_WARPS - 1) / ENV_WARPS, n_inst);
-  k_envelope<double><<<g, ENV_THREADS, 0, st>>>(inst, envs, fidx, formants, formants_late, trk, mouth, pre, out, 0, 0);
+  k_envelope<double><<<g, ENV_THREADS, smem, st>>>(inst, envs, fidx, formants, formants_late, trk, mouth, pre, out, 0, 0, max_f);
+  return cudaGetLastError();
 }
